@@ -2,11 +2,16 @@
 """bench.py — so100 env-steps/s at 65 536 envs/GPU (BASELINE.json metric), one process per GPU.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--task Env01] [--envs-per-gpu 65536]
+                    [--dump-outputs DIR]
 
 A "step" is one `so100_step` launch over every env of this rank: pre-step task logic, 16 physics substeps,
 obs / reward / termination / TimeLimit and in-kernel auto-reset.  Inputs (actions) are resident in HBM when the timed
 region starts; `e2e` repeats the measurement through the host-buffer C-ABI call (pinned host actions in, host
 obs / reward / done out, copies inside the timed region).  Rank 0 prints ONE JSON line.
+
+`--dump-outputs DIR` writes what the last timed step returned (see `dump_outputs`).  The inputs depend on the
+arguments only, so two builds run with the same arguments can be compared output for output.  bench.py writes nothing
+into the source tree (which may be read-only): the CPU leg's -march=native oracle is compiled into the temp directory.
 
 `--impl reference`: the reference's CPU path.  MuJoCo is not installable in this image (no wheel, no network), so the
 timed engine is the repo's fp64 C oracle (kind "port") on all host cores, on a bounded sample of the same workload.
@@ -24,6 +29,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # no __pycache__ in the source tree either
 
 # Algorithmic work per env step (DESIGN.md "Roofline arithmetic"; tools/count_flops.cpp counts the generic recursion with
 # the shipped sweep schedule: 5 Gauss-Seidel sweeps on the first substep of an env step, 3 on the other 15)
@@ -49,7 +55,12 @@ def parse():
     ap.add_argument("--no-ppo", action="store_true", help="skip the Env05 PPO record (BASELINE config 5)")
     ap.add_argument("--no-contact", action="store_true", help="skip the record of the opt-in arm-floor contact physics (SO100_FLAG_ARM_CONTACT)")
     ap.add_argument("--flags", type=int, default=0, help="SO100_FLAG_* bits for the env (e.g. 16 = no arm-floor contact)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the arrays the last timed step returned as DIR/<name>.npy (float32 / float64, at most 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def workload(args) -> str:
@@ -201,8 +212,10 @@ def run_reference(args, rank: int):
         o.step(acts[w % 8], nthreads=threads)
     t0 = time.perf_counter()
     for k in range(args.steps):
-        o.step(acts[k % 8], nthreads=threads)
+        out = o.step(acts[k % 8], nthreads=threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(STEP_OUTPUTS, out)))
     value = n * args.steps / dt
     sample = f"{n} envs x {args.steps} steps of the {args.envs_per_gpu}-env workload, fp64 C oracle{' -O3 -march=native' if native else ''} (MuJoCo not installable here), {threads} threads"
     line = {
@@ -225,6 +238,38 @@ def emit(line: dict):
 # libraries (NCCL prints its version banner) write to fd 1: keep the real stdout aside and point fd 1 at stderr
 _REAL_STDOUT = os.dup(1)
 os.dup2(2, 1)
+
+DUMP_BUDGET_BYTES = 64_000_000  # all ranks' files together, .npy headers included
+
+
+def dump_outputs(out_dir: str, outputs: dict, rank: int = 0, world: int = 1):
+    """Writes one step's outputs (name -> array with one row per env of this rank) as out_dir/<name>.npy: float64 stays
+    float64, everything else becomes float32 (flags and episode lengths are small integers, exact in float32).
+    terminal_obs / ep_return / ep_len are only defined where the episode ended in that step; their other rows hold
+    whatever an earlier step left there and are written as 0.  With several ranks each writes its own env shard with a
+    _rank<r> suffix.  When a rank's arrays exceed its share of DUMP_BUDGET_BYTES, the same fixed, seeded sample of env rows is kept
+    in every array, in env order, and env_index<suffix>.npy lists the (local) rows kept."""
+    import numpy as np
+    arrays = {k: np.asarray(v) for k, v in outputs.items()}
+    arrays = {k: v.astype(np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    ended = (arrays["terminated"] + arrays["truncated"]) > 0
+    for k in ("terminal_obs", "ep_return", "ep_len"):
+        arrays[k][~ended] = 0
+    n = len(ended)
+    row_bytes = sum(v[:1].nbytes for v in arrays.values())
+    keep = min(n, (DUMP_BUDGET_BYTES // world - 4096) // (row_bytes + 8))  # 4 KiB: the headers; 8 B: env_index
+    if keep < n:
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["env_index"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}{suffix}.npy"), v)
+
+
+# what one env step returns, in the order of `Oracle.step`'s tuple and of the fields of a StepResult
+STEP_OUTPUTS = ("obs", "reward", "terminated", "truncated", "terminal_obs", "ep_return", "ep_len")
 
 
 def profile_lookup(task: int, n: int, build_id: str):
@@ -366,6 +411,8 @@ def main():
     total_ms = sum(a.elapsed_time(b) for a, b in ev)
     launches = env.stats()["launches"] - launches0
     stats = env.stats()
+    if args.dump_outputs:  # before the e2e legs step this env further
+        dump_outputs(args.dump_outputs, {k: getattr(res[-1], k).cpu().numpy() for k in STEP_OUTPUTS}, rank, world)
 
     # ---- end to end through the host-buffer C ABI (host actions in, host obs / reward / flags out, every step)
     e2e = None

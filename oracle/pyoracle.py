@@ -54,20 +54,33 @@ _lib = None
 
 def _native_build() -> str | None:
     """-O3 -march=native build for the TIMED CPU legs of bench.py (BASELINE.md §3), compiled on the machine it runs on
-    (the checker itself stays -O2 -ffp-contract=off so that the committed fixtures reproduce bit for bit)."""
+    (the portable oracle build that the tests use stays -O2 -ffp-contract=off so that the committed fixtures reproduce bit
+    for bit).
+    The library goes to a private directory under the temp directory, named after the host's CPU flags and the
+    oracle's sources, so that the source tree is never written and may be read-only."""
     import hashlib
+    import tempfile
     try:
         cpu = next(ln for ln in open("/proc/cpuinfo") if ln.startswith("flags"))
     except Exception:  # noqa: BLE001
         cpu = "unknown"
-    out = os.path.join(_HERE, f"libso100_oracle_native_{hashlib.sha1(cpu.encode()).hexdigest()[:10]}.so")
     src = os.path.join(_HERE, "so100_oracle.c")
-    if not os.path.exists(out) or os.path.getmtime(out) < os.path.getmtime(src):
-        try:
+    h = hashlib.sha1(cpu.encode())
+    for f in (src, os.path.join(_HERE, "so100_oracle.h")):
+        h.update(open(f, "rb").read())
+    d = os.path.join(tempfile.gettempdir(), f"so100_oracle_{os.getuid()}")
+    out = os.path.join(d, f"libso100_oracle_native_{h.hexdigest()[:12]}.so")
+    try:
+        os.makedirs(d, mode=0o700, exist_ok=True)
+        if os.stat(d).st_uid != os.getuid():
+            return None  # someone else's directory: do not load a library from it
+        if not os.path.exists(out):
+            tmp = f"{out}.{os.getpid()}"
             subprocess.check_call(["gcc", "-O3", "-march=native", "-pthread", "-fPIC", "-std=c11", "-D_GNU_SOURCE", "-shared",
-                                   "-o", out, src, "-lm"], stderr=subprocess.DEVNULL)
-        except Exception:  # noqa: BLE001 - no compiler on this host: time the portable build instead
-            return None
+                                   "-o", tmp, src, "-lm"], stderr=subprocess.DEVNULL)
+            os.replace(tmp, out)  # atomic: a concurrent process never loads a half-written file
+    except Exception:  # noqa: BLE001 - no compiler or no writable temp directory: time the portable build instead
+        return None
     return out
 
 

@@ -1,8 +1,11 @@
 """MJCF reader: the committed mesh-free scene carries the reference's numbers (SURVEY.md Appendix A)."""
+import os
+
 import numpy as np
 import pytest
 
-from so100_mujoco_rl_b200.model import euler_to_quat, load_model, quat_to_mat, reference_scene_path
+from conftest import ROOT
+from so100_mujoco_rl_b200.model import euler_to_quat, load_model, quat_to_mat
 
 
 def test_chain_constants(spec):
@@ -27,14 +30,14 @@ def test_euler_is_intrinsic_xyz():
     assert np.allclose(quat_to_mat(q), Rx @ Ry @ Rz, atol=1e-14)
 
 
-@pytest.mark.skipif(reference_scene_path() is None, reason="reference checkout not mounted (never on the GPU box)")
 def test_asset_equals_reference_mjcf(spec):
-    ref = load_model(reference_scene_path())
+    """tests/golden/ref_mjcf.npz: the reference's env01.xml as load_model reads it (tools/gen_golden_from_reference.py)."""
+    ref = np.load(os.path.join(ROOT, "tests", "golden", "ref_mjcf.npz"))
     for f in ("body_pos", "body_quat", "body_ipos", "body_iquat", "body_mass", "body_inertia", "jnt_axis", "jnt_range",
               "jnt_armature", "jnt_frictionloss", "act_kp", "act_dampratio", "act_ctrlrange", "act_forcerange",
               "cam_pos", "cam_quat", "ee_offset", "gravity"):
-        assert np.array_equal(getattr(spec, f), getattr(ref, f)), f
-    assert spec.cam_fovy_deg == ref.cam_fovy_deg and spec.timestep == ref.timestep
+        assert np.array_equal(getattr(spec, f), ref[f]), f
+    assert spec.cam_fovy_deg == ref["cam_fovy_deg"] and spec.timestep == ref["timestep"]
 
 
 def test_unsupported_models_are_rejected(tmp_path, spec):

@@ -1,5 +1,6 @@
 #!/usr/bin/env python
-"""Generates tests/golden/ref_env0{1,2,5,6}.npz by running the REFERENCE'S OWN Python task logic, unmodified.
+"""Generates tests/golden/ref_env0{1,2,5,6}.npz by running the REFERENCE'S OWN Python task logic, unmodified, and
+tests/golden/ref_mjcf.npz, the reference's scene as the MJCF reader parses it.
 
 Runs only in the build container (it imports from /root/reference); the fixtures travel, this script's inputs do not.
 
@@ -297,11 +298,18 @@ def rollout(task, n_envs, steps, seed, max_episode_steps, action_seed):
                 seed=np.int64(seed), max_episode_steps=np.int64(max_episode_steps), task=np.int64(task))
 
 
+MJCF_FIELDS = ("body_pos", "body_quat", "body_ipos", "body_iquat", "body_mass", "body_inertia", "jnt_axis", "jnt_range",
+               "jnt_armature", "jnt_frictionloss", "act_kp", "act_dampratio", "act_ctrlrange", "act_forcerange",
+               "cam_pos", "cam_quat", "ee_offset", "gravity", "cam_fovy_deg", "timestep")
+
+
 def main():
     _install_stubs()
     sys.path.insert(0, REF_SRC)
     out = os.path.join(ROOT, "tests", "golden")
     os.makedirs(out, exist_ok=True)
+    # the reference's MJCF as load_model reads it: tests/test_model.py checks the committed mesh-free scene against it
+    np.savez_compressed(os.path.join(out, "ref_mjcf.npz"), **{f: np.asarray(getattr(SPEC, f)) for f in MJCF_FIELDS})
     for task, n, steps, limit in ((1, 6, 90, 40), (2, 6, 90, 35), (5, 8, 140, 100), (6, 6, 90, 35)):
         d = rollout(task, n, steps, seed=1234 + task, max_episode_steps=limit, action_seed=task)
         path = os.path.join(out, f"ref_env0{task}.npz")
