@@ -358,7 +358,10 @@ __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs&
     // much as a resting contact penetrates (~2e-7 m) - so it asks with a margin, and the contact path redoes its own
     // kinematics with sincosf of the compensated angle: without that, resting contacts flicker on and off from substep to
     // substep (measured: p99.9 |dq| 9e-4 rad against the oracle instead of 3e-7, tools/contact_precision.py).
-    const unsigned touch = PADS && C.pad.n > 0 ? pads_touch<float>(C.dyn, C.kin, C.pad, s, c, SO100_TOUCH_MARGIN) : 0u;
+    // A tail thread (!live, shadowing the launch's last env) never touches: it asks for no pool slot, so that a touching
+    // last env cannot fill its CTA's pool with copies of itself and push the CTA's real touching envs to the serial solve.
+    unsigned touch = PADS && C.pad.n > 0 ? pads_touch<float>(C.dyn, C.kin, C.pad, s, c, SO100_TOUCH_MARGIN) : 0u;
+    if (!live) touch = 0u;
     if (PADS && sub == nsub - 1) e.flags = touch ? (e.flags | F_TOUCH) : (e.flags & ~F_TOUCH);
     float d = 0.0f;
     bool solved = false;
