@@ -317,6 +317,36 @@ int so100_host_constants(const so100_model *model, double *out /*[141]*/);
 #define SO100_N_SOLVER_CONSTANTS 146
 int so100_host_solver_constants(const so100_model *model, float *out, int n_out /* = SO100_N_SOLVER_CONSTANTS */);
 
+/*
+ * Per-env dynamics randomisation.  Opt-in: until ranges are set every env runs on the model's constants.  Once set, each
+ * env holds its own fp32 servo gain kp, damping kv, forcerange and joint friction loss (30 floats per env; at the first
+ * call every env starts from the ctx's constants) and redraws them at every episode reset: the auto-reset in so100_step*
+ * (termination, truncation, non-finite state) and so100_reset (masked or not); nothing else redraws them.  Draws are
+ * keyed by (seed, env_offset + env, tick): results do not depend on sharding, env groups or the host path.  With scales
+ *   s = lo + (hi - lo) u,  u uniform in [0, 1):   kp = kp0 s_kp,  kv = kv0 sqrt(s_kp) s_damping,
+ *   forcerange = forcerange0 s_force (both ends),  frictionloss = frictionloss0 s_frictionloss
+ * where kp0, ... are the model's fp32 constants; s_damping is the damping ratio relative to the model's.  [1, 1] leaves a
+ * parameter at the model's value bit for bit.  Env i then steps bit for bit like env i of a ctx whose model carries its
+ * values (act_dampratio = 0, act_kv = kv).  Link masses, inertias and armature are not randomised.
+ */
+typedef struct so100_param_ranges {   /* scale ranges [lo, hi] per joint; lo == hi == 1 leaves a parameter at the model's value */
+  int32_t struct_size, _pad0;         /* = sizeof(so100_param_ranges) */
+  double kp[SO100_NJ][2];             /* kp = model kp x U, lo > 0 */
+  double damping[SO100_NJ][2];        /* kv = model kv x sqrt(kp scale) x U (damping ratio relative to the model's), lo >= 0 */
+  double forcerange[SO100_NJ][2];     /* both ends of the model's forcerange x U, lo > 0 */
+  double frictionloss[SO100_NJ][2];   /* model frictionloss x U, lo >= 0 */
+} so100_param_ranges;
+/* DEVICE pointers to [6][N] fp32 arrays (SoA, [joint][env]); NULL = skip the field */
+typedef struct so100_param_view { float *kp, *kv, *force_lo, *force_hi, *frictionloss; } so100_param_view;
+
+/* ranges == NULL: off, back to the model's constants and the default kernels.  A change of ranges applies from each env's
+   next reset.  Synchronous. */
+int so100_set_param_ranges(so100_ctx *ctx, const so100_param_ranges *ranges);
+/* Read / overwrite the per-env values (SO100_ERR_STATE while ranges are off); written values hold until the env's next
+   reset.  All three calls return SO100_ERR_STATE while an asynchronous group step is in flight. */
+int so100_get_env_params(so100_ctx *ctx, const so100_param_view *view, void *stream);
+int so100_set_env_params(so100_ctx *ctx, const so100_param_view *view, void *stream);
+
 /* Which step kernel this ctx launches: 0 = generic (constants at run time), 1 = specialised to the baked so100 model. */
 int so100_kernel_variant(so100_ctx *ctx);
 

@@ -17,6 +17,7 @@ import torch
 
 from . import _native
 from .model import ModelSpec, load_model
+from .randomization import PARAM_NAMES, ParamRanges, So100ParamView
 from .tasks import MAX_EPISODE_STEPS, OBS_DIM, make_task_cfg, task_id
 
 NJ = 6
@@ -56,7 +57,7 @@ def _host_ptrs(host: dict, with_terminal: bool) -> tuple:
 class BatchedSo100Env:
     def __init__(self, env: str | int, num_envs: int, device: int | str | torch.device = 0, seed: int = 0,
                  env_offset: int = 0, flags: int = 0, model: ModelSpec | None = None,
-                 max_episode_steps: int | None = None):
+                 max_episode_steps: int | None = None, param_ranges: ParamRanges | None = None):
         self.task = task_id(env)
         self.num_envs = int(num_envs)
         self.obs_dim = OBS_DIM[self.task]
@@ -87,6 +88,9 @@ class BatchedSo100Env:
         self.terminal_obs = torch.zeros((n, od), **f32)
         self.ep_return = torch.zeros(n, **f32)
         self.ep_len = torch.zeros(n, dtype=torch.int32, device=self.device)
+        self.param_ranges: ParamRanges | None = None
+        if param_ranges is not None:
+            self.set_param_ranges(param_ranges)
 
     # ---- lifecycle
     def close(self):
@@ -231,6 +235,37 @@ class BatchedSo100Env:
             keep.append(t)
             setattr(view, name, t.data_ptr())
         _native.check(self._L.so100_set_state(self._h, ctypes.byref(view), self._stream()))
+        torch.cuda.current_stream(self.device).synchronize()
+
+    # ---- per-env dynamics randomisation (randomization.py; include/so100_b200.h, so100_set_param_ranges)
+    def set_param_ranges(self, ranges: ParamRanges | None) -> None:
+        """Redraw kp, kv, forcerange and friction loss of every env at each of its episode resets from these scale ranges;
+        None switches back to the model's constants.  The first call starts every env from the model's values; a later
+        change of ranges applies from each env's next reset."""
+        if ranges is None:
+            _native.check(self._L.so100_set_param_ranges(self._h, None))
+        else:
+            r = ranges.to_ctypes()
+            _native.check(self._L.so100_set_param_ranges(self._h, ctypes.byref(r)))
+        self.param_ranges = ranges
+
+    def get_params(self) -> dict:
+        """Every env's current values: {kp, kv, force_lo, force_hi, frictionloss} -> float32 [6, N] copies."""
+        out = {k: torch.zeros((NJ, self.num_envs), dtype=torch.float32, device=self.device) for k in PARAM_NAMES}
+        view = So100ParamView(*(out[k].data_ptr() for k in PARAM_NAMES))
+        _native.check(self._L.so100_get_env_params(self._h, ctypes.byref(view), self._stream()))
+        return out
+
+    def set_params(self, params: dict) -> None:
+        """Overwrite some or all of the per-env values ([6, N] each); they hold until each env's next reset."""
+        view, keep = So100ParamView(), []
+        for name, t in params.items():
+            if name not in PARAM_NAMES:
+                raise KeyError(f"unknown parameter {name!r}; expected one of {PARAM_NAMES}")
+            t = t.to(device=self.device, dtype=torch.float32).reshape(NJ, self.num_envs).contiguous()
+            keep.append(t)
+            setattr(view, name, t.data_ptr())
+        _native.check(self._L.so100_set_env_params(self._h, ctypes.byref(view), self._stream()))
         torch.cuda.current_stream(self.device).synchronize()
 
     @property

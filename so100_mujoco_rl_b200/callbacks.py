@@ -96,6 +96,9 @@ class TrainCallbacks:
         env = getattr(self.learner, "env", None)
         if env is not None and hasattr(env, "get_state") and hasattr(env, "tick"):  # simulator state: the resumed run continues the same episodes
             ckpt["env"] = {"state": {k: v.cpu() for k, v in env.get_state().items()}, "tick": env.tick, "num_envs": env.num_envs}
+            ranges = getattr(env, "param_ranges", None)  # per-env dynamics (randomization.py): resumed with the same values
+            ckpt["env"]["param_ranges"] = ranges.to_dict() if ranges is not None else None
+            ckpt["env"]["params"] = {k: v.cpu() for k, v in env.get_params().items()} if ranges is not None else None
         torch.save(ckpt, base + ".pt")
         export_sb3_zip(base + ".zip", pol.state_dict_sb3(), {"num_timesteps": self.learner.stats.samples})
         return base

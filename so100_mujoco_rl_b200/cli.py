@@ -43,18 +43,29 @@ def cli(ctx, algorithm, model_path):
 @click.option("--eval-steps", default=0, show_default=True, help="env steps per evaluation (0 = the task's TimeLimit: one full episode per env)")
 @click.option("--save-freq", default=4_000_000, show_default=True, help="samples between checkpoints (main.py:228 uses 40000 for its single env)")
 @click.option("--tensorboard-log", default="logs", show_default=True, help="TensorBoard folder (main.py:30, :62); empty = off")
+@click.option("--randomize", "randomize", default=None,
+              help="per-env dynamics randomisation of the training simulator, redrawn at every episode reset, e.g. "
+                   "'kp=0.7:1.3,damping=0.8:1.2,forcerange=0.8:1.0,frictionloss=0.5:2' (scales of the model's values); "
+                   "evaluation stays on the model's dynamics")
 @click.pass_context
 def train(ctx, environment, num_envs, device, trainer, total_timesteps, n_steps, seed, out, learner_kind, eval_freq, eval_envs,
-          eval_steps, save_freq, tensorboard_log):
+          eval_steps, save_freq, tensorboard_log, randomize):
     algo = ctx.obj["ALGORITHM_NAME"]
     if trainer != "sb3" and algo != "PPO":  # refuse before anything is created on disk
         raise click.UsageError("the native trainer implements PPO; use --trainer sb3 for other algorithms")
+    ranges = None
+    if randomize:
+        from .randomization import ParamRanges
+        try:
+            ranges = ParamRanges.parse(randomize)
+        except ValueError as e:
+            raise click.BadParameter(str(e), param_hint="--randomize") from None
     folder = os.path.join(out, f"{environment}_{algo}")
     os.makedirs(folder, exist_ok=True)
     if trainer == "sb3":
         import stable_baselines3  # noqa: F401  (as main.py:258-262 validates the algorithm name)
         from .vec_env import So100VecEnv
-        env = So100VecEnv(environment, num_envs, device=device, seed=seed)
+        env = So100VecEnv(environment, num_envs, device=device, seed=seed, param_ranges=ranges)
         cls = getattr(stable_baselines3, algo)
         model = cls("MlpPolicy", env, device="cpu", n_steps=n_steps, verbose=1) if not ctx.obj["MODEL_PATH"] else cls.load(ctx.obj["MODEL_PATH"], env=env)
         model.learn(total_timesteps=total_timesteps)
@@ -64,7 +75,7 @@ def train(ctx, environment, num_envs, device, trainer, total_timesteps, n_steps,
     from .batched_env import BatchedSo100Env
     from .callbacks import TrainCallbacks
     from .ppo import PPO, FusedPPO, PPOConfig
-    env = BatchedSo100Env(environment, num_envs, device=device, seed=seed)
+    env = BatchedSo100Env(environment, num_envs, device=device, seed=seed, param_ranges=ranges)
     cfg = PPOConfig(n_steps=n_steps, seed=seed)
     learner = FusedPPO(env, cfg) if learner_kind == "fused" else PPO(env, cfg)
     if ctx.obj["MODEL_PATH"]:  # main.py:201-207: continue from a saved model (weights; a .pt also restores Adam and the counters)
@@ -80,6 +91,11 @@ def train(ctx, environment, num_envs, device, trainer, total_timesteps, n_steps,
         es = ckpt.get("env")
         if es is not None and es.get("num_envs") == env.num_envs:
             env.set_state(es["state"]); env.tick = int(es["tick"])
+            if es.get("params") is not None:  # the same per-env dynamics as when it was saved (and its ranges unless --randomize is given)
+                if env.param_ranges is None:
+                    from .randomization import ParamRanges
+                    env.set_param_ranges(ParamRanges.from_dict(es["param_ranges"]))
+                env.set_params(es["params"])
             learner.obs = env.obs   # (stale by one step at most: refreshed by the first env.step of the next rollout)
         else:
             env.seed(seed + 1_000_003)

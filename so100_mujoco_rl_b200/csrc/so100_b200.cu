@@ -57,7 +57,8 @@ constexpr int kMaxStart = SO100_MAX_START;
 constexpr int kSnap = 12, kAux = 24, kCnt = 4;
 enum { F_EVER_STEPPED = 1, F_HAS_LAST_BLOCK = 2, F_ANGVEL_VALID = 4, F_CENTRE_VALID = 8,
        F_TOUCH = 16 };  // F_TOUCH: a jaw pad touched the floor in the env's last substep (scheduling hint only, no effect on results)
-enum { STREAM_RESET = 0, STREAM_TASK = 1, STREAM_NOISE = 2, STREAM_API_RESET = 3, STREAM_RESET_NOISE = 4 };
+enum { STREAM_RESET = 0, STREAM_TASK = 1, STREAM_NOISE = 2, STREAM_API_RESET = 3, STREAM_RESET_NOISE = 4,
+       STREAM_PARAM_RESET = 8, STREAM_PARAM_API_RESET = 16 };  // per-env parameters: streams 8..13 (auto-reset) and 16..21 (so100_reset)
 
 struct TaskC {
   int task, n, max_steps, n_start, lost_limit, nsub;
@@ -87,6 +88,15 @@ struct Bufs {
   int* cnt;
   const float* start_tab;  // [n_start][6]
   unsigned long long* stats;  // [0] solver non-converged, [1] nan resets, [2] contact solves that dropped corners (> SO_MAX_CON)
+};
+
+// Per-env dynamics parameters (so100_set_param_ranges), drawn at every episode reset.  p: [kParams][n] device array,
+// rows kp[6], kv[6], force_lo[6], force_hi[6], frictionloss[6]; nullptr while ranges are off.  lo / hi: fp32 scale
+// ranges in draw order, kp[6], damping[6], forcerange[6], frictionloss[6].
+constexpr int kParams = 5 * SO_NJ, kParamDraws = 4 * SO_NJ;
+struct ParamIO {
+  float* p;
+  float lo[kParamDraws], hi[kParamDraws];
 };
 
 struct StepIO {
@@ -265,6 +275,30 @@ __device__ __forceinline__ void reset_env(const Consts& C, const Bufs& B, EnvReg
   write_obs<TASK>(t, e, env, tick, STREAM_RESET_NOISE, obs);
 }
 
+// Draws env `env`'s dynamics parameters: 6 Philox blocks on streams stream..stream+5 give 24 uniforms in draw order;
+// scale s = lo + (hi - lo) u; kp = kp0 s_kp, kv = kv0 sqrt(s_kp) s_d, force = force0 s_f, frictionloss = loss0 s_fl, from the
+// ctx's fp32 constants, every operation rounded on its own (no contraction), so that the host reproduces the bits.
+__device__ __forceinline__ void draw_params(const Consts& C, const ParamIO& P, int env, unsigned tick, unsigned stream) {
+  const TaskC& t = C.t;
+  const int n = t.n;
+  float s[kParamDraws];
+#pragma unroll
+  for (int k = 0; k < kParamDraws / 4; k++) {
+    const uint4 r = draw(t, env, tick, stream + k);
+    const unsigned x[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+    for (int m = 0; m < 4; m++) s[4 * k + m] = __fadd_rn(P.lo[4 * k + m], __fmul_rn(__fsub_rn(P.hi[4 * k + m], P.lo[4 * k + m]), u01(x[m])));
+  }
+#pragma unroll
+  for (int j = 0; j < SO_NJ; j++) {
+    P.p[j * n + env] = __fmul_rn(t.act.kp[j], s[j]);
+    P.p[(SO_NJ + j) * n + env] = __fmul_rn(__fmul_rn(t.act.kv[j], sqrtf(s[j])), s[SO_NJ + j]);
+    P.p[(2 * SO_NJ + j) * n + env] = __fmul_rn(t.act.frc_lo[j], s[2 * SO_NJ + j]);
+    P.p[(3 * SO_NJ + j) * n + env] = __fmul_rn(t.act.frc_hi[j], s[2 * SO_NJ + j]);
+    P.p[(4 * SO_NJ + j) * n + env] = __fmul_rn(C.con.fr_loss[j], s[3 * SO_NJ + j]);
+  }
+}
+
 __device__ __forceinline__ float joint_penalty(const TaskC& t, const float* ang) {  // env_base_01.py:144-163
   float r = 0.0f;
 #pragma unroll
@@ -311,9 +345,11 @@ constexpr size_t kPoolBytes = (size_t)kPoolSlots * (CoopSlot::kDoubles * 8 + Coo
 // 16 x mj_step on the arm.  ctrl is constant over the env step, so kp*clip(ctrl) is hoisted.
 // ctrl is carried as an unevaluated sum ctrl_hi + ctrl_lo so that Env01/02's closed loop ctrl = qpos + a*0.075 does not
 // round the 0.075-rad increment to the ulp of a 3-rad angle (that rounding random-walks qpos in a neutrally stable loop).
-template <int TASK, bool SPEC, bool PADS>
+// PARAMS: the env's own kp, kv, forcerange and friction loss (ParamIO; pv = p + env, rows n apart) replace the model's,
+// read once and held in registers over the substeps; every other constant stays the model's.
+template <int TASK, bool SPEC, bool PADS, bool PARAMS>
 __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs& e, const float* ctrl_hi, const float* ctrl_lo, bool live, int nsub,
-                                        const ContactPool& pool) {
+                                        const ContactPool& pool, const float* pv) {
   const TaskC& t = C.t;
   // SPEC: the solver / servo constants of the so100 MJCF are literals (immediates after unrolling), not constant-bank loads
   ConC<float> Kg;
@@ -324,6 +360,15 @@ __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs&
   const ActC<float>& A = SPEC ? Ag : t.act;
   const BlkC<float>& Kb = SPEC ? Bg : t.blk;
   const bool block_moves = TASK != 5 && !(t.flags & SO100_FLAG_STATIC_BLOCK);  // Env05 scripts its block (env03_v1.py:95-122)
+  float pkp[SO_NJ], pkv[SO_NJ], pflo[SO_NJ], pfhi[SO_NJ], ploss[SO_NJ];
+  if (PARAMS) {
+#pragma unroll
+    for (int j = 0; j < SO_NJ; j++) {
+      pkp[j] = pv[j * t.n]; pkv[j] = pv[(SO_NJ + j) * t.n]; pflo[j] = pv[(2 * SO_NJ + j) * t.n];
+      pfhi[j] = pv[(3 * SO_NJ + j) * t.n]; ploss[j] = pv[(4 * SO_NJ + j) * t.n];
+    }
+  }
+  const float* loss = PARAMS ? ploss : K.fr_loss;
   float cc[SO_NJ], cl[SO_NJ];
 #pragma unroll
   for (int j = 0; j < SO_NJ; j++) {
@@ -345,8 +390,8 @@ __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs&
     else dyn_bias_mass<float>(C.dyn, s, c, e.v, bias, M);       // any other model: constants from the ctx
 #pragma unroll
     for (int j = 0; j < SO_NJ; j++) {
-      float f = A.kp[j] * ((cc[j] - e.q[j]) + (cl[j] + e.qc[j])) - A.kv[j] * e.v[j];  // differences first: no cancellation
-      b[j] = clampf(f, A.frc_lo[j], A.frc_hi[j]) - bias[j];
+      float f = (PARAMS ? pkp[j] : A.kp[j]) * ((cc[j] - e.q[j]) + (cl[j] + e.qc[j])) - (PARAMS ? pkv[j] : A.kv[j]) * e.v[j];  // differences first: no cancellation
+      b[j] = clampf(f, PARAMS ? pflo[j] : A.frc_lo[j], PARAMS ? pfhi[j] : A.frc_hi[j]) - bias[j];
     }
     // ctrl changes once per env step, so the first substep's warm start is far: 5 sweeps (each contracts the error
     // ~100x); afterwards qacc moves a few % per substep: 3 sweeps.  The solver adds per-lane sweeps if the last one
@@ -389,7 +434,7 @@ __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs&
           }
           bool serial = slot >= pool.nslot;  // pool exhausted (> kPoolSlots touching envs in this CTA)
           if (!serial) {
-            const int nc = coop_fill(C.dyn, C.kin, C.pad, C.con, pool.slot(slot), cs, cc_, e.q, e.qc, e.v, M, b, e.w, touch);
+            const int nc = coop_fill(C.dyn, C.kin, C.pad, C.con, PARAMS ? ploss : C.con.fr_loss, pool.slot(slot), cs, cc_, e.q, e.qc, e.v, M, b, e.w, touch);
             serial = nc < 0;            // > kCoopCon corners at once
             if (nc > 0) myslot = slot;  // nc == 0: the accurate kinematics found no corner below the floor after all
           }
@@ -400,7 +445,13 @@ __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs&
 #pragma unroll
             for (int k = 0; k < 21; k++) cio.M[k] = M[k];
             int over = 0;
-            int st = contact_solve<float>(C.dyn, C.kin, C.pad, C.con, cio, touch, &over);
+            int st;
+            if (PARAMS) {
+              float lc[SO_NJ];  // a copy for the out-of-line call: ploss itself stays in registers
+#pragma unroll
+              for (int j = 0; j < SO_NJ; j++) lc[j] = ploss[j];
+              st = contact_solve_loss<float>(C.dyn, C.kin, C.pad, C.con, lc, cio, touch, &over);
+            } else st = contact_solve<float>(C.dyn, C.kin, C.pad, C.con, cio, touch, &over);
             if (over && live) atomicAdd(&B.stats[2], 1ULL);
             if (st != 0 && !over) {
 #pragma unroll
@@ -414,7 +465,7 @@ __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs&
       }
       // every other env: the per-dof Gauss-Seidel, BEFORE the cooperative phase, so that M and b are dead across it
       if (!solved && myslot < 0) {
-        d = solve_qacc<float>(K, M, b, e.q, e.qc, e.v, e.w, sub == 0 ? SO100_SWEEPS_FIRST : SO100_SWEEPS_REST);
+        d = solve_qacc<float>(K, loss, M, b, e.q, e.qc, e.v, e.w, sub == 0 ? SO100_SWEEPS_FIRST : SO100_SWEEPS_REST);
         solved = true;
       }
       // Phase B, the whole CTA: groups of kCoopLanes threads run the Newton solves of the filled slots.  Consecutive slots
@@ -445,7 +496,7 @@ __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs&
         }
       }
     }
-    if (!PADS) d = solve_qacc<float>(K, M, b, e.q, e.qc, e.v, e.w, sub == 0 ? SO100_SWEEPS_FIRST : SO100_SWEEPS_REST);
+    if (!PADS) d = solve_qacc<float>(K, loss, M, b, e.q, e.qc, e.v, e.w, sub == 0 ? SO100_SWEEPS_FIRST : SO100_SWEEPS_REST);
     float amax = 1.0f;
 #pragma unroll
     for (int j = 0; j < SO_NJ; j++) {
@@ -464,8 +515,9 @@ __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs&
 }
 
 // ------------------------------------------------------------------------------------------------ kernels
-template <int TASK, bool SPEC, bool PADS>
-__global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) step_kernel(const __grid_constant__ Consts C, const Bufs B, const StepIO io) {
+template <int TASK, bool SPEC, bool PADS, bool PARAMS>
+__global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) step_kernel(const __grid_constant__ Consts C, const Bufs B, const StepIO io,
+                                                                        const __grid_constant__ ParamIO par) {
   constexpr int OD = TASK == 5 ? 8 : 15;
   __shared__ __align__(16) float sh[kBlock * OD];
   static_assert((kBlock * OD) % 4 == 0, "obs rows of a CTA must be a whole number of float4");
@@ -567,7 +619,7 @@ __global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) step_kernel(const __g
           for (int k = 0; k < 3; k++) e.aux[k] = e.blk[k];
         }
       }
-      physics<TASK, SPEC, PADS>(C, B, e, ctrl, ctrl_lo, live, t.nsub, pool);
+      physics<TASK, SPEC, PADS, PARAMS>(C, B, e, ctrl, ctrl_lo, live, t.nsub, pool, PARAMS ? par.p + i : nullptr);
       write_obs<TASK>(t, e, i, tick, STREAM_NOISE, obs);
     } else {  // env03_v1.py:124-201
       float time = (float)e.elapsed * t.dt_env;
@@ -598,7 +650,7 @@ __global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) step_kernel(const __g
       float newcmd[SO_NJ];
 #pragma unroll
       for (int j = 0; j < SO_NJ; j++) { newcmd[j] = e.aux[j] + a[j] * t.step_scale; ctrl[j] = newcmd[j]; ctrl_lo[j] = 0.0f; }  // open loop (Q6)
-      physics<TASK, SPEC, PADS>(C, B, e, ctrl, ctrl_lo, live, t.nsub, pool);
+      physics<TASK, SPEC, PADS, PARAMS>(C, B, e, ctrl, ctrl_lo, live, t.nsub, pool, PARAMS ? par.p + i : nullptr);
       write_obs<TASK>(t, e, i, tick, STREAM_NOISE, obs);
       if (obs[6] == -1.0f && obs[7] == -1.0f) {  // :152-164
         if (e.miss > t.lost_limit) term = true;
@@ -649,6 +701,7 @@ __global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) step_kernel(const __g
       if (live && io.ep_len_out) io.ep_len_out[i] = e.elapsed;
       if (live && io.any_done) *io.any_done = 1;
       reset_env<TASK>(C, B, e, i, tick, STREAM_RESET, obs);
+      if (PARAMS && live) draw_params(C, par, i, tick, STREAM_PARAM_RESET);
       if (live && io.terminal_obs && bad) {
 #pragma unroll
         for (int k = 0; k < OD; k++) io.terminal_obs[(size_t)i * OD + k] = obs[k];
@@ -674,7 +727,8 @@ __global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) step_kernel(const __g
 }
 
 template <int TASK>
-__global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ Consts C, const Bufs B, const uint8_t* mask, float* obs_out, unsigned tick) {
+__global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ Consts C, const Bufs B, const uint8_t* mask, float* obs_out, unsigned tick,
+                                                       const __grid_constant__ ParamIO par) {
   constexpr int OD = TASK == 5 ? 8 : 15;
   const int n = C.t.n, i = blockIdx.x * kBlock + threadIdx.x;
   if (i >= n || (mask && !mask[i])) return;
@@ -682,6 +736,7 @@ __global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ C
   load_env<TASK>(B, n, i, e);
   float obs[OD];
   reset_env<TASK>(C, B, e, i, tick, STREAM_API_RESET, obs);
+  if (par.p) draw_params(C, par, i, tick, STREAM_PARAM_API_RESET);
   store_env<TASK>(B, n, i, e);
 #pragma unroll
   for (int k = 0; k < OD; k++) obs_out[(size_t)i * OD + k] = obs[k];
@@ -689,8 +744,9 @@ __global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ C
 
 // debug / parity triage: n x mj_step under a given ctrl, no task logic (no reward / obs / counters / reset); the snapshot
 // is refreshed with the kinematics of the last substep's start state, as in a full env step
-template <int TASK, bool SPEC>
-__global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) substeps_kernel(const __grid_constant__ Consts C, const Bufs B, const float* ctrl, int nsub) {
+template <int TASK, bool SPEC, bool PARAMS>
+__global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) substeps_kernel(const __grid_constant__ Consts C, const Bufs B, const float* ctrl, int nsub,
+                                                                           const float* par) {
   const int n = C.t.n, base = blockIdx.x * kBlock;
   const bool live = base + (int)threadIdx.x < n;
   const int i = live ? base + (int)threadIdx.x : n - 1;  // tail threads shadow the last env (physics has CTA barriers)
@@ -699,7 +755,7 @@ __global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) substeps_kernel(const
   float ch[SO_NJ], cl[SO_NJ];
 #pragma unroll
   for (int j = 0; j < SO_NJ; j++) { ch[j] = ctrl[(size_t)i * SO_NJ + j]; cl[j] = 0.0f; }
-  physics<TASK, SPEC, true>(C, B, e, ch, cl, live, nsub, ContactPool{nullptr, nullptr, nullptr, 0});
+  physics<TASK, SPEC, true, PARAMS>(C, B, e, ch, cl, live, nsub, ContactPool{nullptr, nullptr, nullptr, 0}, PARAMS ? par + i : nullptr);
   if (live) store_env<TASK>(B, n, i, e);
 }
 
@@ -728,7 +784,7 @@ __global__ void __launch_bounds__(kBlock) forward_kernel(const __grid_constant__
     contact_solve<float>(C.dyn, C.kin, C.pad, C.con, cio, ~0u);
 #pragma unroll
     for (int j = 0; j < SO_NJ; j++) a[j] = cio.a[j];
-  } else solve_qacc<float>(C.con, M, b, q, zc, v, a, 12);
+  } else solve_qacc<float>(C.con, C.con.fr_loss, M, b, q, zc, v, a, 12);
   if (M_out)
 #pragma unroll
     for (int k = 0; k < 21; k++) M_out[k * n + i] = M[k];
@@ -1102,7 +1158,7 @@ static int host_coop_solve(const DynC<float>& D, const KinC<float>& Kn, const Pa
   double sd[CoopSlot::kDoubles];
   memset(sf, 0, sizeof sf); memset(sd, 0, sizeof sd);
   const CoopSlot S{sf, sd};
-  const int nc = coop_fill(D, Kn, P, K, S, io.s, io.c, io.q, io.qc, io.qd, io.M, io.b, io.a, touch);
+  const int nc = coop_fill(D, Kn, P, K, K.fr_loss, S, io.s, io.c, io.q, io.qc, io.qd, io.M, io.b, io.a, touch);
   if (nc < 0) return kNoCoop;
   if (nc == 0) return 0;
   const int st = coop_solve_host(S, nls);
@@ -1157,7 +1213,7 @@ static void host_substeps_t(const DynC<T>& D, const KinC<T>& Kn, const PadC<T>& 
       }
       if (!solved) {
         static const int sw0 = getenv("SO100_SWEEPS0") ? atoi(getenv("SO100_SWEEPS0")) : SO100_SWEEPS_FIRST, sw1 = getenv("SO100_SWEEPS1") ? atoi(getenv("SO100_SWEEPS1")) : SO100_SWEEPS_REST;
-        const T dlast = solve_qacc<T>(K, M, b, q, qc, v, w, sub == 0 ? sw0 : sw1);
+        const T dlast = solve_qacc<T>(K, K.fr_loss, M, b, q, qc, v, w, sub == 0 ? sw0 : sw1);
         T amax = T(1);
         for (int j = 0; j < SO_NJ; j++) amax = std::fmax(amax, std::fabs(w[j]));
         if (stats && dlast > T(2e-3) * amax) stats[4] += 1;  // as physics<> counts Gauss-Seidel substeps that were still moving
@@ -1200,6 +1256,7 @@ struct so100_ctx {
   float* start_tab = nullptr;
   int64_t tick = 0, launches = 0;
   bool specialised = false;  // model == the constants baked into so100_dyn_gen.cuh
+  ParamIO par{};             // per-env dynamics parameters; par.p == nullptr: off (so100_set_param_ranges)
   // staging for the *_host entry points
   float *h_act = nullptr, *h_obs = nullptr, *h_rew = nullptr, *h_tobs = nullptr, *h_epr = nullptr;
   uint8_t *h_term = nullptr, *h_trunc = nullptr;
@@ -1233,7 +1290,7 @@ static void free_ctx(so100_ctx* c) {
   if (!c) return;
   cudaSetDevice(c->device);
   void* ptrs[] = {c->B.qpos, c->B.qvel, c->B.warm, c->B.qcomp, c->B.block, c->B.snap, c->B.aux, c->B.ep_return, c->B.cnt, c->B.stats,
-                  c->start_tab, c->h_act, c->h_obs, c->h_rew, c->h_tobs, c->h_epr, c->h_term, c->h_trunc, c->h_epl};
+                  c->start_tab, c->par.p, c->h_act, c->h_obs, c->h_rew, c->h_tobs, c->h_epr, c->h_term, c->h_trunc, c->h_epl};
   for (void* p : ptrs) if (p) cudaFree(p);
   if (c->d_any_done) cudaFree(c->d_any_done);
   if (c->p_any_done) cudaFreeHost(c->p_any_done);
@@ -1346,8 +1403,10 @@ int so100_create(const so100_model* m, const so100_task_cfg* cfg, int device, so
   {  // the contact pool is > 48 KB of dynamic shared memory: opt in, per device, for this task's step kernels
     cudaError_t e1 = cudaSuccess, e2 = cudaSuccess;
 #define SO100_OPT(T)                                                                                                              \
-  e1 = cudaFuncSetAttribute(step_kernel<T, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPoolBytes);         \
-  e2 = cudaFuncSetAttribute(step_kernel<T, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPoolBytes)
+  e1 = cudaFuncSetAttribute(step_kernel<T, true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPoolBytes);  \
+  e2 = cudaFuncSetAttribute(step_kernel<T, false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPoolBytes); \
+  if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(step_kernel<T, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPoolBytes); \
+  if (e2 == cudaSuccess) e2 = cudaFuncSetAttribute(step_kernel<T, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPoolBytes)
     switch (c->task) {
       case 1: SO100_OPT(1); break;
       case 2: SO100_OPT(2); break;
@@ -1371,10 +1430,10 @@ int so100_reset(so100_ctx* c, const uint8_t* mask_dev, float* obs_dev, void* str
   cudaStream_t st = (cudaStream_t)stream;
   unsigned tick = (unsigned)c->tick;
   switch (c->task) {
-    case 1: reset_kernel<1><<<grid_for(c->n), kBlock, 0, st>>>(c->C, c->B, mask_dev, obs_dev, tick); break;
-    case 2: reset_kernel<2><<<grid_for(c->n), kBlock, 0, st>>>(c->C, c->B, mask_dev, obs_dev, tick); break;
-    case 6: reset_kernel<6><<<grid_for(c->n), kBlock, 0, st>>>(c->C, c->B, mask_dev, obs_dev, tick); break;
-    default: reset_kernel<5><<<grid_for(c->n), kBlock, 0, st>>>(c->C, c->B, mask_dev, obs_dev, tick); break;
+    case 1: reset_kernel<1><<<grid_for(c->n), kBlock, 0, st>>>(c->C, c->B, mask_dev, obs_dev, tick, c->par); break;
+    case 2: reset_kernel<2><<<grid_for(c->n), kBlock, 0, st>>>(c->C, c->B, mask_dev, obs_dev, tick, c->par); break;
+    case 6: reset_kernel<6><<<grid_for(c->n), kBlock, 0, st>>>(c->C, c->B, mask_dev, obs_dev, tick, c->par); break;
+    default: reset_kernel<5><<<grid_for(c->n), kBlock, 0, st>>>(c->C, c->B, mask_dev, obs_dev, tick, c->par); break;
   }
   c->launches++;
   mark_caller_stream_work(c);
@@ -1386,12 +1445,18 @@ static int launch_step(so100_ctx* c, const StepIO& io, cudaStream_t st) {
   const int g = grid_for(io.env_hi - io.env_lo);
   const bool pads = c->C.pad.n > 0;
   const size_t dyn = pads ? kPoolBytes : 0;
-  // three variants per task: model-specialised without / with the arm-floor contact path, and the generic one (any model, with it)
-#define SO100_LAUNCH(T)                                                                                    \
-  do {                                                                                                     \
-    if (c->specialised && !pads) step_kernel<T, true, false><<<g, kBlock, 0, st>>>(c->C, c->B, io);        \
-    else if (c->specialised) step_kernel<T, true, true><<<g, kBlock, dyn, st>>>(c->C, c->B, io);           \
-    else step_kernel<T, false, true><<<g, kBlock, dyn, st>>>(c->C, c->B, io);                              \
+  // three variants per task: model-specialised without / with the arm-floor contact path, and the generic one (any model, with it);
+  // each again with per-env dynamics parameters while ranges are set
+#define SO100_VARIANTS(T, P)                                                                                  \
+  do {                                                                                                        \
+    if (c->specialised && !pads) step_kernel<T, true, false, P><<<g, kBlock, 0, st>>>(c->C, c->B, io, c->par);        \
+    else if (c->specialised) step_kernel<T, true, true, P><<<g, kBlock, dyn, st>>>(c->C, c->B, io, c->par);           \
+    else step_kernel<T, false, true, P><<<g, kBlock, dyn, st>>>(c->C, c->B, io, c->par);                              \
+  } while (0)
+#define SO100_LAUNCH(T)                     \
+  do {                                      \
+    if (c->par.p) SO100_VARIANTS(T, true);  \
+    else SO100_VARIANTS(T, false);          \
   } while (0)
   switch (c->task) {
     case 1: SO100_LAUNCH(1); break;
@@ -1400,6 +1465,7 @@ static int launch_step(so100_ctx* c, const StepIO& io, cudaStream_t st) {
     default: SO100_LAUNCH(5); break;
   }
 #undef SO100_LAUNCH
+#undef SO100_VARIANTS
   c->launches++;
   CU(cudaGetLastError());
   return SO100_OK;
@@ -1435,7 +1501,11 @@ int so100_step_substeps(so100_ctx* c, const float* ctrl_dev, int n_substeps, voi
   CU(cudaSetDevice(c->device));
   cudaStream_t st = (cudaStream_t)stream;
   const int g = grid_for(c->n);
-#define SO100_SUBSTEPS(T, S) substeps_kernel<T, S><<<g, kBlock, 0, st>>>(c->C, c->B, ctrl_dev, n_substeps)
+#define SO100_SUBSTEPS(T, S)                                                                                   \
+  do {                                                                                                         \
+    if (c->par.p) substeps_kernel<T, S, true><<<g, kBlock, 0, st>>>(c->C, c->B, ctrl_dev, n_substeps, c->par.p); \
+    else substeps_kernel<T, S, false><<<g, kBlock, 0, st>>>(c->C, c->B, ctrl_dev, n_substeps, nullptr);        \
+  } while (0)
   switch (c->task) {  // a debug entry: always the generic recursion (the same mathematics; csrc/so100_dyn.cuh)
     case 1: SO100_SUBSTEPS(1, false); break;
     case 2: SO100_SUBSTEPS(2, false); break;
@@ -1715,6 +1785,78 @@ int so100_set_seed(so100_ctx* c, uint64_t seed) {
   return SO100_OK;
 }
 
+// ---- per-env dynamics parameters
+static bool group_step_in_flight(const so100_ctx* c) {
+  for (int g = 0; g < c->n_groups; g++) if (c->g_pending[g]) return true;
+  return false;
+}
+
+int so100_set_param_ranges(so100_ctx* c, const so100_param_ranges* r) {
+  if (!c) return fail(SO100_ERR_ARG, "null argument");
+  if (group_step_in_flight(c)) return fail(SO100_ERR_STATE, "an asynchronous group step is in flight: call so100_step_host_wait first");
+  CU(cudaSetDevice(c->device));
+  if (!r) {  // off: the model's constants and the default kernels again
+    if (c->par.p) {
+      CU(cudaDeviceSynchronize());  // no launch may still read the array
+      CU(cudaFree(c->par.p));
+      c->par.p = nullptr;
+    }
+    return SO100_OK;
+  }
+  if (r->struct_size != (int)sizeof(so100_param_ranges)) return fail(SO100_ERR_ARG, "so100_param_ranges.struct_size mismatch");
+  const double(*rows[4])[2] = {r->kp, r->damping, r->forcerange, r->frictionloss};
+  const char* names[4] = {"kp", "damping", "forcerange", "frictionloss"};
+  const bool positive[4] = {true, false, true, false};
+  float lo[kParamDraws], hi[kParamDraws];
+  for (int g = 0; g < 4; g++) {
+    for (int j = 0; j < SO_NJ; j++) {
+      const double a = rows[g][j][0], b = rows[g][j][1];
+      if (!std::isfinite((float)a) || !std::isfinite((float)b) || !(a <= b))
+        return fail(SO100_ERR_ARG, std::string(names[g]) + ": every range needs finite bounds with lo <= hi");
+      if (positive[g] ? !(a > 0) : !(a >= 0)) return fail(SO100_ERR_ARG, std::string(names[g]) + (positive[g] ? ": lo must be > 0" : ": lo must be >= 0"));
+      lo[g * SO_NJ + j] = (float)a; hi[g * SO_NJ + j] = (float)b;
+    }
+  }
+  if (!c->par.p) {  // first set: every env starts from the ctx's own constants and keeps them until its next reset
+    const size_t n = (size_t)c->n;
+    float* d = nullptr;
+    CU(cudaMalloc((void**)&d, kParams * n * 4));
+    float* h = (float*)malloc(kParams * n * 4);
+    if (!h) { cudaFree(d); return fail(SO100_ERR_CUDA, "out of host memory"); }
+    const TaskC& t = c->C.t;
+    for (int j = 0; j < SO_NJ; j++) {
+      const float v[5] = {t.act.kp[j], t.act.kv[j], t.act.frc_lo[j], t.act.frc_hi[j], c->C.con.fr_loss[j]};
+      for (int k = 0; k < 5; k++) for (size_t i = 0; i < n; i++) h[(k * SO_NJ + j) * n + i] = v[k];
+    }
+    const cudaError_t e = cudaMemcpy(d, h, kParams * n * 4, cudaMemcpyHostToDevice);
+    free(h);
+    if (e != cudaSuccess) { cudaFree(d); return fail(SO100_ERR_CUDA, std::string("cudaMemcpy(params): ") + cudaGetErrorString(e)); }
+    c->par.p = d;
+  }
+  memcpy(c->par.lo, lo, sizeof lo);  // the ranges travel by value with every launch: they apply from each env's next reset
+  memcpy(c->par.hi, hi, sizeof hi);
+  return SO100_OK;
+}
+
+static int copy_params(so100_ctx* c, const so100_param_view* v, void* stream, bool get) {
+  if (!c || !v) return fail(SO100_ERR_ARG, "null argument");
+  if (group_step_in_flight(c)) return fail(SO100_ERR_STATE, "an asynchronous group step is in flight: call so100_step_host_wait first");
+  if (!c->par.p) return fail(SO100_ERR_STATE, "per-env parameters are off: call so100_set_param_ranges first");
+  CU(cudaSetDevice(c->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t n = (size_t)c->n, rows = SO_NJ * n;
+  float* f[5] = {v->kp, v->kv, v->force_lo, v->force_hi, v->frictionloss};
+  for (int k = 0; k < 5; k++) {
+    if (!f[k]) continue;
+    if (get) CU(cudaMemcpyAsync(f[k], c->par.p + k * rows, rows * 4, cudaMemcpyDeviceToDevice, st));
+    else CU(cudaMemcpyAsync(c->par.p + k * rows, f[k], rows * 4, cudaMemcpyDeviceToDevice, st));
+  }
+  mark_caller_stream_work(c);
+  return SO100_OK;
+}
+int so100_get_env_params(so100_ctx* c, const so100_param_view* v, void* stream) { return copy_params(c, v, stream, true); }
+int so100_set_env_params(so100_ctx* c, const so100_param_view* v, void* stream) { return copy_params(c, v, stream, false); }
+
 int so100_forward_dynamics(so100_ctx* c, int n, const float* qpos_dev, const float* qvel_dev, const float* ctrl_dev,
                            float* M_dev, float* bias_dev, float* qacc_dev, float* kin_dev, void* stream) {
   if (!c || n <= 0 || !qpos_dev || !qvel_dev || !ctrl_dev) return fail(SO100_ERR_ARG, "bad argument");
@@ -1786,7 +1928,7 @@ int so100_host_forward(const so100_model* m, int n, const double* qpos, const do
         memcpy(cio.M, M, sizeof M);
         st = contact_solve<float>(Cf.dyn, Cf.kin, Cf.pad, Cf.con, cio, ~0u);
         memcpy(a, cio.a, sizeof a);
-      } else solve_qacc<float>(Cf.con, M, b, q, zc, v, a, sweeps > 0 ? sweeps : 1);
+      } else solve_qacc<float>(Cf.con, Cf.con.fr_loss, M, b, q, zc, v, a, sweeps > 0 ? sweeps : 1);
       if (M_out) for (int k = 0; k < 21; k++) M_out[21 * i + k] = M[k];
       if (bias_out) for (int j = 0; j < SO_NJ; j++) bias_out[6 * i + j] = bias[j];
       if (qacc_out) for (int j = 0; j < SO_NJ; j++) qacc_out[6 * i + j] = a[j];
@@ -1811,7 +1953,7 @@ int so100_host_forward(const so100_model* m, int n, const double* qpos, const do
       memcpy(cio.M, M, sizeof M);
       contact_solve<double>(H.dyn, H.kin, H.pad, H.con, cio, ~0u);
       memcpy(a, cio.a, sizeof a);
-    } else solve_qacc<double>(H.con, M, b, q, zc, v, a, sweeps > 0 ? sweeps : 1);
+    } else solve_qacc<double>(H.con, H.con.fr_loss, M, b, q, zc, v, a, sweeps > 0 ? sweeps : 1);
     if (M_out) memcpy(M_out + 21 * i, M, sizeof M);
     if (bias_out) memcpy(bias_out + 6 * i, bias, sizeof bias);
     if (qacc_out) memcpy(qacc_out + 6 * i, a, sizeof a);

@@ -352,9 +352,10 @@ SO_HD void limit_row(const ConC<T>& K, int j, T m, T q, T qc, T qd, T& xl, T& sD
 // every constraint row touches ONE dof, so each coordinate update is the exact 1-D minimiser.  M ~ armature-dominated
 // (cond < 1.3) => contraction ~1e-2 per sweep (measured against the fp64 Newton oracle, see DESIGN.md).
 // a[] holds the warm start on entry and the solution on exit; returns the largest update of the LAST sweep.
-// qc[] is the compensation term of the fp32 position integration (zeros when T = double).
+// qc[] is the compensation term of the fp32 position integration (zeros when T = double).  loss[] is the friction loss of
+// the dofs: K.fr_loss, or an env's own values (so100_set_param_ranges).
 template <typename T>
-SO_HD T solve_qacc(const ConC<T>& K, const T* M, const T* b, const T* q, const T* qc, const T* qd, T* a, int sweeps) {
+SO_HD T solve_qacc(const ConC<T>& K, const T* loss, const T* M, const T* b, const T* q, const T* qc, const T* qd, T* a, int sweeps) {
   // per-dof constants of this substep.  Friction row only:  t = c - m af,  x = af + (t - clamp(t kap, +-loss)) / m
   //   = (af + t rm) - clamp(t kr, +-lr)   with kr = kap rm, lr = loss rm;  bp = b - m af folds "- m af" into the sum.
   T af[SO_NJ], rm[SO_NJ], kr[SO_NJ], lr[SO_NJ], bp[SO_NJ], xl[SO_NJ], sDl[SO_NJ], rm2[SO_NJ], kap2[SO_NJ], dl[SO_NJ];
@@ -364,7 +365,7 @@ SO_HD T solve_qacc(const ConC<T>& K, const T* M, const T* b, const T* q, const T
     af[j] = -K.fr_B[j] * qd[j];
     rm[j] = so_rcp(m);
     kr[j] = K.fr_D[j] * so_rcp(m + K.fr_D[j]) * rm[j];
-    lr[j] = K.fr_loss[j] * rm[j];
+    lr[j] = loss[j] * rm[j];
     bp[j] = b[j] - m * af[j];
     xl[j] = T(0); sDl[j] = T(0); rm2[j] = T(0); kap2[j] = T(0); dl[j] = T(0);
     if ((q[j] - K.lo[j]) - qc[j] < T(0) || (K.hi[j] - q[j]) + qc[j] < T(0)) {
@@ -393,7 +394,7 @@ SO_HD T solve_qacc(const ConC<T>& K, const T* M, const T* b, const T* q, const T
       T x = so_fma(t, rm[j], af[j]) - so_clamp(t * kr[j], -lr[j], lr[j]);
       if (sDl[j] != T(0)) {  // limit row present: active iff the limit-free minimiser violates it
         T t2 = t + dl[j];
-        T x2 = af[j] + (t2 - so_clamp(t2 * kap2[j], -K.fr_loss[j], K.fr_loss[j])) * rm2[j];
+        T x2 = af[j] + (t2 - so_clamp(t2 * kap2[j], -loss[j], loss[j])) * rm2[j];
         x = sDl[j] * (x - xl[j]) < T(0) ? x2 : x;
       }
       if (TRACK) {
@@ -680,7 +681,7 @@ SO_HD int contact_setup(const DynC<TC>& C, const KinC<TC>& Kc, const PadC<TC>& P
 // was hit or the Hessian was not positive definite; *overflow is set if more than Store::kMaxCon corners penetrated
 // (the solve is then not attempted with this store: the caller retries with a larger one).
 template <typename TC, typename Store>
-SO_HD int contact_newton(const DynC<TC>& C, const KinC<TC>& Kc, const PadC<TC>& P, const ConC<TC>& K, Store& S, const TC* s, const TC* c,
+SO_HD int contact_newton(const DynC<TC>& C, const KinC<TC>& Kc, const PadC<TC>& P, const ConC<TC>& K, const TC* loss, Store& S, const TC* s, const TC* c,
                          const TC* q, const TC* qc, const TC* qd, const TC* M, const TC* b, TC* a, unsigned pad_mask, bool exact_in,
                          int* overflow, int* ls_evals) {
   typedef double T;
@@ -709,7 +710,7 @@ SO_HD int contact_newton(const DynC<TC>& C, const KinC<TC>& Kc, const PadC<TC>& 
       T v = -(T)b[i];
 #pragma unroll
       for (int j = 0; j < SO_NJ; j++) v += (T)(j <= i ? M[midx(i, j)] : M[midx(j, i)]) * x[j];
-      const T fD = K.fr_D[i], fL = K.fr_loss[i];
+      const T fD = K.fr_D[i], fL = loss[i];
       const T t = fD * (x[i] - (T)af[i]);  // Huber friction row: force -clamp(D r, +-loss)
       if (t > -fL && t < fL) { v += t; S.H(midx(i, i)) += fD; }
       else v += t < T(0) ? -fL : fL;
@@ -788,7 +789,7 @@ SO_HD int contact_newton(const DynC<TC>& C, const KinC<TC>& Kc, const PadC<TC>& 
       same = true;
 #pragma unroll
       for (int j = 0; j < SO_NJ; j++) {
-        const T fD = K.fr_D[j], fL = K.fr_loss[j];
+        const T fD = K.fr_D[j], fL = loss[j];
         const T r0 = x[j] - (T)af[j], t0 = fD * r0, t = fD * (r0 + al * p[j]);
         const bool q0 = t0 > -fL && t0 < fL, q1 = t > -fL && t < fL;
         if (q1) { d += t * p[j]; cv += fD * p[j] * p[j]; }
@@ -854,13 +855,25 @@ struct ContactIO {  // inputs / output of the out-of-line solve, copied once at 
 // The solve with thread-local storage for up to SO_MAX_CON contacts, out of line: the host path, and on the device the
 // fallback of a lane that found no slot in the shared-memory pool or more corners than a slot holds.
 template <typename TC>
-SO_NOINLINE int contact_solve(const DynC<TC>& C, const KinC<TC>& Kc, const PadC<TC>& P, const ConC<TC>& K, ContactIO<TC>& io,
-                               unsigned pad_mask, int* overflow = nullptr, int* ls_evals = nullptr) {
+SO_HD int contact_solve_local(const DynC<TC>& C, const KinC<TC>& Kc, const PadC<TC>& P, const ConC<TC>& K, const TC* loss, ContactIO<TC>& io,
+                              unsigned pad_mask, int* overflow, int* ls_evals) {
   ContactLocal<TC, SO_MAX_CON> S;
   int over = 0;
-  const int st = contact_newton<TC>(C, Kc, P, K, S, io.s, io.c, io.q, io.qc, io.qd, io.M, io.b, io.a, pad_mask, sizeof(TC) == 8, &over, ls_evals);
+  const int st = contact_newton<TC>(C, Kc, P, K, loss, S, io.s, io.c, io.q, io.qc, io.qd, io.M, io.b, io.a, pad_mask, sizeof(TC) == 8, &over, ls_evals);
   if (over && overflow) *overflow = 1;
   return over ? -1 : st;
+}
+template <typename TC>
+SO_NOINLINE int contact_solve(const DynC<TC>& C, const KinC<TC>& Kc, const PadC<TC>& P, const ConC<TC>& K, ContactIO<TC>& io,
+                               unsigned pad_mask, int* overflow = nullptr, int* ls_evals = nullptr) {
+  return contact_solve_local<TC>(C, Kc, P, K, K.fr_loss, io, pad_mask, overflow, ls_evals);
+}
+// The same with the env's own friction loss (so100_set_param_ranges): a separate function, so that the call of the
+// model-constant solve above keeps its signature.  loss[] is copied to the callee's frame (a cold path).
+template <typename TC>
+SO_NOINLINE int contact_solve_loss(const DynC<TC>& C, const KinC<TC>& Kc, const PadC<TC>& P, const ConC<TC>& K, const TC* loss, ContactIO<TC>& io,
+                                   unsigned pad_mask, int* overflow) {
+  return contact_solve_local<TC>(C, Kc, P, K, loss, io, pad_mask, overflow, nullptr);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -907,7 +920,7 @@ struct CoopStore {
 
 // Fill a slot (the env's own thread).  Returns the number of contacts: 0 = the accurate kinematics found no corner below
 // the floor (no solve), -1 = more than kCoopCon corners (the caller takes the out-of-line serial solve).
-SO_HD int coop_fill(const DynC<float>& C, const KinC<float>& Kc, const PadC<float>& P, const ConC<float>& K, const CoopSlot& S, const float* s,
+SO_HD int coop_fill(const DynC<float>& C, const KinC<float>& Kc, const PadC<float>& P, const ConC<float>& K, const float* loss, const CoopSlot& S, const float* s,
                     const float* c, const float* q, const float* qc, const float* qd, const float* M, const float* b, const float* a0,
                     unsigned pad_mask) {
   CoopStore st{S};
@@ -924,7 +937,7 @@ SO_HD int coop_fill(const DynC<float>& C, const KinC<float>& Kc, const PadC<floa
       limit_row(K, j, M[midx(j, j)], q[j], qc[j], qd[j], xl, sDl, rm2, kap2);
     }
     S.F(CoopSlot::kB + j) = b[j]; S.F(CoopSlot::kAf + j) = -K.fr_B[j] * qd[j]; S.F(CoopSlot::kXl + j) = xl; S.F(CoopSlot::kSDl + j) = sDl;
-    S.F(CoopSlot::kX0 + j) = a0[j]; S.F(CoopSlot::kFrD + j) = K.fr_D[j]; S.F(CoopSlot::kFrL + j) = K.fr_loss[j];
+    S.F(CoopSlot::kX0 + j) = a0[j]; S.F(CoopSlot::kFrD + j) = K.fr_D[j]; S.F(CoopSlot::kFrL + j) = loss[j];
   }
   S.F(CoopSlot::kMu) = P.mu;
   return nc;

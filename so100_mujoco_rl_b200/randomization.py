@@ -1,0 +1,123 @@
+"""Per-env dynamics randomisation: scale ranges for the servo gain, damping, torque limit and joint friction.
+
+Each env of a `BatchedSo100Env` with ranges set holds its own fp32 kp, kv, forcerange and friction loss and redraws them
+at every episode reset (include/so100_b200.h, so100_param_ranges; DESIGN.md "Per-env dynamics randomisation"):
+
+    s = lo + (hi - lo) u,  u ~ U[0, 1)
+    kp = kp0 s_kp,  kv = kv0 sqrt(s_kp) s_damping,  forcerange = forcerange0 s_forcerange,  frictionloss = frictionloss0 s_frictionloss
+
+where kp0, ... are the model's values.  `damping` is the damping ratio relative to the model's.  A range (1, 1) leaves a
+parameter at the model's value.
+"""
+from __future__ import annotations
+
+import ctypes
+import math
+from dataclasses import dataclass, field
+
+import numpy as np
+
+NJ = 6
+FIELDS = ("kp", "damping", "forcerange", "frictionloss")
+# lo must be > 0 for these (a zero gain or torque limit is not a servo), >= 0 for the others
+_POSITIVE = {"kp": True, "damping": False, "forcerange": True, "frictionloss": False}
+
+
+class So100ParamRanges(ctypes.Structure):
+    """ctypes mirror of `so100_param_ranges`."""
+    _fields_ = [("struct_size", ctypes.c_int32), ("_pad0", ctypes.c_int32)] + \
+               [(f, (ctypes.c_double * 2) * NJ) for f in FIELDS]
+
+
+class So100ParamView(ctypes.Structure):
+    """ctypes mirror of `so100_param_view` (device pointers to [6, N] float32 arrays; NULL = skip)."""
+    _fields_ = [(n, ctypes.c_void_p) for n in ("kp", "kv", "force_lo", "force_hi", "frictionloss")]
+
+
+PARAM_NAMES = ("kp", "kv", "force_lo", "force_hi", "frictionloss")
+
+
+def _ranges(v) -> np.ndarray:
+    """(lo, hi) for every joint, or [[lo, hi]] * 6 -> float64 [6, 2]."""
+    a = np.asarray(v, dtype=np.float64)
+    if a.shape == (2,):
+        a = np.broadcast_to(a, (NJ, 2))
+    if a.shape != (NJ, 2):
+        raise ValueError(f"a range is (lo, hi) or one (lo, hi) per joint ({NJ}), got shape {a.shape}")
+    return np.array(a, dtype=np.float64)
+
+
+@dataclass
+class ParamRanges:
+    """Scale ranges [lo, hi] per joint.  Each field takes a scalar pair (lo, hi), broadcast to every joint, or a [6, 2] array."""
+    kp: np.ndarray = field(default_factory=lambda: (1.0, 1.0))
+    damping: np.ndarray = field(default_factory=lambda: (1.0, 1.0))
+    forcerange: np.ndarray = field(default_factory=lambda: (1.0, 1.0))
+    frictionloss: np.ndarray = field(default_factory=lambda: (1.0, 1.0))
+
+    def __post_init__(self):
+        for f in FIELDS:
+            setattr(self, f, _ranges(getattr(self, f)))
+        self.validate()
+
+    def validate(self) -> None:
+        """The checks so100_set_param_ranges makes: finite fp32 bounds, lo <= hi, lo > 0 (kp, forcerange) or >= 0."""
+        for f in FIELDS:
+            a = getattr(self, f)
+            with np.errstate(over="ignore"):
+                a32 = a.astype(np.float32)
+            for (lo, hi), (lo32, hi32) in zip(a, a32):
+                if not (math.isfinite(lo32) and math.isfinite(hi32) and lo <= hi):
+                    raise ValueError(f"{f}: every range needs finite bounds with lo <= hi, got ({lo}, {hi})")
+                if _POSITIVE[f] and not lo > 0:
+                    raise ValueError(f"{f}: lo must be > 0, got {lo}")
+                if not _POSITIVE[f] and not lo >= 0:
+                    raise ValueError(f"{f}: lo must be >= 0, got {lo}")
+
+    def to_ctypes(self) -> So100ParamRanges:
+        r = So100ParamRanges()
+        r.struct_size = ctypes.sizeof(So100ParamRanges)
+        for f in FIELDS:
+            a = getattr(self, f)
+            dst = getattr(r, f)
+            for j in range(NJ):
+                dst[j][0], dst[j][1] = float(a[j, 0]), float(a[j, 1])
+        return r
+
+    def to_dict(self) -> dict:
+        return {f: getattr(self, f).tolist() for f in FIELDS}
+
+    @classmethod
+    def from_dict(cls, d: dict) -> "ParamRanges":
+        return cls(**{f: d[f] for f in FIELDS})
+
+    def lo_hi_f32(self) -> tuple[np.ndarray, np.ndarray]:
+        """fp32 lo, hi [24] in draw order (kp[6], damping[6], forcerange[6], frictionloss[6]), as the kernel holds them."""
+        a = np.concatenate([getattr(self, f) for f in FIELDS]).astype(np.float32)
+        return a[:, 0].copy(), a[:, 1].copy()
+
+    @classmethod
+    def parse(cls, spec: str) -> "ParamRanges":
+        """`"kp=0.7:1.3,damping=0.8:1.2,forcerange=0.8:1.0,frictionloss=0.5:2"`; fields left out stay at 1:1."""
+        kw = {}
+        for part in (p.strip() for p in spec.split(",")):
+            if not part:
+                continue
+            name, eq, rng = part.partition("=")
+            name = name.strip()
+            if not eq or name not in FIELDS:
+                raise ValueError(f"bad range {part!r}: expected <field>=lo:hi with field one of {', '.join(FIELDS)}")
+            if name in kw:
+                raise ValueError(f"{name} given twice")
+            lo, colon, hi = rng.partition(":")
+            if not colon:
+                raise ValueError(f"bad range {part!r}: expected lo:hi")
+            try:
+                kw[name] = (float(lo), float(hi))
+            except ValueError:
+                raise ValueError(f"bad range {part!r}: bounds must be numbers") from None
+        return cls(**kw)
+
+
+def parse(spec: str) -> ParamRanges:
+    return ParamRanges.parse(spec)

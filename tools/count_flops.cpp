@@ -53,12 +53,12 @@ int main() {
   long act = C::n;
   C::n = 0;
   C zc[6]; for (int j = 0; j < 6; j++) zc[j] = 0;
-  solve_qacc<C>(K, M, b, q, zc, qd, a, 12);  // converge first: the counted calls then run exactly their scheduled sweeps
+  solve_qacc<C>(K, K.fr_loss, M, b, q, zc, qd, a, 12);  // converge first: the counted calls then run exactly their scheduled sweeps
   C::n = 0;
-  solve_qacc<C>(K, M, b, q, zc, qd, a, 5);
+  solve_qacc<C>(K, K.fr_loss, M, b, q, zc, qd, a, 5);
   long solve5 = C::n;
   C::n = 0;
-  solve_qacc<C>(K, M, b, q, zc, qd, a, 3);
+  solve_qacc<C>(K, K.fr_loss, M, b, q, zc, qd, a, 3);
   long solve3 = C::n;
   C::n = 0;
   for (int j = 0; j < 6; j++) { qd[j] += C(0.002) * a[j]; q[j] += C(0.002) * qd[j]; }
