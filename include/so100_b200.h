@@ -347,6 +347,49 @@ int so100_set_param_ranges(so100_ctx *ctx, const so100_param_ranges *ranges);
 int so100_get_env_params(so100_ctx *ctx, const so100_param_view *view, void *stream);
 int so100_set_env_params(so100_ctx *ctx, const so100_param_view *view, void *stream);
 
+/*
+ * Actuator latency and joint-angle observation noise, for policies meant for the physical arm.  Opt-in: until a config
+ * is set, a new servo target acts from the first substep of the env step and the observed joint angles are exact.
+ *
+ * Latency.  Each env holds an integer latency d in [lo, hi] substeps (0 <= lo <= hi <= nsubstep).  In an env step,
+ * substeps 0 .. d-1 run on the env's PREVIOUS servo target and substeps d .. nsubstep-1 on the target this step's action
+ * sets; d = 0 is the behaviour without a config, d = nsubstep runs the whole step on the previous target.  The target is
+ * the full control value before clamping: Env01/02/06 keep the pair (ctrl_hi, ctrl_lo) = (qpos, a * joint_step_scale -
+ * qpos_comp) per env (ctrl_prev); Env05's previous target is its previous command, aux[0:6] of the state.  Substep 0 and
+ * substep d both get the first substep's Gauss-Seidel sweeps, so a latency-d step equals so100_step_substeps(d, previous
+ * target) followed by so100_step_substeps(nsubstep - d, new target).  d is drawn at every episode reset and only then,
+ * d = lo + umulhi(x, hi - lo + 1) on one Philox block (stream 14 at the auto-reset in so100_step*, including the
+ * non-finite forced reset; 22 at so100_reset), and the previous target becomes the reset pose: (qpos_reset, 0) for
+ * Env01/02/06, the start pose in aux for Env05.  so100_step_substeps (explicit ctrl), so100_set_state and Env02
+ * relocations leave d and ctrl_prev alone.
+ *
+ * Noise.  Env01/02/06: obs[:, j] (j < 6, the joint angle) becomes fp32(q_j + fp32(sigma_j z_j)) with z standard normals
+ * (Box-Muller on two Philox blocks, as the PPO act kernel; z[0..5] of the 8 it gives) on streams 24-25 for the step's
+ * observation (also the terminal_obs row), 26-27 for the auto-reset's first observation and 28-29 at so100_reset.  Output
+ * only: state, reward, flags, ep_return and ep_len do not depend on it.  sigma_j == 0 leaves the column's bits untouched.
+ * Env05 observes its commanded angles, which the robot knows exactly: a non-zero sigma there is SO100_ERR_ARG.
+ *
+ * A config applies from each env's next reset (latency) and from the next step (noise).  At the first call every env has
+ * d = 0 and, Env01/02/06, ctrl_prev = the exact current position (qpos, -qpos_comp).  All draws are keyed by (seed,
+ * env_offset + env, tick, stream): shards, env groups and the host path stay bit-exact.
+ */
+typedef struct so100_sim2real {
+  int32_t struct_size;            /* = sizeof(so100_sim2real) */
+  int32_t latency[2];             /* substeps [lo, hi], 0 <= lo <= hi <= nsubstep */
+  int32_t _pad0;
+  double obs_noise[SO100_NJ];     /* std (rad) of the noise on observed joint angle j, finite, >= 0; Env05: all 0 */
+} so100_sim2real;
+/* DEVICE pointers; NULL = skip.  latency [N]; ctrl_prev_hi / _lo [6][N] (Env01/02/06 only: Env05's is aux[0:6]) */
+typedef struct so100_actuator_view { int32_t *latency; float *ctrl_prev_hi, *ctrl_prev_lo; } so100_actuator_view;
+
+/* cfg == NULL: latency and noise off at once, back to the default kernels unless param ranges are set.  Synchronous. */
+int so100_set_sim2real(so100_ctx *ctx, const so100_sim2real *cfg);
+/* Read / overwrite the per-env actuator state (SO100_ERR_STATE while no config is set; SO100_ERR_ARG for ctrl_prev on
+   Env05); written values hold until the env's next reset, and a latency outside [0, nsubstep] acts as the nearer end.
+   All three calls return SO100_ERR_STATE while an asynchronous group step is in flight. */
+int so100_get_actuator_state(so100_ctx *ctx, const so100_actuator_view *view, void *stream);
+int so100_set_actuator_state(so100_ctx *ctx, const so100_actuator_view *view, void *stream);
+
 /* Which step kernel this ctx launches: 0 = generic (constants at run time), 1 = specialised to the baked so100 model. */
 int so100_kernel_variant(so100_ctx *ctx);
 

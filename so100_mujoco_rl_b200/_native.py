@@ -23,6 +23,7 @@ EXPORTS = [
     "so100_host_solver_constants", "so100_set_seed", "so100_step_substeps",
     "so100_host_groups", "so100_host_group_range", "so100_step_host_async", "so100_step_host_wait", "so100_step_host_wait_any",
     "so100_set_param_ranges", "so100_get_env_params", "so100_set_env_params",
+    "so100_set_sim2real", "so100_get_actuator_state", "so100_set_actuator_state",
     # include/so100_ppo.h
     "so100_ppo_param_count", "so100_ppo_workspace_floats", "so100_ppo_act", "so100_ppo_post_step", "so100_ppo_gae",
     "so100_ppo_grad", "so100_ppo_adam", "so100_ppo_permutation",
@@ -74,10 +75,13 @@ def lib() -> ctypes.CDLL:
     L.so100_step_host_async.argtypes = [vp, ci] + [vp] * 8 + [vp]
     L.so100_step_host_wait.argtypes = [vp, ci]
     L.so100_step_host_wait_any.argtypes = [vp, ctypes.POINTER(ci)]
-    from .randomization import So100ParamRanges, So100ParamView
+    from .randomization import So100ActuatorView, So100ParamRanges, So100ParamView, So100Sim2Real
     L.so100_set_param_ranges.argtypes = [vp, ctypes.POINTER(So100ParamRanges)]
     L.so100_get_env_params.argtypes = [vp, ctypes.POINTER(So100ParamView), vp]
     L.so100_set_env_params.argtypes = [vp, ctypes.POINTER(So100ParamView), vp]
+    L.so100_set_sim2real.argtypes = [vp, ctypes.POINTER(So100Sim2Real)]
+    L.so100_get_actuator_state.argtypes = [vp, ctypes.POINTER(So100ActuatorView), vp]
+    L.so100_set_actuator_state.argtypes = [vp, ctypes.POINTER(So100ActuatorView), vp]
     L.so100_get_state.argtypes = [vp, ctypes.POINTER(StateView), vp]
     L.so100_set_state.argtypes = [vp, ctypes.POINTER(StateView), vp]
     L.so100_get_tick.argtypes = [vp, i64p]

@@ -17,7 +17,7 @@ import torch
 
 from . import _native
 from .model import ModelSpec, load_model
-from .randomization import PARAM_NAMES, ParamRanges, So100ParamView
+from .randomization import ACTUATOR_NAMES, PARAM_NAMES, ParamRanges, Sim2Real, So100ActuatorView, So100ParamView
 from .tasks import MAX_EPISODE_STEPS, OBS_DIM, make_task_cfg, task_id
 
 NJ = 6
@@ -57,7 +57,8 @@ def _host_ptrs(host: dict, with_terminal: bool) -> tuple:
 class BatchedSo100Env:
     def __init__(self, env: str | int, num_envs: int, device: int | str | torch.device = 0, seed: int = 0,
                  env_offset: int = 0, flags: int = 0, model: ModelSpec | None = None,
-                 max_episode_steps: int | None = None, param_ranges: ParamRanges | None = None):
+                 max_episode_steps: int | None = None, param_ranges: ParamRanges | None = None,
+                 sim2real: Sim2Real | None = None):
         self.task = task_id(env)
         self.num_envs = int(num_envs)
         self.obs_dim = OBS_DIM[self.task]
@@ -91,6 +92,9 @@ class BatchedSo100Env:
         self.param_ranges: ParamRanges | None = None
         if param_ranges is not None:
             self.set_param_ranges(param_ranges)
+        self.sim2real: Sim2Real | None = None
+        if sim2real is not None:
+            self.set_sim2real(sim2real)
 
     # ---- lifecycle
     def close(self):
@@ -266,6 +270,44 @@ class BatchedSo100Env:
             keep.append(t)
             setattr(view, name, t.data_ptr())
         _native.check(self._L.so100_set_env_params(self._h, ctypes.byref(view), self._stream()))
+        torch.cuda.current_stream(self.device).synchronize()
+
+    # ---- actuator latency and joint-angle observation noise (randomization.py; include/so100_b200.h, so100_set_sim2real)
+    def set_sim2real(self, cfg: Sim2Real | None) -> None:
+        """Draw every env's actuator latency from cfg.latency at each of its episode resets and add Gaussian noise of std
+        cfg.obs_noise to the observed joint angles from the next step; None switches both off.  The first call starts
+        every env at latency 0 with its current position as the previous servo target."""
+        if cfg is None:
+            _native.check(self._L.so100_set_sim2real(self._h, None))
+        else:
+            cfg.validate(nsubstep=self.spec.nsubstep, task=self.task)
+            c = cfg.to_ctypes()
+            _native.check(self._L.so100_set_sim2real(self._h, ctypes.byref(c)))
+        self.sim2real = cfg
+
+    def get_actuator_state(self) -> dict:
+        """Every env's actuator state: {latency: int32 [N]} and, Env01/02/06, {ctrl_prev_hi, ctrl_prev_lo: float32 [6, N]}
+        (the previous servo target; Env05's is aux[0:6] of the state)."""
+        names = ACTUATOR_NAMES if self.task != 5 else ACTUATOR_NAMES[:1]
+        out = {k: torch.zeros(self.num_envs if k == "latency" else (NJ, self.num_envs),
+                              dtype=torch.int32 if k == "latency" else torch.float32, device=self.device) for k in names}
+        view = So100ActuatorView(*(out[k].data_ptr() if k in out else None for k in ACTUATOR_NAMES))
+        _native.check(self._L.so100_get_actuator_state(self._h, ctypes.byref(view), self._stream()))
+        return out
+
+    def set_actuator_state(self, state: dict) -> None:
+        """Overwrite some or all of the actuator state; the values hold until each env's next reset."""
+        view, keep = So100ActuatorView(), []
+        for name, t in state.items():
+            if name not in ACTUATOR_NAMES:
+                raise KeyError(f"unknown actuator field {name!r}; expected one of {ACTUATOR_NAMES}")
+            if name == "latency":
+                t = t.to(device=self.device, dtype=torch.int32).reshape(self.num_envs).contiguous()
+            else:
+                t = t.to(device=self.device, dtype=torch.float32).reshape(NJ, self.num_envs).contiguous()
+            keep.append(t)
+            setattr(view, name, t.data_ptr())
+        _native.check(self._L.so100_set_actuator_state(self._h, ctypes.byref(view), self._stream()))
         torch.cuda.current_stream(self.device).synchronize()
 
     @property

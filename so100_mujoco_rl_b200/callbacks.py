@@ -99,6 +99,9 @@ class TrainCallbacks:
             ranges = getattr(env, "param_ranges", None)  # per-env dynamics (randomization.py): resumed with the same values
             ckpt["env"]["param_ranges"] = ranges.to_dict() if ranges is not None else None
             ckpt["env"]["params"] = {k: v.cpu() for k, v in env.get_params().items()} if ranges is not None else None
+            s2r = getattr(env, "sim2real", None)  # actuator latency / observation noise: resumed with the same actuator state
+            ckpt["env"]["sim2real"] = s2r.to_dict() if s2r is not None else None
+            ckpt["env"]["actuator"] = {k: v.cpu() for k, v in env.get_actuator_state().items()} if s2r is not None else None
         torch.save(ckpt, base + ".pt")
         export_sb3_zip(base + ".zip", pol.state_dict_sb3(), {"num_timesteps": self.learner.stats.samples})
         return base

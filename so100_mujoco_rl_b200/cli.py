@@ -47,9 +47,15 @@ def cli(ctx, algorithm, model_path):
               help="per-env dynamics randomisation of the training simulator, redrawn at every episode reset, e.g. "
                    "'kp=0.7:1.3,damping=0.8:1.2,forcerange=0.8:1.0,frictionloss=0.5:2' (scales of the model's values); "
                    "evaluation stays on the model's dynamics")
+@click.option("--latency", "latency", default=None,
+              help="actuator latency of the training simulator in substeps (2 ms each), LO:HI, drawn per env at every "
+                   "episode reset: a new servo target acts from that substep of the env step; evaluation stays exact")
+@click.option("--obs-noise", "obs_noise", default=None, type=float,
+              help="std (rad) of Gaussian noise on the observed joint angles of the training simulator (Env01/02/06); "
+                   "evaluation stays exact")
 @click.pass_context
 def train(ctx, environment, num_envs, device, trainer, total_timesteps, n_steps, seed, out, learner_kind, eval_freq, eval_envs,
-          eval_steps, save_freq, tensorboard_log, randomize):
+          eval_steps, save_freq, tensorboard_log, randomize, latency, obs_noise):
     algo = ctx.obj["ALGORITHM_NAME"]
     if trainer != "sb3" and algo != "PPO":  # refuse before anything is created on disk
         raise click.UsageError("the native trainer implements PPO; use --trainer sb3 for other algorithms")
@@ -60,12 +66,25 @@ def train(ctx, environment, num_envs, device, trainer, total_timesteps, n_steps,
             ranges = ParamRanges.parse(randomize)
         except ValueError as e:
             raise click.BadParameter(str(e), param_hint="--randomize") from None
+    sim2real = None
+    if latency is not None or obs_noise is not None:
+        from .randomization import Sim2Real
+        from .tasks import task_id
+        try:
+            lat = Sim2Real.parse_latency(latency) if latency is not None else (0, 0)
+        except ValueError as e:
+            raise click.BadParameter(str(e), param_hint="--latency") from None
+        try:
+            sim2real = Sim2Real(latency=lat, obs_noise=obs_noise or 0.0)
+            sim2real.validate(task=task_id(environment))
+        except ValueError as e:
+            raise click.BadParameter(str(e), param_hint="--obs-noise" if str(e).startswith("obs_noise") else "--latency") from None
     folder = os.path.join(out, f"{environment}_{algo}")
     os.makedirs(folder, exist_ok=True)
     if trainer == "sb3":
         import stable_baselines3  # noqa: F401  (as main.py:258-262 validates the algorithm name)
         from .vec_env import So100VecEnv
-        env = So100VecEnv(environment, num_envs, device=device, seed=seed, param_ranges=ranges)
+        env = So100VecEnv(environment, num_envs, device=device, seed=seed, param_ranges=ranges, sim2real=sim2real)
         cls = getattr(stable_baselines3, algo)
         model = cls("MlpPolicy", env, device="cpu", n_steps=n_steps, verbose=1) if not ctx.obj["MODEL_PATH"] else cls.load(ctx.obj["MODEL_PATH"], env=env)
         model.learn(total_timesteps=total_timesteps)
@@ -75,7 +94,7 @@ def train(ctx, environment, num_envs, device, trainer, total_timesteps, n_steps,
     from .batched_env import BatchedSo100Env
     from .callbacks import TrainCallbacks
     from .ppo import PPO, FusedPPO, PPOConfig
-    env = BatchedSo100Env(environment, num_envs, device=device, seed=seed, param_ranges=ranges)
+    env = BatchedSo100Env(environment, num_envs, device=device, seed=seed, param_ranges=ranges, sim2real=sim2real)
     cfg = PPOConfig(n_steps=n_steps, seed=seed)
     learner = FusedPPO(env, cfg) if learner_kind == "fused" else PPO(env, cfg)
     if ctx.obj["MODEL_PATH"]:  # main.py:201-207: continue from a saved model (weights; a .pt also restores Adam and the counters)
@@ -96,6 +115,11 @@ def train(ctx, environment, num_envs, device, trainer, total_timesteps, n_steps,
                     from .randomization import ParamRanges
                     env.set_param_ranges(ParamRanges.from_dict(es["param_ranges"]))
                 env.set_params(es["params"])
+            if es.get("actuator") is not None:  # the same latencies and previous targets (and its config unless --latency / --obs-noise is given)
+                if env.sim2real is None:
+                    from .randomization import Sim2Real
+                    env.set_sim2real(Sim2Real.from_dict(es["sim2real"]))
+                env.set_actuator_state(es["actuator"])
             learner.obs = env.obs   # (stale by one step at most: refreshed by the first env.step of the next rollout)
         else:
             env.seed(seed + 1_000_003)

@@ -58,7 +58,9 @@ constexpr int kSnap = 12, kAux = 24, kCnt = 4;
 enum { F_EVER_STEPPED = 1, F_HAS_LAST_BLOCK = 2, F_ANGVEL_VALID = 4, F_CENTRE_VALID = 8,
        F_TOUCH = 16 };  // F_TOUCH: a jaw pad touched the floor in the env's last substep (scheduling hint only, no effect on results)
 enum { STREAM_RESET = 0, STREAM_TASK = 1, STREAM_NOISE = 2, STREAM_API_RESET = 3, STREAM_RESET_NOISE = 4,
-       STREAM_PARAM_RESET = 8, STREAM_PARAM_API_RESET = 16 };  // per-env parameters: streams 8..13 (auto-reset) and 16..21 (so100_reset)
+       STREAM_PARAM_RESET = 8, STREAM_PARAM_API_RESET = 16,  // per-env parameters: streams 8..13 (auto-reset) and 16..21 (so100_reset)
+       STREAM_LAT_RESET = 14, STREAM_LAT_API_RESET = 22,     // actuator latency: auto-reset, so100_reset
+       STREAM_OBS_NOISE = 24, STREAM_OBS_RESET_NOISE = 26, STREAM_OBS_API_NOISE = 28 };  // joint-angle noise, 2 streams each
 
 struct TaskC {
   int task, n, max_steps, n_start, lost_limit, nsub;
@@ -93,10 +95,20 @@ struct Bufs {
 // Per-env dynamics parameters (so100_set_param_ranges), drawn at every episode reset.  p: [kParams][n] device array,
 // rows kp[6], kv[6], force_lo[6], force_hi[6], frictionloss[6]; nullptr while ranges are off.  lo / hi: fp32 scale
 // ranges in draw order, kp[6], damping[6], forcerange[6], frictionloss[6].
+// Actuator latency and joint-angle observation noise (so100_set_sim2real) travel here as well: latency [n] (substeps;
+// nullptr while no sim2real config is set), ctrl_prev [2][6][n] (Env01/02/06: the previous step's (ctrl_hi, ctrl_lo);
+// nullptr for Env05, whose previous target is aux[0:6]), the latency range drawn at resets, and the noise std per joint.
+// Any of the three settings selects the per-env kernels; while ranges are off, p holds the model's constants and
+// lo = hi = 1, which the reset-time draw reproduces bit for bit.
 constexpr int kParams = 5 * SO_NJ, kParamDraws = 4 * SO_NJ;
 struct ParamIO {
   float* p;
   float lo[kParamDraws], hi[kParamDraws];
+  int* latency;
+  float* ctrl_prev;
+  int lat_lo, lat_hi;
+  float noise[SO_NJ];
+  int noise_on;  // some noise[j] != 0
 };
 
 struct StepIO {
@@ -299,6 +311,39 @@ __device__ __forceinline__ void draw_params(const Consts& C, const ParamIO& P, i
   }
 }
 
+// Actuator state at an episode reset (so100_set_sim2real): a new latency d = lo + umulhi(x, hi - lo + 1) from one Philox
+// block on `stream`, and the previous servo target becomes the reset pose, (q, 0) for Env01/02/06 (Env05's is aux[0:6],
+// which reset_env already set to the start pose): a delayed servo holds the pose instead of chasing ctrl = 0.
+template <int TASK>
+__device__ __forceinline__ void reset_actuator(const TaskC& t, const ParamIO& P, const EnvRegs& e, int env, unsigned tick, unsigned stream) {
+  const uint4 r = draw(t, env, tick, stream);
+  P.latency[env] = P.lat_lo + (int)__umulhi(r.x, (unsigned)(P.lat_hi - P.lat_lo + 1));
+  if (TASK != 5) {
+#pragma unroll
+    for (int j = 0; j < SO_NJ; j++) { P.ctrl_prev[j * t.n + env] = e.q[j]; P.ctrl_prev[(SO_NJ + j) * t.n + env] = 0.0f; }
+  }
+}
+
+// Joint-angle observation noise (Env01/02/06): o[j] = q_j + sigma_j z_j, z standard normals by the Box-Muller transform of
+// act_kernel (so100_ppo_kernels.cuh) on Philox blocks stream, stream + 1; z[0..5] of the 8 it gives.  A joint with
+// sigma_j == 0 keeps its bits (no 0 * z is added).  Output only: nothing the env carries depends on it.
+__device__ __forceinline__ void obs_noise(const TaskC& t, const ParamIO& P, int env, unsigned tick, unsigned stream, float* o) {
+  const uint4 r0 = draw(t, env, tick, stream), r1 = draw(t, env, tick, stream + 1);
+  const unsigned w[SO_NJ] = {r0.x, r0.y, r0.z, r0.w, r1.x, r1.y};  // (u1, u2) pairs; block 1's (z, w) would give z[6..7]
+  float z[SO_NJ];
+#pragma unroll
+  for (int k = 0; k < SO_NJ / 2; k++) {
+    const float u1 = ((float)(w[2 * k] >> 8) + 0.5f) * (1.0f / 16777216.0f), u2 = (float)(w[2 * k + 1] >> 8) * (1.0f / 16777216.0f);
+    const float rad = sqrtf(-2.0f * logf(u1));
+    float sn, cs;
+    sincospif(2.0f * u2, &sn, &cs);
+    z[2 * k] = rad * cs; z[2 * k + 1] = rad * sn;
+  }
+#pragma unroll
+  for (int j = 0; j < SO_NJ; j++)
+    if (P.noise[j] != 0.0f) o[j] = __fadd_rn(o[j], __fmul_rn(P.noise[j], z[j]));
+}
+
 __device__ __forceinline__ float joint_penalty(const TaskC& t, const float* ang) {  // env_base_01.py:144-163
   float r = 0.0f;
 #pragma unroll
@@ -347,9 +392,13 @@ constexpr size_t kPoolBytes = (size_t)kPoolSlots * (CoopSlot::kDoubles * 8 + Coo
 // round the 0.075-rad increment to the ulp of a 3-rad angle (that rounding random-walks qpos in a neutrally stable loop).
 // PARAMS: the env's own kp, kv, forcerange and friction loss (ParamIO; pv = p + env, rows n apart) replace the model's,
 // read once and held in registers over the substeps; every other constant stays the model's.
+// Actuator latency (PARAMS only): (ctrl_hi, ctrl_lo) drive substeps 0 .. d-1, and at substep d (0 < d < nsub) the control
+// switches to the step's own target, reloaded from `next` (Env01/02/06: the env's ctrl_prev column, rows n apart, where the
+// step stored it; Env05: its new command, ctrl_lo 0) so that only one control pair is held over the loop.  Substep d gets
+// the first substep's sweeps: the control jumps there.  d = 0 and next = nullptr: no switch.
 template <int TASK, bool SPEC, bool PADS, bool PARAMS>
 __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs& e, const float* ctrl_hi, const float* ctrl_lo, bool live, int nsub,
-                                        const ContactPool& pool, const float* pv) {
+                                        const ContactPool& pool, const float* pv, int d_switch = 0, const float* next = nullptr) {
   const TaskC& t = C.t;
   // SPEC: the solver / servo constants of the so100 MJCF are literals (immediates after unrolling), not constant-bank loads
   ConC<float> Kg;
@@ -382,6 +431,17 @@ __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs&
   for (int sub = 0; sub < nsub; sub++) {
     __syncthreads();  // keeps a CTA's warps on the same stretch of straight-line code (i-cache), and orders the pool's slot counters
     if (PADS && pool.nslot && threadIdx.x == 0) pool.cnt[(sub + 1) & 1] = 0;
+    if (PARAMS && sub == d_switch && sub > 0) {
+#pragma unroll
+      for (int j = 0; j < SO_NJ; j++) {
+        const float hi = TASK == 5 ? next[j] : next[j * t.n], lo = TASK == 5 ? 0.0f : next[(SO_NJ + j) * t.n];
+        const float sum = hi + lo;
+        const bool in = sum >= A.ctrl_lo[j] && sum <= A.ctrl_hi[j];
+        cc[j] = in ? hi : clampf(sum, A.ctrl_lo[j], A.ctrl_hi[j]);
+        cl[j] = in ? lo : 0.0f;
+      }
+    }
+    const int sweeps = (sub == 0 || (PARAMS && sub == d_switch)) ? SO100_SWEEPS_FIRST : SO100_SWEEPS_REST;
     float s[SO_NJ], c[SO_NJ], bias[SO_NJ], M[21], b[SO_NJ];
 #pragma unroll
     for (int j = 0; j < SO_NJ; j++) so_sincos(e.q[j], &s[j], &c[j]);
@@ -465,7 +525,7 @@ __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs&
       }
       // every other env: the per-dof Gauss-Seidel, BEFORE the cooperative phase, so that M and b are dead across it
       if (!solved && myslot < 0) {
-        d = solve_qacc<float>(K, loss, M, b, e.q, e.qc, e.v, e.w, sub == 0 ? SO100_SWEEPS_FIRST : SO100_SWEEPS_REST);
+        d = solve_qacc<float>(K, loss, M, b, e.q, e.qc, e.v, e.w, sweeps);
         solved = true;
       }
       // Phase B, the whole CTA: groups of kCoopLanes threads run the Newton solves of the filled slots.  Consecutive slots
@@ -496,7 +556,7 @@ __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs&
         }
       }
     }
-    if (!PADS) d = solve_qacc<float>(K, loss, M, b, e.q, e.qc, e.v, e.w, sub == 0 ? SO100_SWEEPS_FIRST : SO100_SWEEPS_REST);
+    if (!PADS) d = solve_qacc<float>(K, loss, M, b, e.q, e.qc, e.v, e.w, sweeps);
     float amax = 1.0f;
 #pragma unroll
     for (int j = 0; j < SO_NJ; j++) {
@@ -591,6 +651,17 @@ __global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) step_kernel(const __g
   {
     EnvRegs e;
     load_env<TASK>(B, n, i, e);
+    // actuator state, loaded with the env state: a later first touch of cold memory waits out the drain of whatever the
+    // L2 holds dirty (measured under bench.py's L2 flush: +30 us per step when these loads came just before physics<>)
+    int d = 0;
+    float ph[SO_NJ], pl[SO_NJ];
+    if (PARAMS && par.latency) {
+      d = par.latency[i];
+      if (TASK != 5) {
+#pragma unroll
+        for (int j = 0; j < SO_NJ; j++) { ph[j] = par.ctrl_prev[j * n + i]; pl[j] = par.ctrl_prev[(SO_NJ + j) * n + i]; }
+      }
+    }
     float rew, ctrl[SO_NJ], ctrl_lo[SO_NJ];
     bool term = false;
     if (TASK == 1 || TASK == 2 || TASK == 6) {
@@ -619,8 +690,18 @@ __global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) step_kernel(const __g
           for (int k = 0; k < 3; k++) e.aux[k] = e.blk[k];
         }
       }
-      physics<TASK, SPEC, PADS, PARAMS>(C, B, e, ctrl, ctrl_lo, live, t.nsub, pool, PARAMS ? par.p + i : nullptr);
+      if (PARAMS && par.latency) {  // the previous target drives substeps 0 .. d-1; this step's target goes to ctrl_prev
+        float* cp = par.ctrl_prev + i;
+#pragma unroll
+        for (int j = 0; j < SO_NJ; j++) {
+          if (live) { cp[j * n] = ctrl[j]; cp[(SO_NJ + j) * n] = ctrl_lo[j]; }
+          if (d > 0) { ctrl[j] = ph[j]; ctrl_lo[j] = pl[j]; }
+        }
+      }
+      physics<TASK, SPEC, PADS, PARAMS>(C, B, e, ctrl, ctrl_lo, live, t.nsub, pool, PARAMS ? par.p + i : nullptr, d,
+                                        PARAMS && par.latency ? par.ctrl_prev + i : nullptr);
       write_obs<TASK>(t, e, i, tick, STREAM_NOISE, obs);
+      if (PARAMS && par.noise_on) obs_noise(t, par, i, tick, STREAM_OBS_NOISE, obs);
     } else {  // env03_v1.py:124-201
       float time = (float)e.elapsed * t.dt_env;
       float f = fminf(time / t.ramp, 1.0f);
@@ -650,7 +731,11 @@ __global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) step_kernel(const __g
       float newcmd[SO_NJ];
 #pragma unroll
       for (int j = 0; j < SO_NJ; j++) { newcmd[j] = e.aux[j] + a[j] * t.step_scale; ctrl[j] = newcmd[j]; ctrl_lo[j] = 0.0f; }  // open loop (Q6)
-      physics<TASK, SPEC, PADS, PARAMS>(C, B, e, ctrl, ctrl_lo, live, t.nsub, pool, PARAMS ? par.p + i : nullptr);
+      if (PARAMS && d > 0) {  // the previous command drives substeps 0 .. d-1
+#pragma unroll
+        for (int j = 0; j < SO_NJ; j++) ctrl[j] = e.aux[j];
+      }
+      physics<TASK, SPEC, PADS, PARAMS>(C, B, e, ctrl, ctrl_lo, live, t.nsub, pool, PARAMS ? par.p + i : nullptr, d, newcmd);
       write_obs<TASK>(t, e, i, tick, STREAM_NOISE, obs);
       if (obs[6] == -1.0f && obs[7] == -1.0f) {  // :152-164
         if (e.miss > t.lost_limit) term = true;
@@ -702,6 +787,8 @@ __global__ void __launch_bounds__(kBlock, SO100_MINBLOCKS) step_kernel(const __g
       if (live && io.any_done) *io.any_done = 1;
       reset_env<TASK>(C, B, e, i, tick, STREAM_RESET, obs);
       if (PARAMS && live) draw_params(C, par, i, tick, STREAM_PARAM_RESET);
+      if (PARAMS && live && par.latency) reset_actuator<TASK>(t, par, e, i, tick, STREAM_LAT_RESET);
+      if (PARAMS && TASK != 5 && par.noise_on) obs_noise(t, par, i, tick, STREAM_OBS_RESET_NOISE, obs);
       if (live && io.terminal_obs && bad) {
 #pragma unroll
         for (int k = 0; k < OD; k++) io.terminal_obs[(size_t)i * OD + k] = obs[k];
@@ -737,9 +824,19 @@ __global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ C
   float obs[OD];
   reset_env<TASK>(C, B, e, i, tick, STREAM_API_RESET, obs);
   if (par.p) draw_params(C, par, i, tick, STREAM_PARAM_API_RESET);
+  if (par.latency) reset_actuator<TASK>(C.t, par, e, i, tick, STREAM_LAT_API_RESET);
+  if (TASK != 5 && par.noise_on) obs_noise(C.t, par, i, tick, STREAM_OBS_API_NOISE, obs);
   store_env<TASK>(B, n, i, e);
 #pragma unroll
   for (int k = 0; k < OD; k++) obs_out[(size_t)i * OD + k] = obs[k];
+}
+
+// ctrl_prev at the first so100_set_sim2real: the exact current position, (qpos, -qpos_comp); m = 6 n
+__global__ void __launch_bounds__(kBlock) actuator_init_kernel(const float* qpos, const float* qcomp, float* ctrl_prev, int m) {
+  const int k = blockIdx.x * kBlock + threadIdx.x;
+  if (k >= m) return;
+  ctrl_prev[k] = qpos[k];
+  ctrl_prev[m + k] = -qcomp[k];
 }
 
 // debug / parity triage: n x mj_step under a given ctrl, no task logic (no reward / obs / counters / reset); the snapshot
@@ -1256,7 +1353,8 @@ struct so100_ctx {
   float* start_tab = nullptr;
   int64_t tick = 0, launches = 0;
   bool specialised = false;  // model == the constants baked into so100_dyn_gen.cuh
-  ParamIO par{};             // per-env dynamics parameters; par.p == nullptr: off (so100_set_param_ranges)
+  ParamIO par{};             // per-env kernels' data; par.p == nullptr: the default kernels (neither ranges nor a sim2real config set)
+  bool ranges_on = false;    // so100_set_param_ranges set (else par.p, if allocated, holds the model's constants, lo = hi = 1)
   // staging for the *_host entry points
   float *h_act = nullptr, *h_obs = nullptr, *h_rew = nullptr, *h_tobs = nullptr, *h_epr = nullptr;
   uint8_t *h_term = nullptr, *h_trunc = nullptr;
@@ -1290,7 +1388,7 @@ static void free_ctx(so100_ctx* c) {
   if (!c) return;
   cudaSetDevice(c->device);
   void* ptrs[] = {c->B.qpos, c->B.qvel, c->B.warm, c->B.qcomp, c->B.block, c->B.snap, c->B.aux, c->B.ep_return, c->B.cnt, c->B.stats,
-                  c->start_tab, c->par.p, c->h_act, c->h_obs, c->h_rew, c->h_tobs, c->h_epr, c->h_term, c->h_trunc, c->h_epl};
+                  c->start_tab, c->par.p, c->par.latency, c->par.ctrl_prev, c->h_act, c->h_obs, c->h_rew, c->h_tobs, c->h_epr, c->h_term, c->h_trunc, c->h_epl};
   for (void* p : ptrs) if (p) cudaFree(p);
   if (c->d_any_done) cudaFree(c->d_any_done);
   if (c->p_any_done) cudaFreeHost(c->p_any_done);
@@ -1785,23 +1883,51 @@ int so100_set_seed(so100_ctx* c, uint64_t seed) {
   return SO100_OK;
 }
 
-// ---- per-env dynamics parameters
+// ---- per-env dynamics parameters, actuator latency, joint-angle observation noise
 static bool group_step_in_flight(const so100_ctx* c) {
   for (int g = 0; g < c->n_groups; g++) if (c->g_pending[g]) return true;
   return false;
+}
+
+// every env's parameters = the ctx's constants, and lo = hi = 1 (what the reset-time draw then reproduces); allocates
+// the array on first use
+static int fill_model_params(so100_ctx* c) {
+  const size_t n = (size_t)c->n;
+  float* d = c->par.p;
+  if (!d) CU(cudaMalloc((void**)&d, kParams * n * 4));
+  float* h = (float*)malloc(kParams * n * 4);
+  if (!h) { if (!c->par.p) cudaFree(d); return fail(SO100_ERR_CUDA, "out of host memory"); }
+  const TaskC& t = c->C.t;
+  for (int j = 0; j < SO_NJ; j++) {
+    const float v[5] = {t.act.kp[j], t.act.kv[j], t.act.frc_lo[j], t.act.frc_hi[j], c->C.con.fr_loss[j]};
+    for (int k = 0; k < 5; k++) for (size_t i = 0; i < n; i++) h[(k * SO_NJ + j) * n + i] = v[k];
+  }
+  const cudaError_t e = cudaMemcpy(d, h, kParams * n * 4, cudaMemcpyHostToDevice);
+  free(h);
+  if (e != cudaSuccess) { if (!c->par.p) cudaFree(d); return fail(SO100_ERR_CUDA, std::string("cudaMemcpy(params): ") + cudaGetErrorString(e)); }
+  c->par.p = d;
+  for (int k = 0; k < kParamDraws; k++) c->par.lo[k] = c->par.hi[k] = 1.0f;
+  return SO100_OK;
+}
+
+static int free_model_params(so100_ctx* c) {
+  if (c->par.p) {
+    CU(cudaDeviceSynchronize());  // no launch may still read the array
+    CU(cudaFree(c->par.p));
+    c->par.p = nullptr;
+  }
+  return SO100_OK;
 }
 
 int so100_set_param_ranges(so100_ctx* c, const so100_param_ranges* r) {
   if (!c) return fail(SO100_ERR_ARG, "null argument");
   if (group_step_in_flight(c)) return fail(SO100_ERR_STATE, "an asynchronous group step is in flight: call so100_step_host_wait first");
   CU(cudaSetDevice(c->device));
-  if (!r) {  // off: the model's constants and the default kernels again
-    if (c->par.p) {
-      CU(cudaDeviceSynchronize());  // no launch may still read the array
-      CU(cudaFree(c->par.p));
-      c->par.p = nullptr;
-    }
-    return SO100_OK;
+  if (!r) {  // off: the model's constants, and the default kernels again unless a sim2real config keeps the per-env ones
+    c->ranges_on = false;
+    if (!c->par.latency) return free_model_params(c);
+    CU(cudaDeviceSynchronize());
+    return fill_model_params(c);
   }
   if (r->struct_size != (int)sizeof(so100_param_ranges)) return fail(SO100_ERR_ARG, "so100_param_ranges.struct_size mismatch");
   const double(*rows[4])[2] = {r->kp, r->damping, r->forcerange, r->frictionloss};
@@ -1817,31 +1943,19 @@ int so100_set_param_ranges(so100_ctx* c, const so100_param_ranges* r) {
       lo[g * SO_NJ + j] = (float)a; hi[g * SO_NJ + j] = (float)b;
     }
   }
-  if (!c->par.p) {  // first set: every env starts from the ctx's own constants and keeps them until its next reset
-    const size_t n = (size_t)c->n;
-    float* d = nullptr;
-    CU(cudaMalloc((void**)&d, kParams * n * 4));
-    float* h = (float*)malloc(kParams * n * 4);
-    if (!h) { cudaFree(d); return fail(SO100_ERR_CUDA, "out of host memory"); }
-    const TaskC& t = c->C.t;
-    for (int j = 0; j < SO_NJ; j++) {
-      const float v[5] = {t.act.kp[j], t.act.kv[j], t.act.frc_lo[j], t.act.frc_hi[j], c->C.con.fr_loss[j]};
-      for (int k = 0; k < 5; k++) for (size_t i = 0; i < n; i++) h[(k * SO_NJ + j) * n + i] = v[k];
-    }
-    const cudaError_t e = cudaMemcpy(d, h, kParams * n * 4, cudaMemcpyHostToDevice);
-    free(h);
-    if (e != cudaSuccess) { cudaFree(d); return fail(SO100_ERR_CUDA, std::string("cudaMemcpy(params): ") + cudaGetErrorString(e)); }
-    c->par.p = d;
-  }
+  // first set: every env starts from the ctx's own constants and keeps them until its next reset (a sim2real config
+  // already holds them there)
+  if (!c->par.p) if (int rc = fill_model_params(c)) return rc;
   memcpy(c->par.lo, lo, sizeof lo);  // the ranges travel by value with every launch: they apply from each env's next reset
   memcpy(c->par.hi, hi, sizeof hi);
+  c->ranges_on = true;
   return SO100_OK;
 }
 
 static int copy_params(so100_ctx* c, const so100_param_view* v, void* stream, bool get) {
   if (!c || !v) return fail(SO100_ERR_ARG, "null argument");
   if (group_step_in_flight(c)) return fail(SO100_ERR_STATE, "an asynchronous group step is in flight: call so100_step_host_wait first");
-  if (!c->par.p) return fail(SO100_ERR_STATE, "per-env parameters are off: call so100_set_param_ranges first");
+  if (!c->ranges_on) return fail(SO100_ERR_STATE, "per-env parameters are off: call so100_set_param_ranges first");
   CU(cudaSetDevice(c->device));
   cudaStream_t st = (cudaStream_t)stream;
   const size_t n = (size_t)c->n, rows = SO_NJ * n;
@@ -1856,6 +1970,78 @@ static int copy_params(so100_ctx* c, const so100_param_view* v, void* stream, bo
 }
 int so100_get_env_params(so100_ctx* c, const so100_param_view* v, void* stream) { return copy_params(c, v, stream, true); }
 int so100_set_env_params(so100_ctx* c, const so100_param_view* v, void* stream) { return copy_params(c, v, stream, false); }
+
+int so100_set_sim2real(so100_ctx* c, const so100_sim2real* cfg) {
+  if (!c) return fail(SO100_ERR_ARG, "null argument");
+  if (group_step_in_flight(c)) return fail(SO100_ERR_STATE, "an asynchronous group step is in flight: call so100_step_host_wait first");
+  CU(cudaSetDevice(c->device));
+  if (!cfg) {  // off: no latency, no noise; the default kernels again unless ranges keep the per-env ones
+    if (c->par.latency) {
+      CU(cudaDeviceSynchronize());
+      CU(cudaFree(c->par.latency));
+      if (c->par.ctrl_prev) CU(cudaFree(c->par.ctrl_prev));
+      c->par.latency = nullptr; c->par.ctrl_prev = nullptr;
+    }
+    c->par.lat_lo = c->par.lat_hi = 0;
+    for (int j = 0; j < SO_NJ; j++) c->par.noise[j] = 0.0f;
+    c->par.noise_on = 0;
+    return c->ranges_on ? SO100_OK : free_model_params(c);
+  }
+  if (cfg->struct_size != (int)sizeof(so100_sim2real)) return fail(SO100_ERR_ARG, "so100_sim2real.struct_size mismatch");
+  const int nsub = c->C.t.nsub;
+  if (!(0 <= cfg->latency[0] && cfg->latency[0] <= cfg->latency[1] && cfg->latency[1] <= nsub))
+    return fail(SO100_ERR_ARG, "latency: need 0 <= lo <= hi <= nsubstep (" + std::to_string(nsub) + ")");
+  float noise[SO_NJ];
+  int noise_on = 0;
+  for (int j = 0; j < SO_NJ; j++) {
+    const double s = cfg->obs_noise[j];
+    if (!std::isfinite((float)s) || !(s >= 0)) return fail(SO100_ERR_ARG, "obs_noise: every std must be finite and >= 0");
+    noise[j] = (float)s;
+    noise_on |= noise[j] != 0.0f;
+  }
+  if (noise_on && c->task == SO100_TASK_ENV05)
+    return fail(SO100_ERR_ARG, "obs_noise: Env05 observes its commanded angles, which carry no noise");
+  if (!c->par.p) if (int rc = fill_model_params(c)) return rc;
+  if (!c->par.latency) {  // first set: every env at d = 0, and its previous target the exact current position (q, -qc)
+    const size_t n = (size_t)c->n;
+    CU(cudaDeviceSynchronize());  // the state as the caller's queued work leaves it
+    CU(cudaMalloc((void**)&c->par.latency, n * 4));
+    CU(cudaMemset(c->par.latency, 0, n * 4));
+    if (c->task != SO100_TASK_ENV05) {
+      CU(cudaMalloc((void**)&c->par.ctrl_prev, 2 * SO_NJ * n * 4));
+      actuator_init_kernel<<<grid_for(c->n * SO_NJ), kBlock>>>(c->B.qpos, c->B.qcomp, c->par.ctrl_prev, c->n * SO_NJ);
+      CU(cudaGetLastError());
+    }
+    CU(cudaDeviceSynchronize());
+  }
+  c->par.lat_lo = cfg->latency[0]; c->par.lat_hi = cfg->latency[1];  // by value with every launch: from each env's next reset
+  for (int j = 0; j < SO_NJ; j++) c->par.noise[j] = noise[j];       // from the next step
+  c->par.noise_on = noise_on;
+  return SO100_OK;
+}
+
+static int copy_actuator(so100_ctx* c, const so100_actuator_view* v, void* stream, bool get) {
+  if (!c || !v) return fail(SO100_ERR_ARG, "null argument");
+  if (group_step_in_flight(c)) return fail(SO100_ERR_STATE, "an asynchronous group step is in flight: call so100_step_host_wait first");
+  if (!c->par.latency) return fail(SO100_ERR_STATE, "latency is off: call so100_set_sim2real first");
+  if (!c->par.ctrl_prev && (v->ctrl_prev_hi || v->ctrl_prev_lo))
+    return fail(SO100_ERR_ARG, "Env05 has no ctrl_prev: its previous target is aux[0:6] of the state");
+  CU(cudaSetDevice(c->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t n = (size_t)c->n, rows = SO_NJ * n;
+  void* dev[3] = {c->par.latency, c->par.ctrl_prev, c->par.ctrl_prev ? c->par.ctrl_prev + rows : nullptr};
+  void* usr[3] = {v->latency, v->ctrl_prev_hi, v->ctrl_prev_lo};
+  const size_t bytes[3] = {n * 4, rows * 4, rows * 4};
+  for (int k = 0; k < 3; k++) {
+    if (!usr[k]) continue;
+    if (get) CU(cudaMemcpyAsync(usr[k], dev[k], bytes[k], cudaMemcpyDeviceToDevice, st));
+    else CU(cudaMemcpyAsync(dev[k], usr[k], bytes[k], cudaMemcpyDeviceToDevice, st));
+  }
+  mark_caller_stream_work(c);
+  return SO100_OK;
+}
+int so100_get_actuator_state(so100_ctx* c, const so100_actuator_view* v, void* stream) { return copy_actuator(c, v, stream, true); }
+int so100_set_actuator_state(so100_ctx* c, const so100_actuator_view* v, void* stream) { return copy_actuator(c, v, stream, false); }
 
 int so100_forward_dynamics(so100_ctx* c, int n, const float* qpos_dev, const float* qvel_dev, const float* ctrl_dev,
                            float* M_dev, float* bias_dev, float* qacc_dev, float* kin_dev, void* stream) {

@@ -8,6 +8,10 @@ at every episode reset (include/so100_b200.h, so100_param_ranges; DESIGN.md "Per
 
 where kp0, ... are the model's values.  `damping` is the damping ratio relative to the model's.  A range (1, 1) leaves a
 parameter at the model's value.
+
+`Sim2Real` sets actuator latency (a new servo target acts from substep d of the env step, d drawn per env in [lo, hi]
+at every episode reset) and Gaussian noise on the observed joint angles (include/so100_b200.h, so100_sim2real;
+DESIGN.md "Actuator latency and joint-angle observation noise").
 """
 from __future__ import annotations
 
@@ -121,3 +125,81 @@ class ParamRanges:
 
 def parse(spec: str) -> ParamRanges:
     return ParamRanges.parse(spec)
+
+
+# ---------------------------------------------------------------------------------------------------------------- sim2real
+class So100Sim2Real(ctypes.Structure):
+    """ctypes mirror of `so100_sim2real`."""
+    _fields_ = [("struct_size", ctypes.c_int32), ("latency", ctypes.c_int32 * 2), ("_pad0", ctypes.c_int32),
+                ("obs_noise", ctypes.c_double * NJ)]
+
+
+class So100ActuatorView(ctypes.Structure):
+    """ctypes mirror of `so100_actuator_view` (device pointers: latency [N] int32, ctrl_prev_hi / _lo [6, N] float32)."""
+    _fields_ = [(n, ctypes.c_void_p) for n in ("latency", "ctrl_prev_hi", "ctrl_prev_lo")]
+
+
+ACTUATOR_NAMES = ("latency", "ctrl_prev_hi", "ctrl_prev_lo")
+
+
+@dataclass
+class Sim2Real:
+    """Actuator latency in substeps, drawn per env in [lo, hi] at every episode reset, and the std (rad) of the Gaussian
+    noise on each observed joint angle (a scalar for every joint, or 6 values).  Neither has a default that stands for the
+    physical arm: both are the user's to set."""
+    latency: tuple = (0, 0)
+    obs_noise: np.ndarray = 0.0
+
+    def __post_init__(self):
+        lat = tuple(self.latency)
+        if len(lat) != 2 or not all(isinstance(x, (int, np.integer)) and not isinstance(x, bool) for x in lat):
+            raise ValueError(f"latency is (lo, hi) in whole substeps, got {self.latency!r}")
+        self.latency = (int(lat[0]), int(lat[1]))
+        a = np.asarray(self.obs_noise, dtype=np.float64)
+        if a.shape == ():
+            a = np.full(NJ, float(a))
+        if a.shape != (NJ,):
+            raise ValueError(f"obs_noise is one std or one per joint ({NJ}), got shape {a.shape}")
+        self.obs_noise = a
+        self.validate(nsubstep=math.inf)  # the upper latency bound is the model's: checked where the model is known
+
+    def validate(self, nsubstep: int | None = None, task: int | None = None) -> None:
+        """The checks so100_set_sim2real makes: 0 <= lo <= hi <= nsubstep (the model's, by default the so100 model's),
+        finite fp32 std >= 0, and no noise on Env05 (task 5), whose observed angles are its exact commands."""
+        if nsubstep is None:
+            from .model import ModelSpec
+            nsubstep = ModelSpec.__dataclass_fields__["nsubstep"].default
+        lo, hi = self.latency
+        if not 0 <= lo <= hi <= nsubstep:
+            raise ValueError(f"latency: need 0 <= lo <= hi <= nsubstep ({nsubstep}), got ({lo}, {hi})")
+        with np.errstate(over="ignore"):
+            a32 = self.obs_noise.astype(np.float32)
+        for s, s32 in zip(self.obs_noise, a32):
+            if not (math.isfinite(s32) and s >= 0):
+                raise ValueError(f"obs_noise: every std must be finite and >= 0, got {s}")
+        if task == 5 and (a32 != 0).any():
+            raise ValueError("obs_noise: Env05 observes its commanded angles, which carry no noise")
+
+    def to_ctypes(self) -> So100Sim2Real:
+        c = So100Sim2Real()
+        c.struct_size = ctypes.sizeof(So100Sim2Real)
+        c.latency[0], c.latency[1] = self.latency
+        for j in range(NJ):
+            c.obs_noise[j] = float(self.obs_noise[j])
+        return c
+
+    def to_dict(self) -> dict:
+        return {"latency": list(self.latency), "obs_noise": self.obs_noise.tolist()}
+
+    @classmethod
+    def from_dict(cls, d: dict) -> "Sim2Real":
+        return cls(latency=tuple(d["latency"]), obs_noise=d["obs_noise"])
+
+    @staticmethod
+    def parse_latency(spec: str) -> tuple[int, int]:
+        """`"LO:HI"` (or `"D"` for a fixed latency) in substeps."""
+        lo, colon, hi = spec.strip().partition(":")
+        try:
+            return (int(lo), int(hi if colon else lo))
+        except ValueError:
+            raise ValueError(f"bad latency {spec!r}: expected LO:HI in whole substeps") from None

@@ -33,10 +33,11 @@ except Exception:  # noqa: BLE001
 class TorchBackend:
     """Host-buffer face of BatchedSo100Env for the adapter: numpy in, numpy out, pinned staging buffers."""
 
-    def __init__(self, env_id, num_envs, device=0, seed=0, env_offset=0, flags=0, max_episode_steps=None, param_ranges=None):
+    def __init__(self, env_id, num_envs, device=0, seed=0, env_offset=0, flags=0, max_episode_steps=None, param_ranges=None,
+                 sim2real=None):
         from .batched_env import BatchedSo100Env  # needs CUDA; imported lazily so that CPU-only tooling can import this module
         self.env = BatchedSo100Env(env_id, num_envs, device=device, seed=seed, env_offset=env_offset, flags=flags,
-                                   max_episode_steps=max_episode_steps, param_ranges=param_ranges)
+                                   max_episode_steps=max_episode_steps, param_ranges=param_ranges, sim2real=sim2real)
         self.host = self.env.alloc_host()
         self.np = {k: v.numpy() for k, v in self.host.items()}
 
@@ -61,7 +62,7 @@ class So100VecEnv(_VecEnvBase):
     metadata = {"render_modes": ["human", "rgb_array", "depth_array"], "render_fps": 31}  # env_base_01.py:26-33
 
     def __init__(self, env_id: str | int, num_envs: int, device: int = 0, seed: int = 0, backend: Any = None,
-                 clip_actions: bool = True, max_episode_steps: int | None = None, param_ranges=None):
+                 clip_actions: bool = True, max_episode_steps: int | None = None, param_ranges=None, sim2real=None):
         self.task = task_id(env_id)
         self.env_id = env_id
         spec = load_model()
@@ -79,7 +80,8 @@ class So100VecEnv(_VecEnvBase):
         self.max_episode_steps = int(max_episode_steps or MAX_EPISODE_STEPS[self.task])
         self.clip_actions = clip_actions
         self._backend = backend if backend is not None else TorchBackend(
-            env_id, num_envs, device=device, seed=seed, max_episode_steps=self.max_episode_steps, param_ranges=param_ranges)
+            env_id, num_envs, device=device, seed=seed, max_episode_steps=self.max_episode_steps, param_ranges=param_ranges,
+            sim2real=sim2real)
         self._actions = None
         self._t0 = time.time()
         self.obs_dim = OBS_DIM[self.task]
