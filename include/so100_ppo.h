@@ -72,7 +72,8 @@ int so100_ppo_permutation(int n, uint64_t key, int64_t *idx_out, void *stream);
 /*
  * Gradient of  pg_loss + vf_coef * v_loss - ent_coef * entropy  over the minibatch idx[0..mb) of the flattened rollout
  * buffers (obs [S][od], act [S][6], logp_old [S], adv [S], ret [S]); advantages are normalised over the minibatch
- * ((a - mean) / (std_unbiased + 1e-8)) when normalize != 0.  grad [param_count] is overwritten; loss_out[3] =
+ * ((a - mean) / (std_unbiased + 1e-8)) when normalize != 0 and mb > 1; a one-sample minibatch keeps its raw advantage,
+ * as SB3 2.x does (normalising one sample would zero the policy gradient).  grad [param_count] is overwritten; loss_out[3] =
  * {pg_loss, v_loss, approx_kl}.  workspace: so100_ppo_workspace_floats() floats.  Deterministic (fixed tile order).
  */
 int so100_ppo_grad(int obs_dim, const float *params, const float *obs, const float *act, const float *logp_old,
@@ -81,7 +82,8 @@ int so100_ppo_grad(int obs_dim, const float *params, const float *obs, const flo
 
 /*
  * torch.nn.utils.clip_grad_norm_(max_norm) followed by one torch.optim.Adam step (no amsgrad, no weight decay).
- * step_count (device int32) is incremented; grad_scale multiplies grad first (1/world after an all-reduce sum).
+ * step_count (device int32) is incremented; grad_scale multiplies grad first (1/world after an all-reduce sum), and the
+ * norm that is clipped is that of the scaled gradient.  max_grad_norm <= 0 disables clipping.
  */
 int so100_ppo_adam(int n_params, float *params, const float *grad, float *exp_avg, float *exp_avg_sq,
                    int32_t *step_count, float grad_scale, float max_grad_norm, float lr, float beta1, float beta2,

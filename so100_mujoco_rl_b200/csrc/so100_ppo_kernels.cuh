@@ -1073,6 +1073,7 @@ int so100_ppo_grad(int obs_dim, const float* params, const float* obs, const flo
   cudaStream_t st = (cudaStream_t)stream;
   // fp64 partials behind the gradient partials; (total + 4) * MAX_CTAS floats is a multiple of 8 bytes
   double* stats = reinterpret_cast<double*>(workspace + (size_t)SO100_PPO_MAX_CTAS * (L.total + 4));
+  normalize = normalize && mb > 1;  // SB3 normalises only when len(advantages) > 1: one sample keeps its raw advantage
   if (normalize) ppo::adv_stats_kernel<<<ppo::kStatCtas, 256, 0, st>>>(adv, idx, mb, stats);
   ppo::grad_kernel<<<grid, ppo::NT, ppo::kGradSmemFloats * 4, st>>>(L, params, obs, act, logp_old, adv, ret, idx, mb, stats, clip_range, vf_coef,
                                                                    ent_coef, normalize, workspace);

@@ -268,7 +268,7 @@ class PPO(_LearnLoop):
     def _minibatch_step(self, idx, flat, adv, ret):
         cfg = self.cfg
         a = adv[idx]
-        if cfg.normalize_advantage:
+        if cfg.normalize_advantage and a.numel() > 1:  # SB3 2.x: the std of one sample is NaN, so it is left raw
             a = (a - a.mean()) / (a.std() + 1e-8)
         v, logp, ent = self.policy.evaluate(flat["obs"][idx], flat["act"][idx])
         lr = logp - flat["logp"][idx]

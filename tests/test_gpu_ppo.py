@@ -98,7 +98,7 @@ def _torch_minibatch_grad(pol, obs, act, logp_old, adv, ret, idx, clip, vf_coef,
     for p in pol.parameters():
         p.grad = None
     a = adv[idx]
-    if normalize:
+    if normalize and a.numel() > 1:
         a = (a - a.mean()) / (a.std() + 1e-8)
     v, logp, ent = pol.evaluate(obs[idx], act[idx])
     lr = logp - logp_old[idx]
@@ -190,7 +190,7 @@ def test_fused_ppo_tracks_the_torch_learner_and_learns():
     env.close()
 
 
-@pytest.mark.parametrize("n", [1, 2, 1000, 4096, 65536 * 32 + 17])
+@pytest.mark.parametrize("n", [1, 2, 3, 1000, 4096, 65536, 65537, 2 ** 20 - 1, 65536 * 32 + 17])
 def test_permutation_is_a_bijection_and_depends_on_the_key(n):
     L, check = _lib()
     a, b = torch.zeros(n, dtype=torch.int64, device="cuda"), torch.zeros(n, dtype=torch.int64, device="cuda")
@@ -285,7 +285,7 @@ np.savez({out!r}, a=a.cpu().numpy(), lp=lp.cpu().numpy(), v=v.cpu().numpy())
 """
 
 
-@pytest.mark.parametrize("od,n", [(15, 777), (8, 4096)])
+@pytest.mark.parametrize("od,n", [(15, 777), (8, 4096), (16, 300_000)])
 def test_act_tcgen05_and_mma_kernels_agree(od, n, tmp_path):
     """The rollout-inference kernel on tcgen05 / TMEM (the default) and the warp-level mma.sync one (SO100_PPO_ACT_MMA=1,
     read once per process, hence the subprocesses) compute the same fp32-level forward pass: same noise, values and

@@ -88,6 +88,20 @@ def test_ppo_learns_a_toy_task():
     assert algo.stats.samples == 256 * 16 * 30
 
 
+def test_one_sample_minibatches_stay_finite():
+    """num_envs * n_steps = 8 with 8 minibatches: every minibatch holds one sample.  SB3 2.x leaves a lone advantage
+    unnormalised (the std of one sample is NaN); the learner must do the same and keep finite weights and losses."""
+    from so100_mujoco_rl_b200.ppo import pack_params
+    algo = PPO(ToyEnv(4, limit=4), PPOConfig(n_steps=2, n_epochs=2, n_minibatches=8, seed=6))
+    p0 = pack_params(algo.policy)
+    hist = []
+    algo.learn(total_samples=4 * 2 * 3, log_every=0, callback=hist.append)
+    p1 = pack_params(algo.policy)
+    assert torch.isfinite(p1).all() and not torch.equal(p0, p1)
+    assert all(np.isfinite(h["pg_loss"]) and np.isfinite(h["v_loss"]) and np.isfinite(h["approx_kl"]) for h in hist)
+    assert any(h["pg_loss"] != 0.0 for h in hist)   # the policy gradient is not zeroed
+
+
 def test_truncation_bootstraps_with_terminal_value():
     env = ToyEnv(8, limit=2)
     algo = PPO(env, PPOConfig(n_steps=2, n_epochs=1, n_minibatches=1))
