@@ -14,6 +14,7 @@
  *   so100_ppo_permutation <- RolloutBuffer.get: the per-epoch shuffle of the sample indices
  *   so100_ppo_grad       <- PPO.train: policy.evaluate_actions + losses + loss.backward() for one minibatch
  *   so100_ppo_adam       <- clip_grad_norm_ + Adam.step
+ *   so100_ppo_sde_act, so100_ppo_sde_grad <- the same two with use_sde=True (gSDE, at the end of this header)
  *
  * All pointers are DEVICE pointers owned by the caller (torch tensors); nothing is allocated, nothing synchronises;
  * work is enqueued on `stream`.  Return value: SO100_OK or a negative SO100_ERR_* code (so100_last_error()).
@@ -88,6 +89,40 @@ int so100_ppo_grad(int obs_dim, const float *params, const float *obs, const flo
 int so100_ppo_adam(int n_params, float *params, const float *grad, float *exp_avg, float *exp_avg_sq,
                    int32_t *step_count, float grad_scale, float max_grad_norm, float lr, float beta1, float beta2,
                    float eps, void *stream);
+
+/*
+ * Generalized State-Dependent Exploration (gSDE): SB3's PPO(use_sde=True) with StateDependentNoiseDistribution
+ * (full_std, no expln, learn_features=False, epsilon 1e-6).  h = the policy tower's second hidden layer (64 tanh outputs).
+ *
+ * Parameter vector (so100_ppo_sde_param_count(obs_dim) entries): the layout above with log_std[6] replaced by
+ * log_std[64][6] (row-major, SB3's tensor shape), still last.  Every offset before log_std is the same in both layouts,
+ * which is why so100_ppo_post_step (value tower only), so100_ppo_gae, so100_ppo_permutation and so100_ppo_adam (with
+ * n_params = the gSDE count) serve both unchanged.
+ *
+ * Distribution:  std = exp(log_std), S = exp(2 log_std);  E[k][j] = std[k][j] z[k][j] per env;
+ *   action = mean + h E,  var_j = sum_k h_k^2 S[k][j],  scale_j = sqrt(var_j + 1e-6),  log_prob = log N(action; mean, scale),
+ *   entropy = sum_j (0.5 + log sqrt(2 pi) + log scale_j).  The variance sends gradient to log_std only, never to the tower.
+ *
+ * Draw layout of E (not stored: regenerated in registers at every call): normal number i = 64 j + k of env e is position
+ * i % 4 of the Philox-4x32-10 block keyed (seed_lo, seed_hi) with counter (env_offset + e, noise_key, 0x5D00 + i / 4, 0);
+ * words (0, 1) and (2, 3) of a block give positions (0, 1) and (2, 3) through the Box-Muller transform of so100_ppo_act:
+ *   u1 = ((w0 >> 8) + 0.5) 2^-24,  u2 = (w1 >> 8) 2^-24,  r = sqrt(-2 log u1),  z0 = r cos(2 pi u2),  z1 = r sin(2 pi u2).
+ * The same (seed, env, noise_key) and log_std give the same E, whatever the call's n, env_offset split or tick.
+ */
+int so100_ppo_sde_param_count(int obs_dim);           /* 11207 for obs_dim 15, 10311 for obs_dim 8; <0 if unsupported */
+int64_t so100_ppo_sde_workspace_floats(int obs_dim);  /* workspace of so100_ppo_sde_grad */
+
+/* so100_ppo_act's contract with the gSDE distribution; noise_key (in place of tick) selects the exploration matrices.
+ * deterministic != 0: act_raw = mean, and logp is the log-prob of the mean. */
+int so100_ppo_sde_act(int obs_dim, const float *params, const float *obs, int n, uint64_t seed, int64_t env_offset,
+                      uint32_t noise_key, int deterministic, float *act_raw, float *act_clip, float *logp, float *value,
+                      float *obs_copy, void *stream);
+
+/* so100_ppo_grad's signature and contract with the gSDE log-prob and entropy; grad [so100_ppo_sde_param_count],
+ * workspace so100_ppo_sde_workspace_floats() floats. */
+int so100_ppo_sde_grad(int obs_dim, const float *params, const float *obs, const float *act, const float *logp_old,
+                       const float *adv, const float *ret, const int64_t *idx, int mb, float clip_range, float vf_coef,
+                       float ent_coef, int normalize, float *workspace, float *grad, float *loss_out, void *stream);
 
 #ifdef __cplusplus
 }

@@ -27,6 +27,7 @@ EXPORTS = [
     # include/so100_ppo.h
     "so100_ppo_param_count", "so100_ppo_workspace_floats", "so100_ppo_act", "so100_ppo_post_step", "so100_ppo_gae",
     "so100_ppo_grad", "so100_ppo_adam", "so100_ppo_permutation",
+    "so100_ppo_sde_param_count", "so100_ppo_sde_workspace_floats", "so100_ppo_sde_act", "so100_ppo_sde_grad",
 ]
 
 
@@ -105,10 +106,15 @@ def lib() -> ctypes.CDLL:
     L.so100_ppo_grad.argtypes = [ci, vp, vp, vp, vp, vp, vp, vp, ci, cf, cf, cf, ci, vp, vp, vp, vp]
     L.so100_ppo_permutation.argtypes = [ci, u64, vp, vp]
     L.so100_ppo_adam.argtypes = [ci, vp, vp, vp, vp, vp, cf, cf, cf, cf, cf, cf, vp]
+    L.so100_ppo_sde_param_count.argtypes = [ci]
+    L.so100_ppo_sde_workspace_floats.argtypes = [ci]
+    L.so100_ppo_sde_act.argtypes = L.so100_ppo_act.argtypes
+    L.so100_ppo_sde_grad.argtypes = L.so100_ppo_grad.argtypes
     for name in EXPORTS:
         if name not in ("so100_last_error", "so100_destroy", "so100_build_id"):
             getattr(L, name).restype = ci
     L.so100_ppo_workspace_floats.restype = i64
+    L.so100_ppo_sde_workspace_floats.restype = i64
     if L.so100_abi_version() != 3:
         raise ImportError("libso100_b200.so has an unexpected ABI version; rebuild it")
     _lib = L

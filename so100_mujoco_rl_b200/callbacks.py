@@ -103,7 +103,11 @@ class TrainCallbacks:
             ckpt["env"]["sim2real"] = s2r.to_dict() if s2r is not None else None
             ckpt["env"]["actuator"] = {k: v.cpu() for k, v in env.get_actuator_state().items()} if s2r is not None else None
         torch.save(ckpt, base + ".pt")
-        export_sb3_zip(base + ".zip", pol.state_dict_sb3(), {"num_timesteps": self.learner.stats.samples})
+        meta = {"num_timesteps": self.learner.stats.samples}
+        cfg = getattr(self.learner, "cfg", None)
+        if getattr(cfg, "use_sde", False):  # SB3 reads these from `data`; policy.pth holds the [64, 6] log_std
+            meta.update(use_sde=True, sde_sample_freq=cfg.sde_sample_freq)
+        export_sb3_zip(base + ".zip", pol.state_dict_sb3(), meta)
         return base
 
     def __call__(self, rec: dict) -> None:

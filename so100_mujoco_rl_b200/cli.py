@@ -53,12 +53,31 @@ def cli(ctx, algorithm, model_path):
 @click.option("--obs-noise", "obs_noise", default=None, type=float,
               help="std (rad) of Gaussian noise on the observed joint angles of the training simulator (Env01/02/06); "
                    "evaluation stays exact")
+@click.option("--use-sde", "use_sde", is_flag=True, default=False,
+              help="generalized State-Dependent Exploration (SB3 use_sde): action noise h E from the policy's last hidden layer, "
+                   "E redrawn per env once per rollout; smooth commands instead of per-step jitter")
+@click.option("--sde-sample-freq", "sde_sample_freq", default=None, type=int,
+              help="with --use-sde: redraw the exploration matrices every N rollout steps (SB3 sde_sample_freq; default -1 = once per rollout)")
+@click.option("--log-std-init", "log_std_init", default=0.0, show_default=True, type=float,
+              help="initial log_std of the policy (SB3 policy kwarg log_std_init); gSDE runs usually start lower, e.g. -2")
 @click.pass_context
 def train(ctx, environment, num_envs, device, trainer, total_timesteps, n_steps, seed, out, learner_kind, eval_freq, eval_envs,
-          eval_steps, save_freq, tensorboard_log, randomize, latency, obs_noise):
+          eval_steps, save_freq, tensorboard_log, randomize, latency, obs_noise, use_sde, sde_sample_freq, log_std_init):
     algo = ctx.obj["ALGORITHM_NAME"]
     if trainer != "sb3" and algo != "PPO":  # refuse before anything is created on disk
         raise click.UsageError("the native trainer implements PPO; use --trainer sb3 for other algorithms")
+    if sde_sample_freq is not None and not use_sde:
+        raise click.BadParameter("needs --use-sde", param_hint="--sde-sample-freq")
+    if sde_sample_freq is None:
+        sde_sample_freq = -1
+    elif sde_sample_freq == 0 or sde_sample_freq < -1:
+        raise click.BadParameter("must be a positive number of steps or -1 (once per rollout)", param_hint="--sde-sample-freq")
+    ckpt = None
+    if ctx.obj["MODEL_PATH"] and trainer != "sb3":  # a run resumes with the exploration it was trained with
+        ckpt, saved_sde = _load_checkpoint(ctx.obj["MODEL_PATH"])
+        if saved_sde != use_sde:
+            raise click.UsageError(f"{ctx.obj['MODEL_PATH']} holds a {'gSDE' if saved_sde else 'plain Gaussian'} policy: "
+                                   f"{'add' if saved_sde else 'drop'} --use-sde to continue it")
     ranges = None
     if randomize:
         from .randomization import ParamRanges
@@ -86,7 +105,13 @@ def train(ctx, environment, num_envs, device, trainer, total_timesteps, n_steps,
         from .vec_env import So100VecEnv
         env = So100VecEnv(environment, num_envs, device=device, seed=seed, param_ranges=ranges, sim2real=sim2real)
         cls = getattr(stable_baselines3, algo)
-        model = cls("MlpPolicy", env, device="cpu", n_steps=n_steps, verbose=1) if not ctx.obj["MODEL_PATH"] else cls.load(ctx.obj["MODEL_PATH"], env=env)
+        kw = {}
+        if use_sde:
+            kw.update(use_sde=True, sde_sample_freq=sde_sample_freq)
+        if log_std_init != 0.0:
+            kw["policy_kwargs"] = dict(log_std_init=log_std_init)
+        model = cls("MlpPolicy", env, device="cpu", n_steps=n_steps, verbose=1, **kw) if not ctx.obj["MODEL_PATH"] \
+            else cls.load(ctx.obj["MODEL_PATH"], env=env, **kw)
         model.learn(total_timesteps=total_timesteps)
         model.save(os.path.join(folder, "final_model"))
         return
@@ -95,11 +120,10 @@ def train(ctx, environment, num_envs, device, trainer, total_timesteps, n_steps,
     from .callbacks import TrainCallbacks
     from .ppo import PPO, FusedPPO, PPOConfig
     env = BatchedSo100Env(environment, num_envs, device=device, seed=seed, param_ranges=ranges, sim2real=sim2real)
-    cfg = PPOConfig(n_steps=n_steps, seed=seed)
+    cfg = PPOConfig(n_steps=n_steps, seed=seed, use_sde=use_sde, sde_sample_freq=sde_sample_freq, log_std_init=log_std_init)
     learner = FusedPPO(env, cfg) if learner_kind == "fused" else PPO(env, cfg)
     if ctx.obj["MODEL_PATH"]:  # main.py:201-207: continue from a saved model (weights; a .pt also restores Adam and the counters)
         path = ctx.obj["MODEL_PATH"]
-        ckpt = torch.load(path, map_location="cpu") if path.endswith(".pt") else {}
         full = ckpt.get("learner")
         if full is not None:
             learner.load_state_dict(full)
@@ -137,16 +161,28 @@ def train(ctx, environment, num_envs, device, trainer, total_timesteps, n_steps,
                            "best_eval": cb.best, "stopped": cb.stop_reason, "last": stats.history[-1] if stats.history else None}))
 
 
+def _load_checkpoint(path):
+    """(the .pt checkpoint or {} for a .zip, whether its policy is gSDE's): a gSDE policy's log_std is [64, 6]."""
+    import torch
+    from .callbacks import load_sb3_zip
+    if path.endswith(".zip"):
+        return {}, load_sb3_zip(path)["log_std"].dim() == 2
+    ckpt = torch.load(path, map_location="cpu")
+    return ckpt, ckpt["policy"]["log_std"].dim() == 2
+
+
 def _load_policy(path, obs_dim, device):
-    """A policy saved by this package (.pt) or a Stable-Baselines3 style archive (.zip, policy.pth inside)."""
+    """A policy saved by this package (.pt) or a Stable-Baselines3 style archive (.zip, policy.pth inside); plain or gSDE,
+    told apart by the shape of log_std."""
     import torch
     from .callbacks import load_sb3_zip
     from .ppo import MlpPolicy
-    policy = MlpPolicy(obs_dim, 6)
+    sd = load_sb3_zip(path) if path.endswith(".zip") else torch.load(path, map_location="cpu")["policy"]
+    policy = MlpPolicy(obs_dim, 6, use_sde=sd["log_std"].dim() == 2)
     if path.endswith(".zip"):
-        policy.load_state_dict_sb3(load_sb3_zip(path))
+        policy.load_state_dict_sb3(sd)
     else:
-        policy.load_state_dict(torch.load(path, map_location="cpu")["policy"])
+        policy.load_state_dict(sd)
     return policy.to(device)
 
 

@@ -31,7 +31,8 @@ constexpr float LOG_SQRT_2PI = 0.91893853320467274178f;
 struct Layout {  // offsets into the flat parameter vector
   int od, W1[2], b1[2], W2[2], b2[2], W3[2], b3[2], log_std, total;
 };
-__host__ __device__ inline Layout make_layout(int od) {
+// sde: gSDE's log_std[HID][ACT] in place of log_std[ACT]; every offset before it is the same in both layouts
+__host__ __device__ inline Layout make_layout(int od, bool sde = false) {
   Layout L;
   L.od = od;
   int o = 0;
@@ -44,7 +45,7 @@ __host__ __device__ inline Layout make_layout(int od) {
     L.W3[t] = o; o += nout * HID;
     L.b3[t] = o; o += nout;
   }
-  L.log_std = o; o += ACT;
+  L.log_std = o; o += sde ? HID * ACT : ACT;
   L.total = o;
   return L;
 }
@@ -188,9 +189,57 @@ __device__ __forceinline__ void head_forward(const TowerS& T, const float* H2, f
   __syncthreads();
 }
 
+// ------------------------------------------------------------------------------------------------ gSDE (DESIGN.md §7d)
+// SB3's StateDependentNoiseDistribution (full_std, no expln, learn_features=False): with h = the policy tower's last
+// hidden layer, the action is mean + h E, E[k][j] = exp(log_std[k][j]) z[k][j] drawn per env, and the distribution is
+// Normal(mean, sqrt(var + 1e-6)) with var_j = sum_k h_k^2 S[k][j], S = exp(2 log_std).  E is never stored: normal number
+// i = 64 j + k of an env is position i % 4 of Philox block (seed, env_offset + env, noise_key, 0x5D00 + i / 4, 0), through
+// the Box-Muller transform of the plain noise (words 0,1 and 2,3).  Both inference kernels and the gradient kernel split
+// the 64 features into four groups of 16, each an fp32 FMA chain from zero in ascending k, combined as (g0 + g1) + (g2 + g3).
+constexpr unsigned kSdeStream = 0x5D00u;
+constexpr float kSdeEps = 1e-6f;
+
+// group [k0, k0 + 16) of the noise sum_k h_k fl(std_kj z_kj) (when `noise`; else zeros) and of var_j = sum_k fl(h_k^2) S_kj.
+// The Box-Muller lines restate the act kernels' own (left in place there, so that their plain instantiations keep their SASS).
+__device__ __forceinline__ void sde_partial(const float (&h)[16], int k0, unsigned seed_lo, unsigned seed_hi, unsigned env, unsigned key, bool noise,
+                                            const float* sstd, const float* sS, float (&nz)[ACT], float (&vr)[ACT]) {
+#pragma unroll
+  for (int j = 0; j < ACT; j++) { nz[j] = 0.0f; vr[j] = 0.0f; }
+#pragma unroll
+  for (int k = 0; k < 16; k++) {
+    const float h2 = h[k] * h[k];
+#pragma unroll
+    for (int j = 0; j < ACT; j++) vr[j] = fmaf(h2, sS[(k0 + k) * ACT + j], vr[j]);
+  }
+  if (!noise) return;
+#pragma unroll 1
+  for (int j = 0; j < ACT; j++) {
+#pragma unroll
+    for (int b = 0; b < 4; b++) {
+      const uint4 r = philox4x32(seed_lo, seed_hi, env, key, kSdeStream + 16u * j + (unsigned)(k0 >> 2) + b, 0u);
+      const unsigned w[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+      for (int q = 0; q < 2; q++) {
+        const float u1 = ((float)(w[2 * q] >> 8) + 0.5f) * (1.0f / 16777216.0f), u2 = (float)(w[2 * q + 1] >> 8) * (1.0f / 16777216.0f);
+        const float rad = sqrtf(-2.0f * logf(u1));
+        float sn, cs;
+        sincospif(2.0f * u2, &sn, &cs);
+        const int k = 4 * b + 2 * q;
+        nz[j] = fmaf(h[k], sstd[(k0 + k) * ACT + j] * (rad * cs), nz[j]);
+        nz[j] = fmaf(h[k + 1], sstd[(k0 + k + 1) * ACT + j] * (rad * sn), nz[j]);
+      }
+    }
+  }
+}
+// one action's term of the gSDE log-prob, given isig2 = 1 / (var + 1e-6)
+__device__ __forceinline__ float sde_logp_term(float d, float v, float isig2) { return -0.5f * d * d * isig2 - 0.5f * logf(v) - LOG_SQRT_2PI; }
+
 // ------------------------------------------------------------------------------------------------ rollout inference
 constexpr int kActSmemFloats = 2 * tower_floats(false) + K1 * LD + 2 * HID * LD + 8 * TB + 32 * TB + 8;
+constexpr int kActSmemFloatsSde = kActSmemFloats + 2 * HID * ACT;  // + std and S; the partials reuse H1
+static_assert(4 * 2 * ACT * TB <= HID * LD, "act_kernel<SDE>: the partials fit the H1 buffer");
 
+template <bool SDE>
 __global__ void __launch_bounds__(NT) act_kernel(Layout L, const float* __restrict__ P, const float* __restrict__ obs, int n, unsigned seed_lo,
                                                  unsigned seed_hi, long long env_offset, unsigned tick, int deterministic, float* act_raw,
                                                  float* act_clip, float* logp, float* value, float* obs_copy) {
@@ -204,10 +253,16 @@ __global__ void __launch_bounds__(NT) act_kernel(Layout L, const float* __restri
   float* out = p; p += 8 * TB;
   float* scratch = p; p += 32 * TB;
   float* ls = p;
+  float* sstd = ls + 8;             // (SDE) exp(log_std) [HID][ACT]
+  float* sS = sstd + HID * ACT;     // (SDE) exp(2 log_std)
   const int tid = threadIdx.x, od = L.od;
   load_tower(L, P, 0, T[0], false);
   load_tower(L, P, 1, T[1], false);
-  if (tid < ACT) ls[tid] = P[L.log_std + tid];
+  if constexpr (SDE) {
+    for (int e = tid; e < HID * ACT; e += NT) { sstd[e] = expf(P[L.log_std + e]); sS[e] = expf(2.0f * P[L.log_std + e]); }
+  } else {
+    if (tid < ACT) ls[tid] = P[L.log_std + tid];
+  }
   const Own o = own_64x64();
   const int ntiles = (n + TB - 1) / TB;
   for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {  // persistent: the weights are staged once per CTA
@@ -227,6 +282,32 @@ __global__ void __launch_bounds__(NT) act_kernel(Layout L, const float* __restri
     head_forward<1>(T[1], H2, out + 7 * TB, scratch);  // value in row 7
     tower_forward(T[0], X, H1, nullptr, H2, nullptr, o);
     head_forward<ACT>(T[0], H2, out, scratch);
+    if constexpr (SDE) {  // thread (q, s): feature group q of sample s; partials -> the H1 buffer (h1 is dead) [4][2 ACT][TB]
+      const int q = tid >> 6, s = tid & 63, g = base + s;
+      float h[16], nz[ACT], vr[ACT];
+#pragma unroll
+      for (int k = 0; k < 16; k++) h[k] = H2[(16 * q + k) * LD + s];
+      sde_partial(h, 16 * q, seed_lo, seed_hi, (unsigned)(env_offset + g), tick, !deterministic && g < n, sstd, sS, nz, vr);
+#pragma unroll
+      for (int j = 0; j < ACT; j++) { H1[(q * 2 * ACT + j) * TB + s] = nz[j]; H1[(q * 2 * ACT + ACT + j) * TB + s] = vr[j]; }
+      __syncthreads();
+      if (tid < TB && base + tid < n) {
+        const int g = base + tid;
+        auto sum4 = [&](int r) { return (H1[r * TB + tid] + H1[(2 * ACT + r) * TB + tid]) + (H1[(4 * ACT + r) * TB + tid] + H1[(6 * ACT + r) * TB + tid]); };
+        float lp = 0.0f;
+#pragma unroll
+        for (int k = 0; k < ACT; k++) {
+          const float mean = out[k * TB + tid], a = deterministic ? mean : mean + sum4(k);
+          const float v = sum4(ACT + k) + kSdeEps, d = a - mean;
+          lp += sde_logp_term(d, v, 1.0f / v);
+          if (act_raw) act_raw[(size_t)g * ACT + k] = a;
+          if (act_clip) act_clip[(size_t)g * ACT + k] = fminf(fmaxf(a, -1.0f), 1.0f);
+        }
+        if (logp) logp[g] = lp;
+        if (value) value[g] = out[7 * TB + tid];
+      }
+      continue;
+    }
     if (tid < TB && base + tid < n) {
       const int g = base + tid;
       float eps[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -277,10 +358,14 @@ struct ActTc {  // byte offsets into dynamic shared memory
   static constexpr int BIAS = W3 + 2 * 2 * 16 * 64 * 4;  // b1[2][64], b2[2][64], b3[2][8], log_std[8]
   static constexpr int BAR = BIAS + (2 * 64 + 2 * 64 + 16 + 8) * 4;
   static constexpr int BYTES = BAR + 16;
+  // gSDE only: exp(log_std) and exp(2 log_std) [64][6], then warpgroup 1's partials [2 ACT][128]
+  static constexpr int SDE_STD = BYTES, SDE_S = SDE_STD + 64 * 6 * 4, SDE_X = SDE_S + 64 * 6 * 4;
+  static constexpr int BYTES_SDE = SDE_X + 2 * 6 * 128 * 4;
   // TMEM columns (256 per CTA)
   static constexpr uint32_t cD = 0, cAh = 64, cAl = 128, cXh = 192, cXl = 208, cHead = 224;
 };
 static_assert(2 * (ActTc::BYTES + 1024) <= 227 * 1024, "act_kernel_tc: two CTAs per SM");
+static_assert(2 * (ActTc::BYTES_SDE + 1024) <= 227 * 1024, "act_kernel_tc<SDE>: two CTAs per SM");
 
 // one layer's epilogue for this thread's half of the 64 columns: h = tanh(D + bias) -> hi / lo rows of the next layer's A (TMEM)
 __device__ __forceinline__ void tc_epilogue_tanh(uint32_t tmem_row, int col0, const float* bias) {
@@ -306,6 +391,7 @@ __device__ __forceinline__ void tc_gemm3(uint32_t tmem_d, uint32_t ah, uint32_t 
   }
 }
 
+template <bool SDE>
 __global__ void __launch_bounds__(NTC, 2) act_kernel_tc(Layout L, const float* __restrict__ P, const float* __restrict__ obs, int n, unsigned seed_lo,
                                                         unsigned seed_hi, long long env_offset, unsigned tick, int deterministic, float* act_raw,
                                                         float* act_clip, float* logp, float* value, float* obs_copy) {
@@ -347,7 +433,14 @@ __global__ void __launch_bounds__(NTC, 2) act_kernel_tc(Layout L, const float* _
     for (int e = tid; e < HID; e += NTC) { b1[64 * t + e] = P[L.b1[t] + e]; b2[64 * t + e] = P[L.b2[t] + e]; }
     for (int e = tid; e < 8; e += NTC) b3[8 * t + e] = e < nout ? P[L.b3[t] + e] : 0.0f;
   }
-  if (tid < 8) ls[tid] = tid < ACT ? P[L.log_std + tid] : 0.0f;
+  float* sstd = reinterpret_cast<float*>(smc + ActTc::SDE_STD);
+  float* sS = reinterpret_cast<float*>(smc + ActTc::SDE_S);
+  float* xch = reinterpret_cast<float*>(smc + ActTc::SDE_X);
+  if constexpr (SDE) {
+    for (int e = tid; e < HID * ACT; e += NTC) { sstd[e] = expf(P[L.log_std + e]); sS[e] = expf(2.0f * P[L.log_std + e]); }
+  } else {
+    if (tid < 8) ls[tid] = tid < ACT ? P[L.log_std + tid] : 0.0f;
+  }
   tc::fence_smem_to_mma();
   tc::fence_before_sync();
   __syncthreads();
@@ -413,7 +506,44 @@ __global__ void __launch_bounds__(NTC, 2) act_kernel_tc(Layout L, const float* _
     // heads: warpgroup 0 samples the action from the six means, warpgroup 1 stores the value
     float o16[16];
     tc::tmem_ld16(tmem_row + ActTc::cHead + 16 * (half ? 1 : 0), o16);
-    if (g < n) {
+    if constexpr (SDE) {  // the policy tower's h2 = hi + lo (exact) is still in TMEM: warpgroup w takes features 32 w .. 32 w + 31
+      float nz[ACT], vr[ACT];
+#pragma unroll
+      for (int c = 0; c < 2; c++) {
+        float hi[16], lo[16], h[16], pn[ACT], pv[ACT];
+        tc::tmem_ld16(tmem_row + ActTc::cAh + 32 * half + 16 * c, hi);
+        tc::tmem_ld16(tmem_row + ActTc::cAl + 32 * half + 16 * c, lo);
+#pragma unroll
+        for (int i = 0; i < 16; i++) h[i] = hi[i] + lo[i];
+        sde_partial(h, 32 * half + 16 * c, seed_lo, seed_hi, (unsigned)(env_offset + g), tick, !deterministic && g < n, sstd, sS, pn, pv);
+#pragma unroll
+        for (int j = 0; j < ACT; j++) {
+          if (c == 0) { nz[j] = pn[j]; vr[j] = pv[j]; }
+          else { nz[j] = nz[j] + pn[j]; vr[j] = vr[j] + pv[j]; }
+        }
+      }
+      if (half) {
+#pragma unroll
+        for (int j = 0; j < ACT; j++) { xch[j * TM + row] = nz[j]; xch[(ACT + j) * TM + row] = vr[j]; }
+      }
+      __syncthreads();
+      if (g < n) {
+        if (half) {
+          if (value) value[g] = o16[0] + b3[8];
+        } else {
+          float lp = 0.0f;
+#pragma unroll
+          for (int k = 0; k < ACT; k++) {
+            const float mean = o16[k] + b3[k], a = deterministic ? mean : mean + (nz[k] + xch[k * TM + row]);
+            const float v = (vr[k] + xch[(ACT + k) * TM + row]) + kSdeEps, d = a - mean;
+            lp += sde_logp_term(d, v, 1.0f / v);
+            if (act_raw) act_raw[(size_t)g * ACT + k] = a;
+            if (act_clip) act_clip[(size_t)g * ACT + k] = fminf(fmaxf(a, -1.0f), 1.0f);
+          }
+          if (logp) logp[g] = lp;
+        }
+      }
+    } else if (g < n) {
       if (half) {
         if (value) value[g] = o16[0] + b3[8];
       } else {
@@ -578,6 +708,13 @@ constexpr int kGradSmemFloats = 2 * tower_floats(false)  // weights of both towe
                                 + 8 * GT + 8 * GT        // head outputs, head gradients
                                 + 6 * GT + 4 * GT + 32 * GT + 16;  // actions, (logp_old, adv, ret, valid), head scratch, log_std
 static_assert(kGradSmemFloats * 4 <= 113 * 1024, "two gradient CTAs must fit one SM");
+constexpr int kGradSmemFloatsSde = kGradSmemFloats + HID * ACT + 2 * ACT * GT;  // + S = exp(2 log_std), var and dL/dvar per sample
+static_assert(kGradSmemFloatsSde * 4 <= 113 * 1024, "two gSDE gradient CTAs must fit one SM");
+// the gSDE arrays behind log_std[16]: S = exp(2 log_std) [HID][ACT], var and dL/dvar [ACT][GT]
+struct GradSde {
+  float *S, *var, *dvar;
+  __device__ __forceinline__ static GradSde at(float* ls) { return GradSde{ls + 16, ls + 16 + HID * ACT, ls + 16 + HID * ACT + ACT * GT}; }
+};
 
 // A given row-major (A[m][k] at Ar[m * lda + k]) instead of K-major: same MMA, 2-way conflicted fragment loads
 template <int K, int NTILE, int lda, int ldb>
@@ -642,6 +779,7 @@ __device__ __forceinline__ void head_forward_g(const TowerS& T, const float* H2,
   __syncthreads();
 }
 
+template <bool SDE>
 __global__ void __launch_bounds__(NT, 2) grad_kernel(Layout L, const float* __restrict__ P, const float* __restrict__ obs, const float* __restrict__ act,
                                                     const float* __restrict__ logp_old, const float* __restrict__ adv, const float* __restrict__ ret,
                                                     const int64_t* __restrict__ idx, int mb, const double* __restrict__ adv_part, float clip,
@@ -664,7 +802,7 @@ __global__ void __launch_bounds__(NT, 2) grad_kernel(Layout L, const float* __re
   float* sRet = p; p += GT;
   float* sValid = p; p += GT;
   float* scratch = p; p += 32 * GT;
-  float* ls = p;
+  float* ls = p;  // log_std[6]; (SDE) then the GradSde arrays (addressed only inside the SDE branches)
 
   const int tid = threadIdx.x, od = L.od, w = tid >> 5, lane = tid & 31;
   const Own oA{16 * (w & 3), 16 * (w >> 2), lane >> 2, lane & 3};  // 64 features x 32 samples: 16 x 16 per warp
@@ -673,7 +811,12 @@ __global__ void __launch_bounds__(NT, 2) grad_kernel(Layout L, const float* __re
   const int sg = tid >> 6, fk = tid & 63;  // (group of 8 samples, feature) mapping of the reductions over a tile's samples
   load_tower(L, P, 0, T[0], false);
   load_tower(L, P, 1, T[1], false);
-  if (tid < ACT) ls[tid] = P[L.log_std + tid];
+  if constexpr (SDE) {
+    float* sS = GradSde::at(ls).S;
+    for (int e = tid; e < HID * ACT; e += NT) sS[e] = expf(2.0f * P[L.log_std + e]);
+  } else {
+    if (tid < ACT) ls[tid] = P[L.log_std + tid];
+  }
   float a_mean = 0.0f, a_rstd = 1.0f;
   if (normalize) {  // every thread combines the partials in the same order: identical values everywhere
     double s1 = 0.0, s2 = 0.0;
@@ -687,6 +830,7 @@ __global__ void __launch_bounds__(NT, 2) grad_kernel(Layout L, const float* __re
   // gradient accumulators, persistent over the CTA's tiles; each thread owns fixed parameters of both towers
   //   gW2 / gW1: the thread's MMA accumulator fragments of dW2 (dW1^T);  gW3p / gb2p / gb1p: partial sums over the thread's
   //   8-sample group (combined across the 4 groups at the end);  gOut / gLs / loss sums: per sample slot (threads 0..31)
+  //   (SDE: gLs holds the partial sums of dvar_sj h2_sk^2 over the thread's 8-sample group for k = fk, all six j)
   float gW2[2][4][4], gW1[2][1][4], gW3p[ACT + 1], gb2p[2] = {0, 0}, gb1p[2] = {0, 0}, gOut[ACT + 1], gLs[ACT];
   float sPg = 0.0f, sV = 0.0f, sKl = 0.0f;
 #pragma unroll
@@ -760,6 +904,33 @@ __global__ void __launch_bounds__(NT, 2) grad_kernel(Layout L, const float* __re
       }
       if (t == 0) head_forward_g<ACT>(W, H2, out, scratch);
       else head_forward_g<1>(W, H2, out, scratch);
+      if constexpr (SDE) {
+        if (t == 0) {  // var[j][s] = sum_k fl(h2_ks^2) S_kj: the head's shape and order (4 groups of 16 k), h2^2 in, S as weights
+          const GradSde X2 = GradSde::at(ls);
+          const float *sS = X2.S;
+          float* sVar = X2.var;
+          const int kg = tid >> 5, s = tid & 31;
+          if (tid < 4 * GT) {
+            float acc[ACT];
+#pragma unroll
+            for (int j = 0; j < ACT; j++) acc[j] = 0.0f;
+#pragma unroll
+            for (int k = 16 * kg; k < 16 * kg + 16; k++) {
+              const float h = H2[k * LDG + s], h2 = h * h;
+#pragma unroll
+              for (int j = 0; j < ACT; j++) acc[j] = fmaf(h2, sS[k * ACT + j], acc[j]);
+            }
+#pragma unroll
+            for (int j = 0; j < ACT; j++) scratch[(kg * 8 + j) * GT + s] = acc[j];
+          }
+          __syncthreads();
+          for (int e = tid; e < ACT * GT; e += NT) {
+            const int j = e / GT, c = e % GT;
+            sVar[e] = (scratch[j * GT + c] + scratch[(8 + j) * GT + c]) + (scratch[(16 + j) * GT + c] + scratch[(24 + j) * GT + c]);
+          }
+          __syncthreads();
+        }
+      }
       // ---- loss and its gradient with respect to the head outputs (one thread per sample)
       if (tid < GT) {
         const float valid = sValid[tid];
@@ -767,9 +938,16 @@ __global__ void __launch_bounds__(NT, 2) grad_kernel(Layout L, const float* __re
           float lp = 0.0f, d[ACT], isig2[ACT];
 #pragma unroll
           for (int k = 0; k < ACT; k++) {
-            isig2[k] = expf(-2.0f * ls[k]);
-            d[k] = sAct[k * GT + tid] - out[k * GT + tid];
-            lp += -0.5f * d[k] * d[k] * isig2[k] - ls[k] - LOG_SQRT_2PI;
+            if constexpr (SDE) {
+              const float v = GradSde::at(ls).var[k * GT + tid] + kSdeEps;
+              isig2[k] = 1.0f / v;
+              d[k] = sAct[k * GT + tid] - out[k * GT + tid];
+              lp += sde_logp_term(d[k], v, isig2[k]);
+            } else {
+              isig2[k] = expf(-2.0f * ls[k]);
+              d[k] = sAct[k * GT + tid] - out[k * GT + tid];
+              lp += -0.5f * d[k] * d[k] * isig2[k] - ls[k] - LOG_SQRT_2PI;
+            }
           }
           const float lr = lp - sOld[tid], ratio = expf(lr);
           const float A = (sAdv[tid] - a_mean) * a_rstd;
@@ -787,7 +965,9 @@ __global__ void __launch_bounds__(NT, 2) grad_kernel(Layout L, const float* __re
             const float dm = dlp * d[k] * isig2[k];
             dOut[k * GT + tid] = dm;
             gOut[k] += dm;  // d b3
-            gLs[k] += dlp * (d[k] * d[k] * isig2[k] - 1.0f) - ent_coef * inv_mb * valid;
+            // d/d log_std of the diagonal Gaussian; for gSDE the same bracket is d/d log(var): dL/dvar = bracket / (2 var)
+            if constexpr (SDE) GradSde::at(ls).dvar[k * GT + tid] = 0.5f * (dlp * (d[k] * d[k] * isig2[k] - 1.0f) - ent_coef * inv_mb * valid) * isig2[k];
+            else gLs[k] += dlp * (d[k] * d[k] * isig2[k] - 1.0f) - ent_coef * inv_mb * valid;
           }
           sPg += -fminf(x1, x2) * valid;
           sKl += ((ratio - 1.0f) - lr) * valid;
@@ -867,6 +1047,16 @@ __global__ void __launch_bounds__(NT, 2) grad_kernel(Layout L, const float* __re
           float& acc = gW3p[t == 0 ? q : ACT];
           acc = fmaf(g4.x, h[0], acc); acc = fmaf(g4.y, h[1], acc); acc = fmaf(g4.z, h[2], acc); acc = fmaf(g4.w, h[3], acc);
         }
+        if constexpr (SDE) {
+          if (t == 0) {  // sum_s dvar_sj fl(h2_sk^2): dW3's sum with h2^2 in place of h2
+#pragma unroll
+            for (int j = 0; j < ACT; j++) {
+              const float4 g4 = *reinterpret_cast<const float4*>(GradSde::at(ls).dvar + j * GT + s0);
+              float& acc = gLs[j];
+              acc = fmaf(g4.x, h[0] * h[0], acc); acc = fmaf(g4.y, h[1] * h[1], acc); acc = fmaf(g4.z, h[2] * h[2], acc); acc = fmaf(g4.w, h[3] * h[3], acc);
+            }
+          }
+        }
       }
       __syncthreads();  // the next tower (or tile) overwrites the activation buffers
     }
@@ -892,7 +1082,17 @@ __global__ void __launch_bounds__(NT, 2) grad_kernel(Layout L, const float* __re
   for (int o = 0; o < ACT + 1; o++) scr[(sg * 8 + o) * HID + fk] = gW3p[o];
 #pragma unroll
   for (int t = 0; t < 2; t++) { scr[2048 + (2 * t) * 256 + sg * HID + fk] = gb2p[t]; scr[2048 + (2 * t + 1) * 256 + sg * HID + fk] = gb1p[t]; }
+  if constexpr (SDE) {
+    for (int j = 0; j < ACT; j++) scr[3072 + (sg * ACT + j) * HID + fk] = gLs[j];
+  }
   __syncthreads();
+  if constexpr (SDE) {  // d log_std_kj = 2 S_kj sum_s dvar_sj h2_sk^2, the four sample groups combined as for dW3
+    for (int e = tid; e < HID * ACT; e += NT) {
+      const int k = e / ACT, j = e % ACT;
+      const float* q = scr + 3072 + j * HID + k;
+      G[L.log_std + e] = 2.0f * GradSde::at(ls).S[e] * ((q[0] + q[ACT * HID]) + (q[2 * ACT * HID] + q[3 * ACT * HID]));
+    }
+  }
   for (int e = tid; e < (ACT + 1) * HID; e += NT) {
     const int o = e / HID, k = e % HID;
     const float v = (scr[o * HID + k] + scr[(8 + o) * HID + k]) + (scr[(16 + o) * HID + k] + scr[(24 + o) * HID + k]);
@@ -911,7 +1111,7 @@ __global__ void __launch_bounds__(NT, 2) grad_kernel(Layout L, const float* __re
     scr[12 * GT + tid] = gOut[ACT]; scr[13 * GT + tid] = sPg; scr[14 * GT + tid] = sV; scr[15 * GT + tid] = sKl;
   }
   __syncthreads();
-  if (tid < 16) {
+  if (tid < 16 && !(SDE && tid >= ACT && tid < 2 * ACT)) {  // (gSDE: log_std was written above)
     float v = 0.0f;
     for (int k = 0; k < GT; k++) v += scr[tid * GT + k];
     const int dst = tid < ACT ? L.b3[0] + tid : tid < 2 * ACT ? L.log_std + tid - ACT : tid == 12 ? L.b3[1] : L.total + tid - 13;
@@ -974,6 +1174,14 @@ int64_t so100_ppo_workspace_floats(int obs_dim) {
   const int n = so100_ppo_param_count(obs_dim);
   return n < 0 ? n : (int64_t)SO100_PPO_MAX_CTAS * (n + 4) + 4 * ppo::kStatCtas;
 }
+int so100_ppo_sde_param_count(int obs_dim) {
+  if (obs_dim < 1 || obs_dim > ppo::K1) return fail(SO100_ERR_ARG, "obs_dim must be 1..16");
+  return ppo::make_layout(obs_dim, true).total;
+}
+int64_t so100_ppo_sde_workspace_floats(int obs_dim) {
+  const int n = so100_ppo_sde_param_count(obs_dim);
+  return n < 0 ? n : (int64_t)SO100_PPO_MAX_CTAS * (n + 4) + 4 * ppo::kStatCtas;
+}
 
 // The learner's buffers say which GPU they live on: make it current (the entry points take no device argument, and the
 // caller's current device need not be the one its tensors are on).
@@ -992,8 +1200,10 @@ static int ppo_smem_optin(const void* fn, int floats) {  // per device; the call
   return SO100_OK;
 }
 
-int so100_ppo_act(int obs_dim, const float* params, const float* obs, int n, uint64_t seed, int64_t env_offset, uint32_t tick,
-                  int deterministic, float* act_raw, float* act_clip, float* logp, float* value, float* obs_copy, void* stream) {
+extern "C++" {
+template <bool SDE>
+static int ppo_act(int obs_dim, const float* params, const float* obs, int n, uint64_t seed, int64_t env_offset, uint32_t tick,
+                   int deterministic, float* act_raw, float* act_clip, float* logp, float* value, float* obs_copy, void* stream) {
   if (so100_ppo_param_count(obs_dim) < 0) return SO100_ERR_ARG;
   if (!params || !obs || n <= 0) return fail(SO100_ERR_ARG, "bad argument");
   int rc = ppo_use_device_of(params);
@@ -1001,24 +1211,37 @@ int so100_ppo_act(int obs_dim, const float* params, const float* obs, int n, uin
   int dev = 0, sms = 0;
   CU(cudaGetDevice(&dev));
   CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  const ppo::Layout L = ppo::make_layout(obs_dim, SDE);
   static const bool use_mma = getenv("SO100_PPO_ACT_MMA") != nullptr;  // A/B knob: the warp-level mma.sync version
   if (!use_mma) {  // tcgen05 / TMEM: 128-sample tiles, two persistent CTAs per SM
-    CU(cudaFuncSetAttribute((const void*)ppo::act_kernel_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, ppo::ActTc::BYTES));
+    const int bytes = SDE ? ppo::ActTc::BYTES_SDE : ppo::ActTc::BYTES;
+    CU(cudaFuncSetAttribute((const void*)ppo::act_kernel_tc<SDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
     const int ntiles = (n + ppo::TM - 1) / ppo::TM, grid = ntiles < 2 * sms ? ntiles : 2 * sms;
-    ppo::act_kernel_tc<<<grid, ppo::NTC, ppo::ActTc::BYTES, (cudaStream_t)stream>>>(
-        ppo::make_layout(obs_dim), params, obs, n, (unsigned)(seed & 0xFFFFFFFFull), (unsigned)(seed >> 32), env_offset, tick, deterministic,
+    ppo::act_kernel_tc<SDE><<<grid, ppo::NTC, bytes, (cudaStream_t)stream>>>(
+        L, params, obs, n, (unsigned)(seed & 0xFFFFFFFFull), (unsigned)(seed >> 32), env_offset, tick, deterministic,
         act_raw, act_clip, logp, value, obs_copy);
     CU(cudaGetLastError());
     return SO100_OK;
   }
-  rc = ppo_smem_optin((const void*)ppo::act_kernel, ppo::kActSmemFloats);
+  const int floats = SDE ? ppo::kActSmemFloatsSde : ppo::kActSmemFloats;
+  rc = ppo_smem_optin((const void*)ppo::act_kernel<SDE>, floats);
   if (rc) return rc;
-  const int ntiles = (n + ppo::TB - 1) / ppo::TB, grid = ntiles < 2 * sms ? ntiles : 2 * sms;  // 85 KB of shared memory: two CTAs per SM
-  ppo::act_kernel<<<grid, ppo::NT, ppo::kActSmemFloats * 4, (cudaStream_t)stream>>>(
-      ppo::make_layout(obs_dim), params, obs, n, (unsigned)(seed & 0xFFFFFFFFull), (unsigned)(seed >> 32), env_offset, tick, deterministic,
+  const int ntiles = (n + ppo::TB - 1) / ppo::TB, grid = ntiles < 2 * sms ? ntiles : 2 * sms;  // ~103 KB of shared memory: two CTAs per SM
+  ppo::act_kernel<SDE><<<grid, ppo::NT, floats * 4, (cudaStream_t)stream>>>(
+      L, params, obs, n, (unsigned)(seed & 0xFFFFFFFFull), (unsigned)(seed >> 32), env_offset, tick, deterministic,
       act_raw, act_clip, logp, value, obs_copy);
   CU(cudaGetLastError());
   return SO100_OK;
+}
+}  // extern "C++"
+
+int so100_ppo_act(int obs_dim, const float* params, const float* obs, int n, uint64_t seed, int64_t env_offset, uint32_t tick,
+                  int deterministic, float* act_raw, float* act_clip, float* logp, float* value, float* obs_copy, void* stream) {
+  return ppo_act<false>(obs_dim, params, obs, n, seed, env_offset, tick, deterministic, act_raw, act_clip, logp, value, obs_copy, stream);
+}
+int so100_ppo_sde_act(int obs_dim, const float* params, const float* obs, int n, uint64_t seed, int64_t env_offset, uint32_t noise_key,
+                      int deterministic, float* act_raw, float* act_clip, float* logp, float* value, float* obs_copy, void* stream) {
+  return ppo_act<true>(obs_dim, params, obs, n, seed, env_offset, noise_key, deterministic, act_raw, act_clip, logp, value, obs_copy, stream);
 }
 
 int so100_ppo_post_step(int obs_dim, const float* params, int n, const float* reward, const uint8_t* terminated, const uint8_t* truncated,
@@ -1054,15 +1277,18 @@ int so100_ppo_permutation(int n, uint64_t key, int64_t* idx_out, void* stream) {
   return SO100_OK;
 }
 
-int so100_ppo_grad(int obs_dim, const float* params, const float* obs, const float* act, const float* logp_old, const float* adv,
-                   const float* ret, const int64_t* idx, int mb, float clip_range, float vf_coef, float ent_coef, int normalize,
-                   float* workspace, float* grad, float* loss_out, void* stream) {
+extern "C++" {
+template <bool SDE>
+static int ppo_grad(int obs_dim, const float* params, const float* obs, const float* act, const float* logp_old, const float* adv,
+                    const float* ret, const int64_t* idx, int mb, float clip_range, float vf_coef, float ent_coef, int normalize,
+                    float* workspace, float* grad, float* loss_out, void* stream) {
   if (so100_ppo_param_count(obs_dim) < 0) return SO100_ERR_ARG;
   if (!params || !obs || !act || !logp_old || !adv || !ret || !idx || mb <= 0 || !workspace || !grad) return fail(SO100_ERR_ARG, "bad argument");
-  const ppo::Layout L = ppo::make_layout(obs_dim);
+  const ppo::Layout L = ppo::make_layout(obs_dim, SDE);
+  const int smem_floats = SDE ? ppo::kGradSmemFloatsSde : ppo::kGradSmemFloats;
   int rc = ppo_use_device_of(params);
   if (rc) return rc;
-  rc = ppo_smem_optin((const void*)ppo::grad_kernel, ppo::kGradSmemFloats);
+  rc = ppo_smem_optin((const void*)ppo::grad_kernel<SDE>, smem_floats);
   if (rc) return rc;
   int dev = 0, sms = 0;
   CU(cudaGetDevice(&dev));
@@ -1075,11 +1301,25 @@ int so100_ppo_grad(int obs_dim, const float* params, const float* obs, const flo
   double* stats = reinterpret_cast<double*>(workspace + (size_t)SO100_PPO_MAX_CTAS * (L.total + 4));
   normalize = normalize && mb > 1;  // SB3 normalises only when len(advantages) > 1: one sample keeps its raw advantage
   if (normalize) ppo::adv_stats_kernel<<<ppo::kStatCtas, 256, 0, st>>>(adv, idx, mb, stats);
-  ppo::grad_kernel<<<grid, ppo::NT, ppo::kGradSmemFloats * 4, st>>>(L, params, obs, act, logp_old, adv, ret, idx, mb, stats, clip_range, vf_coef,
-                                                                   ent_coef, normalize, workspace);
+  ppo::grad_kernel<SDE><<<grid, ppo::NT, smem_floats * 4, st>>>(L, params, obs, act, logp_old, adv, ret, idx, mb, stats, clip_range, vf_coef,
+                                                               ent_coef, normalize, workspace);
   ppo::reduce_kernel<<<(L.total + 3 + 255) / 256, 256, 0, st>>>(workspace, grid, L.total, mb, grad, loss_out);
   CU(cudaGetLastError());
   return SO100_OK;
+}
+}  // extern "C++"
+
+int so100_ppo_grad(int obs_dim, const float* params, const float* obs, const float* act, const float* logp_old, const float* adv,
+                   const float* ret, const int64_t* idx, int mb, float clip_range, float vf_coef, float ent_coef, int normalize,
+                   float* workspace, float* grad, float* loss_out, void* stream) {
+  return ppo_grad<false>(obs_dim, params, obs, act, logp_old, adv, ret, idx, mb, clip_range, vf_coef, ent_coef, normalize, workspace, grad,
+                         loss_out, stream);
+}
+int so100_ppo_sde_grad(int obs_dim, const float* params, const float* obs, const float* act, const float* logp_old, const float* adv,
+                       const float* ret, const int64_t* idx, int mb, float clip_range, float vf_coef, float ent_coef, int normalize,
+                       float* workspace, float* grad, float* loss_out, void* stream) {
+  return ppo_grad<true>(obs_dim, params, obs, act, logp_old, adv, ret, idx, mb, clip_range, vf_coef, ent_coef, normalize, workspace, grad,
+                        loss_out, stream);
 }
 
 int so100_ppo_adam(int n_params, float* params, const float* grad, float* exp_avg, float* exp_avg_sq, int32_t* step_count, float grad_scale,

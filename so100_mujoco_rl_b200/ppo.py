@@ -18,11 +18,16 @@ Two learners share the hyper-parameters, the rollout geometry and the `learn()` 
                   forward + loss + backward per minibatch (`so100_ppo_grad`) and clip + Adam (`so100_ppo_adam`); torch only
                   owns the buffers, draws the minibatch permutation and runs the NCCL all-reduce.
 
+Both support SB3's `use_sde=True` / `sde_sample_freq` (generalized State-Dependent Exploration, DESIGN.md §7d): the action
+noise is h E with h the policy tower's last hidden layer and E a 64x6 matrix per env redrawn once per rollout (or every
+`sde_sample_freq` steps), so the commanded actions change only as fast as the state does.
+
 Data parallel: one process per GPU, each with its own env shard; gradients are averaged with ONE flat all-reduce per
 minibatch (NCCL over NVLink; ~10 k fp32 values, latency bound).  The env step path itself has no collective.
 """
 from __future__ import annotations
 
+import dataclasses
 import math
 import time
 from dataclasses import dataclass, field
@@ -38,23 +43,56 @@ def _ortho(layer: nn.Linear, gain: float) -> nn.Linear:
     return layer
 
 
-class MlpPolicy(nn.Module):
-    """SB3 ActorCriticPolicy with net_arch dict(pi=[64, 64], vf=[64, 64]), tanh, DiagGaussian head."""
+SDE_EPS = 1e-6  # StateDependentNoiseDistribution.epsilon
 
-    def __init__(self, obs_dim: int, act_dim: int, hidden: int = 64, log_std_init: float = 0.0):
+
+class MlpPolicy(nn.Module):
+    """SB3 ActorCriticPolicy with net_arch dict(pi=[64, 64], vf=[64, 64]), tanh, DiagGaussian head; with use_sde=True
+    SB3's StateDependentNoiseDistribution (full_std, no expln, learn_features=False): log_std is [hidden, act_dim]."""
+
+    def __init__(self, obs_dim: int, act_dim: int, hidden: int = 64, log_std_init: float = 0.0, use_sde: bool = False):
         super().__init__()
         g = math.sqrt(2.0)
         self.pi = nn.Sequential(_ortho(nn.Linear(obs_dim, hidden), g), nn.Tanh(), _ortho(nn.Linear(hidden, hidden), g), nn.Tanh())
         self.vf = nn.Sequential(_ortho(nn.Linear(obs_dim, hidden), g), nn.Tanh(), _ortho(nn.Linear(hidden, hidden), g), nn.Tanh())
         self.action_net = _ortho(nn.Linear(hidden, act_dim), 0.01)
         self.value_net = _ortho(nn.Linear(hidden, 1), 1.0)
-        self.log_std = nn.Parameter(torch.full((act_dim,), float(log_std_init)))
+        self.use_sde = bool(use_sde)
+        self.log_std = nn.Parameter(torch.full((hidden, act_dim) if self.use_sde else (act_dim,), float(log_std_init)))
+        self.exploration_mat = self.exploration_matrices = None  # gSDE: drawn by reset_noise
 
     def value(self, obs: torch.Tensor) -> torch.Tensor:
         return self.value_net(self.vf(obs)).squeeze(-1)
 
+    def _dist(self, obs: torch.Tensor):
+        """(h, mean, log scale): the log scale is log_std itself, or per sample for gSDE: 0.5 log(h^2 exp(2 log_std) + eps),
+        with h detached (learn_features=False: the variance sends gradient to log_std only)."""
+        h = self.pi(obs)
+        mean = self.action_net(h)
+        if not self.use_sde:
+            return h, mean, self.log_std
+        var = (h.detach() ** 2) @ torch.exp(self.log_std) ** 2
+        return h, mean, 0.5 * torch.log(var + SDE_EPS)
+
     def dist_params(self, obs: torch.Tensor):
-        return self.action_net(self.pi(obs)), self.log_std
+        _, mean, log_std = self._dist(obs)
+        return mean, log_std
+
+    def reset_noise(self, n_envs: int = 1) -> None:
+        """StateDependentNoiseDistribution.sample_weights: E ~ Normal(0, exp(log_std)), one matrix per env (and one shared)."""
+        with torch.no_grad():
+            std = torch.exp(self.log_std)
+            self.exploration_mat = std * torch.randn_like(std)
+            self.exploration_matrices = std * torch.randn((n_envs, *std.shape), device=std.device, dtype=std.dtype)
+
+    def sde_noise(self, h: torch.Tensor) -> torch.Tensor:
+        """h E per sample (SB3 get_noise): bmm with the per-env matrices, or the shared matrix when the batch differs."""
+        if self.exploration_mat is None:
+            self.reset_noise(h.shape[0])
+        h = h.detach()
+        if h.shape[0] == 1 or h.shape[0] != self.exploration_matrices.shape[0]:
+            return h @ self.exploration_mat
+        return torch.bmm(h.unsqueeze(1), self.exploration_matrices).squeeze(1)
 
     @staticmethod
     def log_prob(mean, log_std, actions):
@@ -62,8 +100,13 @@ class MlpPolicy(nn.Module):
         return (-((actions - mean) ** 2) / (2 * var) - log_std - 0.5 * math.log(2 * math.pi)).sum(-1)
 
     def act(self, obs: torch.Tensor, deterministic: bool = False):
-        mean, log_std = self.dist_params(obs)
-        a = mean if deterministic else mean + torch.exp(log_std) * torch.randn_like(mean)
+        h, mean, log_std = self._dist(obs)
+        if deterministic:
+            a = mean
+        elif self.use_sde:
+            a = mean + self.sde_noise(h)
+        else:
+            a = mean + torch.exp(log_std) * torch.randn_like(mean)
         return a, self.log_prob(mean, log_std, a), self.value(obs)
 
     def evaluate(self, obs, actions):
@@ -112,13 +155,25 @@ def compute_gae(rewards, values, dones, last_value, gamma: float, lam: float):
     return adv, adv + values
 
 
-def param_layout(obs_dim: int, act_dim: int = 6, hidden: int = 64):
-    """(name, shape) in the order of the flat parameter vector of include/so100_ppo.h."""
+def param_layout(obs_dim: int, act_dim: int = 6, hidden: int = 64, use_sde: bool = False):
+    """(name, shape) in the order of the flat parameter vector of include/so100_ppo.h (gSDE: log_std [hidden, act_dim])."""
     out = []
     for tower, nout in (("pi", act_dim), ("vf", 1)):
         out += [(f"{tower}.W1", (hidden, obs_dim)), (f"{tower}.b1", (hidden,)), (f"{tower}.W2", (hidden, hidden)),
                 (f"{tower}.b2", (hidden,)), (f"{tower}.W3", (nout, hidden)), (f"{tower}.b3", (nout,))]
-    return out + [("log_std", (act_dim,))]
+    return out + [("log_std", (hidden, act_dim) if use_sde else (act_dim,))]
+
+
+def sde_redraw(t: int, sample_freq: int) -> bool:
+    """SB3 collect_rollouts: reset_noise at the start of every rollout and, when sample_freq > 0, at every rollout step t
+    with t % sample_freq == 0."""
+    return t == 0 or (sample_freq > 0 and t % sample_freq == 0)
+
+
+def sde_noise_key(t: int, tick: int, sample_freq: int, key: int) -> int:
+    """Noise key of the exploration matrices at rollout step t: the current tick where a fresh draw starts, else the key
+    in use."""
+    return tick if sde_redraw(t, sample_freq) else key
 
 
 def _policy_tensors(policy: "MlpPolicy"):
@@ -158,6 +213,9 @@ class PPOConfig:
     normalize_advantage: bool = True
     seed: int = 0
     cuda_graph: bool = True  # capture one optimiser step (the 2x64 MLPs are launch-bound: ~10x faster updates)
+    use_sde: bool = False    # gSDE exploration (SB3 use_sde)
+    sde_sample_freq: int = -1  # redraw the exploration matrices every n steps; -1: once per rollout (SB3 sde_sample_freq)
+    log_std_init: float = 0.0  # SB3's policy kwarg, for both distributions
 
 
 @dataclass
@@ -211,7 +269,7 @@ class PPO(_LearnLoop):
         self.env, self.cfg = env, cfg or PPOConfig()
         self.device = env.device
         torch.manual_seed(self.cfg.seed)
-        self.policy = MlpPolicy(env.obs_dim, env.act_dim).to(self.device)
+        self.policy = MlpPolicy(env.obs_dim, env.act_dim, log_std_init=self.cfg.log_std_init, use_sde=self.cfg.use_sde).to(self.device)
         self.opt = torch.optim.Adam(self.policy.parameters(), lr=self.cfg.lr, eps=1e-5,
                                     capturable=self.device.type == "cuda" and self.cfg.cuda_graph)
         self.world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
@@ -233,6 +291,8 @@ class PPO(_LearnLoop):
     def collect(self):
         cfg, b = self.cfg, self.buf
         for t in range(cfg.n_steps):
+            if cfg.use_sde and sde_redraw(t, cfg.sde_sample_freq):
+                self.policy.reset_noise(self.env.num_envs)
             a, logp, v = self.policy.act(self.obs)
             b["obs"][t], b["act"][t], b["logp"][t], b["val"][t] = self.obs, a, logp, v
             r = self.env.step(torch.clamp(a, -1.0, 1.0))  # SB3 clips Box actions before env.step (logp is of the raw action)
@@ -353,7 +413,8 @@ class PPO(_LearnLoop):
 
     def state_dict(self) -> dict:
         """Everything a resumed run needs: weights, Adam moments and step, sample counter."""
-        return {"kind": "torch", "policy": self.policy.state_dict(), "optimizer": self.opt.state_dict(), "samples": self.stats.samples}
+        return {"kind": "torch", "policy": self.policy.state_dict(), "optimizer": self.opt.state_dict(), "samples": self.stats.samples,
+                "config": dataclasses.asdict(self.cfg)}
 
     def load_state_dict(self, sd: dict) -> None:
         self.policy.load_state_dict(sd["policy"])
@@ -379,9 +440,13 @@ class FusedPPO(_LearnLoop):
             raise ValueError("FusedPPO runs on CUDA devices only (use PPO for CPU tensors)")
         self._L, self._check, self._ct = _native.lib(), _native.check, ctypes
         self.od, n, T = env.obs_dim, env.num_envs, self.cfg.n_steps
-        self.n_params = self._check(self._L.so100_ppo_param_count(self.od))
+        self.sde = bool(self.cfg.use_sde)  # gSDE: the _sde_ entry points for act and grad, the shared ones for the rest
+        self._act_fn = self._L.so100_ppo_sde_act if self.sde else self._L.so100_ppo_act
+        self._grad_fn = self._L.so100_ppo_sde_grad if self.sde else self._L.so100_ppo_grad
+        self.n_params = self._check((self._L.so100_ppo_sde_param_count if self.sde else self._L.so100_ppo_param_count)(self.od))
+        self.n_log_std = 64 * env.act_dim if self.sde else env.act_dim
         torch.manual_seed(self.cfg.seed)
-        self.params = pack_params(MlpPolicy(self.od, env.act_dim)).to(self.device)
+        self.params = pack_params(self._new_policy()).to(self.device)
         self.world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
         if self.world > 1:
             dist.broadcast(self.params, src=0)
@@ -389,7 +454,8 @@ class FusedPPO(_LearnLoop):
         self.exp_avg, self.exp_avg_sq = torch.zeros(self.n_params, **f), torch.zeros(self.n_params, **f)
         self.grad = torch.zeros(self.n_params, **f)
         self.step_count = torch.zeros(1, device=self.device, dtype=torch.int32)
-        self.workspace = torch.zeros(int(self._L.so100_ppo_workspace_floats(self.od)), **f)
+        ws = self._L.so100_ppo_sde_workspace_floats if self.sde else self._L.so100_ppo_workspace_floats
+        self.workspace = torch.zeros(int(ws(self.od)), **f)
         self.loss = torch.zeros(3, **f)
         self.buf = {"obs": torch.zeros((T, n, self.od), **f), "act": torch.zeros((T, n, env.act_dim), **f), "logp": torch.zeros((T, n), **f),
                     "val": torch.zeros((T, n), **f), "rew": torch.zeros((T, n), **f), "done": torch.zeros((T, n), **f)}
@@ -397,6 +463,7 @@ class FusedPPO(_LearnLoop):
         self.act_clip, self.last_val = torch.zeros((n, env.act_dim), **f), torch.zeros(n, **f)
         self._acc = torch.zeros(4, device=self.device, dtype=torch.float64)
         self.env_offset, self.tick = int(env_offset), 0
+        self.sde_key = 0  # gSDE: noise key of the exploration matrices in use
         self._perm, self._epoch = None, 0
         self.obs = env.reset()
         self.stats = PPOStats()
@@ -404,15 +471,19 @@ class FusedPPO(_LearnLoop):
     def _stream(self) -> int:
         return torch.cuda.current_stream(self.device).cuda_stream
 
+    def _new_policy(self) -> MlpPolicy:
+        return MlpPolicy(self.od, 6, log_std_init=self.cfg.log_std_init, use_sde=self.sde)
+
     def act(self, obs: torch.Tensor, deterministic: bool = False):
-        """Policy inference on arbitrary observations [n, od] -> (raw action, clipped action, log-prob, value)."""
+        """Policy inference on arbitrary observations [n, od] -> (raw action, clipped action, log-prob, value).
+        gSDE draws with the exploration matrices in use (those of the last rollout step)."""
         n = obs.shape[0]
         f = dict(device=self.device, dtype=torch.float32)
         a, c, lp, v = torch.empty((n, 6), **f), torch.empty((n, 6), **f), torch.empty(n, **f), torch.empty(n, **f)
         self.tick += 1
-        self._check(self._L.so100_ppo_act(self.od, self.params.data_ptr(), obs.contiguous().data_ptr(), n, self.cfg.seed, self.env_offset,
-                                          self.tick, int(deterministic), a.data_ptr(), c.data_ptr(), lp.data_ptr(), v.data_ptr(), None,
-                                          self._stream()))
+        self._check(self._act_fn(self.od, self.params.data_ptr(), obs.contiguous().data_ptr(), n, self.cfg.seed, self.env_offset,
+                                 self.sde_key if self.sde else self.tick, int(deterministic), a.data_ptr(), c.data_ptr(), lp.data_ptr(),
+                                 v.data_ptr(), None, self._stream()))
         return a, c, lp, v
 
     @torch.no_grad()
@@ -421,15 +492,18 @@ class FusedPPO(_LearnLoop):
         n = self.env.num_envs
         for t in range(cfg.n_steps):
             self.tick += 1
-            self._check(L.so100_ppo_act(self.od, P, self.obs.data_ptr(), n, cfg.seed, self.env_offset, self.tick, 0, b["act"][t].data_ptr(),
-                                        self.act_clip.data_ptr(), b["logp"][t].data_ptr(), b["val"][t].data_ptr(), b["obs"][t].data_ptr(), st))
+            key = self.tick
+            if self.sde:
+                key = self.sde_key = sde_noise_key(t, self.tick, cfg.sde_sample_freq, self.sde_key)
+            self._check(self._act_fn(self.od, P, self.obs.data_ptr(), n, cfg.seed, self.env_offset, key, 0, b["act"][t].data_ptr(),
+                                     self.act_clip.data_ptr(), b["logp"][t].data_ptr(), b["val"][t].data_ptr(), b["obs"][t].data_ptr(), st))
             r = self.env.step(self.act_clip)  # SB3 clips Box actions before env.step (the log-prob is of the raw action)
             self._check(L.so100_ppo_post_step(self.od, P, n, r.reward.data_ptr(), r.terminated.data_ptr(), r.truncated.data_ptr(),
                                               r.terminal_obs.data_ptr(), r.ep_return.data_ptr(), r.ep_len.data_ptr(), cfg.gamma,
                                               b["rew"][t].data_ptr(), b["done"][t].data_ptr(), self._acc.data_ptr(), st))
             self.obs = r.obs
-        self._check(L.so100_ppo_act(self.od, P, self.obs.data_ptr(), n, cfg.seed, self.env_offset, self.tick, 1, None, None, None,
-                                    self.last_val.data_ptr(), None, st))
+        self._check(self._act_fn(self.od, P, self.obs.data_ptr(), n, cfg.seed, self.env_offset, self.tick, 1, None, None, None,
+                                 self.last_val.data_ptr(), None, st))
         self._check(L.so100_ppo_gae(b["rew"].data_ptr(), b["val"].data_ptr(), b["done"].data_ptr(), self.last_val.data_ptr(), cfg.n_steps, n,
                                     cfg.gamma, cfg.gae_lambda, self.adv.data_ptr(), self.ret.data_ptr(), st))
         return self.adv, self.ret
@@ -437,7 +511,7 @@ class FusedPPO(_LearnLoop):
     def minibatch_step(self, idx: torch.Tensor, adv: torch.Tensor, ret: torch.Tensor):
         """One optimiser step on the samples idx (int64, device) of the flattened rollout buffers."""
         cfg, b, L, st = self.cfg, self.buf, self._L, self._stream()
-        self._check(L.so100_ppo_grad(self.od, self.params.data_ptr(), b["obs"].data_ptr(), b["act"].data_ptr(), b["logp"].data_ptr(),
+        self._check(self._grad_fn(self.od, self.params.data_ptr(), b["obs"].data_ptr(), b["act"].data_ptr(), b["logp"].data_ptr(),
                                      adv.data_ptr(), ret.data_ptr(), idx.data_ptr(), idx.numel(), cfg.clip_range, cfg.vf_coef, cfg.ent_coef,
                                      int(cfg.normalize_advantage), self.workspace.data_ptr(), self.grad.data_ptr(), self.loss.data_ptr(), st))
         if self.world > 1:
@@ -462,29 +536,33 @@ class FusedPPO(_LearnLoop):
         return {"pg_loss": pg, "v_loss": vl, "approx_kl": kl}
 
     def _log_std_mean(self) -> float:
-        return float(self.params[-6:].mean())
+        return float(self.params[-self.n_log_std:].mean())
 
     def load_policy(self, policy: MlpPolicy) -> None:
         """Continue from the weights of a torch MlpPolicy (Adam moments restart)."""
+        if policy.use_sde != self.sde:
+            raise ValueError(f"the policy {'uses' if policy.use_sde else 'does not use'} gSDE and the learner {'does' if self.sde else 'does not'}")
         self.params.copy_(pack_params(policy).to(self.device))
         self.exp_avg.zero_(); self.exp_avg_sq.zero_(); self.step_count.zero_()
 
     def state_dict(self) -> dict:
         """Everything a resumed run needs: weights (as an MlpPolicy state dict), Adam moments and step, counters."""
         return {"kind": "fused", "policy": self.policy.state_dict(), "exp_avg": self.exp_avg.clone(), "exp_avg_sq": self.exp_avg_sq.clone(),
-                "step_count": int(self.step_count.item()), "tick": self.tick, "epoch": self._epoch, "samples": self.stats.samples}
+                "step_count": int(self.step_count.item()), "tick": self.tick, "epoch": self._epoch, "samples": self.stats.samples,
+                "sde_key": self.sde_key, "config": dataclasses.asdict(self.cfg)}
 
     def load_state_dict(self, sd: dict) -> None:
-        pol = MlpPolicy(self.od, 6)
+        pol = self._new_policy()
         pol.load_state_dict(sd["policy"])
         self.load_policy(pol)
         if sd.get("kind") == "fused":
             self.exp_avg.copy_(sd["exp_avg"].to(self.device)); self.exp_avg_sq.copy_(sd["exp_avg_sq"].to(self.device))
             self.step_count.fill_(int(sd["step_count"]))
             self.tick, self._epoch = int(sd.get("tick", 0)), int(sd.get("epoch", 0))
+            self.sde_key = int(sd.get("sde_key", 0))
         self.stats.samples = int(sd.get("samples", 0))
 
     @property
     def policy(self) -> MlpPolicy:
         """The current weights as a torch MlpPolicy (export, evaluation, tests)."""
-        return unpack_params(self.params, MlpPolicy(self.od, 6).to(self.device))
+        return unpack_params(self.params, self._new_policy().to(self.device))
