@@ -556,7 +556,7 @@ __device__ __forceinline__ void physics(const Consts& C, const Bufs& B, EnvRegs&
         }
       }
     }
-    if (!PADS) d = solve_qacc<float>(K, loss, M, b, e.q, e.qc, e.v, e.w, sweeps);
+    if (!PADS) d = solve_qacc<float, true>(K, loss, M, b, e.q, e.qc, e.v, e.w, sweeps);  // every lane is here (barrier above)
     float amax = 1.0f;
 #pragma unroll
     for (int j = 0; j < SO_NJ; j++) {

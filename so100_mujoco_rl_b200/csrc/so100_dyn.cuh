@@ -354,11 +354,15 @@ SO_HD void limit_row(const ConC<T>& K, int j, T m, T q, T qc, T qd, T& xl, T& sD
 // a[] holds the warm start on entry and the solution on exit; returns the largest update of the LAST sweep.
 // qc[] is the compensation term of the fp32 position integration (zeros when T = double).  loss[] is the friction loss of
 // the dofs: K.fr_loss, or an env's own values (so100_set_param_ranges).
-template <typename T>
+// WARP_ROWS (device, all 32 lanes converged at the call): the limit rows are set up and swept per dof on a warp-uniform
+// branch, taken when ANY lane of the warp has a row on that dof; lanes without one keep their values through selects
+// (sDl = 0 makes the row's activity test false), so every lane's result is bit for bit the per-lane branch's.
+template <typename T, bool WARP_ROWS = false>
 SO_HD T solve_qacc(const ConC<T>& K, const T* loss, const T* M, const T* b, const T* q, const T* qc, const T* qd, T* a, int sweeps) {
   // per-dof constants of this substep.  Friction row only:  t = c - m af,  x = af + (t - clamp(t kap, +-loss)) / m
   //   = (af + t rm) - clamp(t kr, +-lr)   with kr = kap rm, lr = loss rm;  bp = b - m af folds "- m af" into the sum.
   T af[SO_NJ], rm[SO_NJ], kr[SO_NJ], lr[SO_NJ], bp[SO_NJ], xl[SO_NJ], sDl[SO_NJ], rm2[SO_NJ], kap2[SO_NJ], dl[SO_NJ];
+  unsigned own = 0u;  // WARP_ROWS: bit j = this lane's joint j is outside its range
 #pragma unroll
   for (int j = 0; j < SO_NJ; j++) {
     T m = M[midx(j, j)];
@@ -367,10 +371,32 @@ SO_HD T solve_qacc(const ConC<T>& K, const T* loss, const T* M, const T* b, cons
     kr[j] = K.fr_D[j] * so_rcp(m + K.fr_D[j]) * rm[j];
     lr[j] = loss[j] * rm[j];
     bp[j] = b[j] - m * af[j];
-    xl[j] = T(0); sDl[j] = T(0); rm2[j] = T(0); kap2[j] = T(0); dl[j] = T(0);
-    if ((q[j] - K.lo[j]) - qc[j] < T(0) || (K.hi[j] - q[j]) + qc[j] < T(0)) {
-      limit_row(K, j, m, q[j], qc[j], qd[j], xl[j], sDl[j], rm2[j], kap2[j]);
-      dl[j] = (sDl[j] < T(0) ? -sDl[j] : sDl[j]) * (xl[j] - af[j]);  // t with the limit row active = t + Dl (xl - af)
+    const bool out = (q[j] - K.lo[j]) - qc[j] < T(0) || (K.hi[j] - q[j]) + qc[j] < T(0);
+    if (WARP_ROWS) {
+      own |= out ? 1u << j : 0u;
+    } else {
+      xl[j] = T(0); sDl[j] = T(0); rm2[j] = T(0); kap2[j] = T(0); dl[j] = T(0);
+      if (out) {
+        limit_row(K, j, m, q[j], qc[j], qd[j], xl[j], sDl[j], rm2[j], kap2[j]);
+        dl[j] = (sDl[j] < T(0) ? -sDl[j] : sDl[j]) * (xl[j] - af[j]);  // t with the limit row active = t + Dl (xl - af)
+      }
+    }
+  }
+  unsigned rows = own;  // WARP_ROWS: bit j = some lane of the warp has a limit row on dof j (xl .. dl are set only then)
+#ifdef __CUDA_ARCH__
+  if (WARP_ROWS) rows = __reduce_or_sync(0xffffffffu, own);
+#endif
+  if (WARP_ROWS) {
+#pragma unroll
+    for (int j = 0; j < SO_NJ; j++) {
+      if (rows & (1u << j)) {
+        T xl_, sDl_, rm2_, kap2_;
+        limit_row(K, j, M[midx(j, j)], q[j], qc[j], qd[j], xl_, sDl_, rm2_, kap2_);
+        const T dl_ = (sDl_ < T(0) ? -sDl_ : sDl_) * (xl_ - af[j]);
+        const bool mine = own & (1u << j);
+        xl[j] = mine ? xl_ : T(0); sDl[j] = mine ? sDl_ : T(0); rm2[j] = mine ? rm2_ : T(0); kap2[j] = mine ? kap2_ : T(0);
+        dl[j] = mine ? dl_ : T(0);
+      }
     }
   }
   T last = T(0), amax = T(1);  // amax: scale of the iterate, refreshed by every tracked sweep (a warm start left by a
@@ -392,7 +418,7 @@ SO_HD T solve_qacc(const ConC<T>& K, const T* loss, const T* M, const T* b, cons
       }
       t -= (prev < j ? M[midx(j, prev)] : M[midx(prev, j)]) * a[prev];
       T x = so_fma(t, rm[j], af[j]) - so_clamp(t * kr[j], -lr[j], lr[j]);
-      if (sDl[j] != T(0)) {  // limit row present: active iff the limit-free minimiser violates it
+      if (WARP_ROWS ? (rows & (1u << j)) != 0u : sDl[j] != T(0)) {  // limit row present: active iff the limit-free minimiser violates it
         T t2 = t + dl[j];
         T x2 = af[j] + (t2 - so_clamp(t2 * kap2[j], -loss[j], loss[j])) * rm2[j];
         x = sDl[j] * (x - xl[j]) < T(0) ? x2 : x;

@@ -38,11 +38,14 @@ class G:
     def __init__(self):
         self.nodes = []  # (kind, a, b) with a/b = node ids, or payload for const/var
         self.memo = {}
+        self.region = None  # the part of the recursion being built: its operations are counted under this name
+        self.node_region = []
 
     def _mk(self, key):
         if key not in self.memo:
             self.memo[key] = len(self.nodes)
             self.nodes.append(key)
+            self.node_region.append(self.region)
         return self.memo[key]
 
     def const(self, x):
@@ -195,6 +198,7 @@ def add_composite(L, m, h, I, pm, ph, pI):
 
 def build(flat):
     g = G()
+    g.region = "RNE forward"  # including the planar merges of the joint angles
     s = [g.var(f"s[{i}]") for i in range(NJ)]
     c = [g.var(f"c[{i}]") for i in range(NJ)]
     qd = [g.var(f"qd[{i}]") for i in range(NJ)]
@@ -223,6 +227,7 @@ def build(flat):
     cm, ch, cI = links[-1].m, links[-1].h, links[-1].I
     for i in range(NJ - 1, -1, -1):
         bias[i] = n[i][2]
+        g.region = "M entries"
         M[(i, i)] = cI[2] + links[i].arm
         cf, cn = [-ch[1], ch[0], zero], [cI[4], cI[5], cI[2]]
         for j in range(i - 1, -1, -1):
@@ -232,10 +237,12 @@ def build(flat):
             M[(i, j)] = cn[2]
         if i > 0:
             L = links[i]
+            g.region = "RNE backward"
             fp = L.to_parent(f[i])
             npv = vadd(L.to_parent(n[i]), cross(L.p, fp))
             f[i - 1] = vadd(f[i - 1], fp)
             n[i - 1] = vadd(n[i - 1], npv)
+            g.region = "composite inertia"
             cm, ch, cI = add_composite(L, cm, ch, cI, links[i - 1].m, links[i - 1].h, links[i - 1].I)
     outs = [(f"bias[{i}]", bias[i]) for i in range(NJ)]
     outs += [(f"M[{i * (i + 1) // 2 + j}]", M[(i, j)]) for i in range(NJ) for j in range(i + 1)]
@@ -283,13 +290,15 @@ def emit(g, outs):
             return a
         return f"t{n}"
 
-    lines, nop = [], {"fma": 0, "mul": 0, "add": 0}
+    nop = {r: {"fma": 0, "mul": 0, "add": 0} for r in dict.fromkeys(g.node_region)}  # regions in recursion order
+    lines = []
     for n in sorted(live):
         k, a, b = g.nodes[n]
         if k in ("const", "var") or n in fused:
             continue
+        cnt = nop[g.node_region[n]]
         if k == "mul":
-            lines.append(f"  const T t{n} = {ref(a)} * {ref(b)};"); nop["mul"] += 1
+            lines.append(f"  const T t{n} = {ref(a)} * {ref(b)};"); cnt["mul"] += 1
             continue
         fa, fb = a in fused, b in fused
         if fa or fb:
@@ -301,9 +310,9 @@ def emit(g, outs):
                 e = f"so_fma({ref(x)}, {ref(y)}, -{ref(o)})"
             else:      # o - m
                 e = f"so_fma(-{ref(x)}, {ref(y)}, {ref(o)})"
-            nop["fma"] += 1
+            cnt["fma"] += 1
         else:
-            e = f"{ref(a)} {'+' if k == 'add' else '-'} {ref(b)}"; nop["add"] += 1
+            e = f"{ref(a)} {'+' if k == 'add' else '-'} {ref(b)}"; cnt["add"] += 1
         lines.append(f"  const T t{n} = {e};")
     for name, v in outs:
         lines.append(f"  {name} = {'-' if v.s < 0 else ''}{ref(v.n)};")
@@ -372,14 +381,19 @@ def render():
     flat = host_constants()
     sflat = host_solver_constants()
     g, outs, planar = build(flat)
-    lines, nop = emit(g, outs)
+    lines, by_region = emit(g, outs)
+    nop = {k: sum(r[k] for r in by_region.values()) for k in ("fma", "mul", "add")}
     hexd = ",\n    ".join(", ".join(float(x).hex() for x in flat[i:i + 4]) for i in range(0, 141, 4))
     total = nop["fma"] + nop["mul"] + nop["add"]
+    regions = "\n".join(f"//   {name:18s} {r['fma']:4d} fma + {r['mul']:4d} mul + {r['add']:4d} add/sub = {sum(r.values()):4d}"
+                        for name, r in by_region.items())
     hdr = f"""// GENERATED by tools/gen_so100_dyn.py from so100_mujoco_rl_b200/assets/so100_scene.xml — do not edit.
 // so100 arm: bias[6] = RNE(q, qd, 0) incl. gravity and M[21] = joint-space inertia (packed lower triangle, armature
 // included), specialised to the model's fp32 constants.  Same recursion as so100_dyn.cuh::dyn_bias_mass.
 // Straight-line: {nop['fma']} fma + {nop['mul']} mul + {nop['add']} add/sub = {total} instructions
 // ({2 * nop['fma'] + nop['mul'] + nop['add']} FLOP); planar-merged links: {[i for i, p in enumerate(planar) if p]}.
+// By the part of the recursion that creates each operation:
+{regions}
 #pragma once
 #include "so100_dyn.cuh"
 
