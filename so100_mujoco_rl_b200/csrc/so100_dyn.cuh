@@ -30,6 +30,20 @@ SO_HD double so_fma(double a, double b, double c) { return a * b + c; }
 template <typename T>
 SO_HD T so_fma(T a, T b, T c) { return a * b + c; }
 
+// A separate multiplication / addition that ptxas may not contract into an fma: the generated dynamics says where it
+// fuses, so every kernel that inlines it rounds the same way whatever the surrounding code.
+#ifdef __CUDA_ARCH__
+SO_HD float so_mul(float a, float b) { return __fmul_rn(a, b); }
+SO_HD float so_add(float a, float b) { return __fadd_rn(a, b); }
+SO_HD float so_sub(float a, float b) { return __fsub_rn(a, b); }
+#endif
+template <typename T>
+SO_HD T so_mul(T a, T b) { return a * b; }
+template <typename T>
+SO_HD T so_add(T a, T b) { return a + b; }
+template <typename T>
+SO_HD T so_sub(T a, T b) { return a - b; }
+
 // sin/cos of a joint angle inside the substep loop.  Device fp32: MUFU.SIN / MUFU.COS (|err| <= 2^-21.2 on [-pi, pi],
 // CUDA C Programming Guide table of intrinsics; joint ranges of this model stay inside +-3.1416).  A 4e-7 error in
 // sin/cos moves a gravity torque of <= 1 N m by 4e-7 N m, i.e. the servo's equilibrium by 1e-8 rad; the task

@@ -3,12 +3,14 @@
 straight-line code specialised to the MJCF's numbers ("model parsed once on the host").
 
 How: the SAME recursion as csrc/so100_dyn.cuh (link-local RNEA + composite rigid bodies) is executed symbolically on a
-hash-consed expression DAG whose leaves are sin/cos of the joint angles, the joint velocities and the fp32-rounded
-link constants the library derives (so100_host_constants).  Folding removes every multiplication by 0.0f / 1.0f /
--1.0f and every addition of 0 (the so100 frames are axis-aligned up to ~6e-6, so most rotation entries fold), links
-whose constant rotation is planar about the joint axis are merged with the joint angle by the angle-addition
-identity, common sub-expressions are shared, and a*b+c is emitted as fmaf.  Folding uses exactly the constants the
-generic kernel multiplies by, so both kernels compute the same fp32 model; only the rounding order differs.
+hash-consed expression DAG whose leaves are sin/cos of the joint angles, the joint velocities and link constants
+derived from the ones the library computes (so100_host_constants).  Every link frame is first turned about its joint
+axis (`reframe`, in fp64, rounded to fp32 once) so that each constant rotation is Rx(alpha) Rz(theta) with alpha a
+quarter turn up to ~1e-5 rad; the Rz(theta) is merged with the joint angle by the angle-addition identity.  Folding
+then removes every multiplication by 0.0f / 1.0f / -1.0f and every addition of 0, common sub-expressions are shared,
+and a*b+c is emitted as an fma.  Bias forces and M do not depend on the frames, so both kernels compute the same
+model; only the fp32 rounding differs.  Every operation is emitted explicitly (so_fma / so_mul / so_add / so_sub), so
+no kernel that inlines the code can contract it differently from another.
 
 The generated header also carries the fp64 constants it was built from; so100_create compares them with the model it
 is given and launches the generic kernel when they differ (any other MJCF still works, only slower).
@@ -135,20 +137,82 @@ def vadd(a, b):
     return [x + y for x, y in zip(a, b)]
 
 
+def _rz(c, s):
+    return np.array([[c, -s, 0.0], [s, c, 0.0], [0.0, 0.0, 1.0]])
+
+
+QUARTER = [(1.0, 0.0), (0.0, 1.0), (-1.0, 0.0), (0.0, -1.0)]  # exact cos, sin of k * 90 degrees
+SNAP = 1e-9  # fp64 residue of the MJCF's quaternions, far below fp32 rounding: treated as 0
+
+
+def _sym(I):
+    return np.array([[I[0], I[3], I[4]], [I[3], I[1], I[5]], [I[4], I[5], I[2]]])
+
+
+def reframe(flat):
+    """The link constants in modified-DH-like frames, in fp64.
+
+    Each link frame may turn about its own joint axis (and the base frame about gravity) without changing bias or M.
+    Frame i is turned by phi_i so that the constant rotation of link i + 1 is Rx(alpha) Rz(theta): a rotation about x
+    whose alpha is a quarter turn up to ~1e-5 rad, then a turn about the joint axis that merges with the joint angle.
+    phi_0 .. phi_4 are exact quarter turns (the inertial constants are only permuted); the last link is turned by its
+    own small residual so that it needs no merge, and link 0's rotation goes into the base frame (gravity rotates).
+    Each frame's origin may also slide along its joint axis: it moves to where link i + 1's origin has z = 0.
+    Returns per link (ct, st, (ca, sa) or None, p, m, h, I, arm) and a0."""
+    R = [np.array(flat[23 * i:23 * i + 9]).reshape(3, 3) for i in range(NJ)]
+    phi = []
+    for i in range(NJ - 1):
+        Rn = R[i + 1]
+        k = 0 if Rn[0, 2] == 0 and Rn[1, 2] == 0 else round(np.degrees(np.arctan2(Rn[0, 2], -Rn[1, 2])) / 90) % 4
+        phi.append(_rz(*QUARTER[k]))
+    R5 = phi[-1].T @ R[-1]
+    b = np.arctan2(R5[2, 0], R5[2, 1])
+    phi.append(_rz(np.cos(b), -np.sin(b)))
+    base = R[0] @ phi[0]
+    rot, p, h, S, m = [], [], [], [], [flat[23 * i + 12] for i in range(NJ)]
+    for i in range(NJ):
+        f = flat[23 * i:23 * i + 23]
+        Rp = np.eye(3) if i == 0 else phi[i - 1].T @ R[i] @ phi[i]
+        ct, st, ca, sa = (0.0 if abs(x) < SNAP else x for x in (Rp[0, 0], -Rp[0, 1], Rp[2, 2], -Rp[1, 2]))
+        Rx = np.array([[1.0, 0.0, 0.0], [0.0, ca, -sa], [0.0, sa, ca]])
+        assert np.abs(Rx @ _rz(ct, st) - Rp).max() < SNAP, f"link {i}: constant rotation is not Rx(alpha) Rz(theta)"
+        rot.append((ct, st, ca, sa))
+        p.append(np.array(f[9:12]) if i == 0 else phi[i - 1].T @ np.array(f[9:12]))  # link 0's origin is never used
+        h.append(phi[i].T @ np.array(f[13:16]))
+        S.append(phi[i].T @ _sym(f[16:22]) @ phi[i])
+    # frame i's origin slides along its joint axis onto the plane z = 0 of link i + 1's origin; the inertia moves to the
+    # new origin (about o' = o + d z: I' = I + (|h'|^2 - |h|^2) / m E - (h' h'^T - h h^T) / m, h' = h - m d z)
+    for i in range(NJ - 1):
+        d = p[i + 1][2]
+        p[i + 1] = np.array([p[i + 1][0], p[i + 1][1], 0.0])
+        if i > 0:
+            p[i] = p[i] + d * np.array([0.0, -rot[i][3], rot[i][2]])
+        hn = h[i] - np.array([0.0, 0.0, m[i] * d])
+        S[i] = S[i] + (hn @ hn - h[i] @ h[i]) / m[i] * np.eye(3) - (np.outer(hn, hn) - np.outer(h[i], h[i])) / m[i]
+        h[i] = hn
+    links = []
+    for i in range(NJ):
+        ct, st, ca, sa = rot[i]
+        I = [S[i][0, 0], S[i][1, 1], S[i][2, 2], S[i][0, 1], S[i][0, 2], S[i][1, 2]]
+        links.append((ct, st, None if (ca, sa) == (1.0, 0.0) else (ca, sa), list(p[i]), m[i], list(h[i]), I, flat[23 * i + 22]))
+    a0 = base.T @ np.array(flat[138:141])
+    return links, [0.0 if abs(x) < SNAP * abs(a0).max() else x for x in a0]
+
+
 class Link:
-    def __init__(self, g, flat, sj, cj):
-        f = [float(np.float32(x)) for x in flat]
-        R = np.array(f[0:9]).reshape(3, 3)
-        self.p, self.m, self.h, self.I, self.arm = f[9:12], f[12], f[13:16], f[16:22], f[22]
-        # planar constant rotation about the joint axis: R = Rz(theta)  =>  R*Rz(q) = Rz(theta + q)
-        self.planar = (R[2, 2] == 1.0 and R[0, 2] == 0 and R[1, 2] == 0 and R[2, 0] == 0 and R[2, 1] == 0
-                       and R[0, 0] == R[1, 1] and R[0, 1] == -R[1, 0])
-        if self.planar:
-            ct, st = R[0, 0], R[1, 0]
-            self.s, self.c = sj * ct + cj * st, cj * ct - sj * st
+    def __init__(self, g, frame, sj, cj):
+        ct, st, rx, p, m, h, I, arm = frame
+        r32 = lambda v: [float(np.float32(x)) for x in v]  # noqa: E731
+        self.p, self.m, self.h, self.I, self.arm = r32(p), r32([m])[0], r32(h), r32(I), r32([arm])[0]
+        # the turn about the joint axis merges with the joint angle: Rz(theta) Rz(q) = Rz(theta + q)
+        ct, st = r32([ct, st])
+        self.planar = (ct, st) != (1.0, 0.0)
+        self.s, self.c = (sj * ct + cj * st, cj * ct - sj * st) if self.planar else (sj, cj)
+        if rx is None:
             self.R = None
         else:
-            self.s, self.c, self.R = sj, cj, R
+            ca, sa = r32(rx)
+            self.R = np.array([[1.0, 0.0, 0.0], [0.0, ca, -sa], [0.0, sa, ca]])
 
     def to_parent(self, v):
         x, y, z = self.c * v[0] - self.s * v[1], self.s * v[0] + self.c * v[1], v[2]
@@ -203,13 +267,14 @@ def build(flat):
     c = [g.var(f"c[{i}]") for i in range(NJ)]
     qd = [g.var(f"qd[{i}]") for i in range(NJ)]
     K = lambda x: g.const(x)  # noqa: E731
-    links = [Link(g, flat[23 * i:23 * i + 23], s[i], c[i]) for i in range(NJ)]
+    frames, a0 = reframe(flat)
+    links = [Link(g, frames[i], s[i], c[i]) for i in range(NJ)]
     for L in links:
         L.p = [K(x) for x in L.p]; L.h = [K(x) for x in L.h]; L.I = [K(x) for x in L.I]
         L.m = K(L.m); L.arm = K(L.arm)
         if L.R is not None:
             L.R = np.array([[K(x) for x in row] for row in L.R], dtype=object)
-    a0 = [K(x) for x in flat[138:141]]
+    a0 = [K(x) for x in a0]
     zero = K(0.0)
     w, wd, a = [zero] * 3, [zero] * 3, a0
     f, n = [None] * NJ, [None] * NJ
@@ -272,15 +337,29 @@ def emit(g, outs):
             uses[b] = uses.get(b, 0) + 1
     for _, v in outs:
         uses[v.n] = uses.get(v.n, 0) + 1
-    # a mul that feeds exactly one add/sub is fused into it (one product per fma)
-    fused = set()
+    # a mul that feeds exactly one add/sub is fused into it (one product per fma); then a mul whose every consumer is an
+    # add/sub with no product fused yet is formed inside each of them (k fma instead of one mul and k additions)
+    consumers = {}
+    for n in sorted(live):
+        k, a, b = g.nodes[n]
+        if k in ("add", "sub", "mul"):
+            consumers.setdefault(a, []).append(n); consumers.setdefault(b, []).append(n)
+    fuse_into = {}  # add/sub node -> the mul it forms
     for n in sorted(live):
         k, a, b = g.nodes[n]
         if k in ("add", "sub"):
             for x in (a, b):
                 if g.nodes[x][0] == "mul" and uses.get(x, 0) == 1:
-                    fused.add(x)
+                    fuse_into[n] = x
                     break
+    outn = {v.n for _, v in outs}
+    for n in sorted(live):
+        cs = consumers.get(n, [])
+        if (g.nodes[n][0] == "mul" and len(cs) > 1 and n not in outn
+                and all(g.nodes[x][0] in ("add", "sub") and x not in fuse_into for x in cs)):
+            for x in cs:
+                fuse_into[x] = n
+    fused = set(fuse_into.values())
 
     def ref(n):
         k, a, b = g.nodes[n]
@@ -298,11 +377,11 @@ def emit(g, outs):
             continue
         cnt = nop[g.node_region[n]]
         if k == "mul":
-            lines.append(f"  const T t{n} = {ref(a)} * {ref(b)};"); cnt["mul"] += 1
+            lines.append(f"  const T t{n} = so_mul({ref(a)}, {ref(b)});"); cnt["mul"] += 1
             continue
-        fa, fb = a in fused, b in fused
-        if fa or fb:
-            m, o = (a, b) if fa else (b, a)
+        if n in fuse_into:
+            m = fuse_into[n]
+            fa, o = m == a, b if m == a else a
             _, x, y = g.nodes[m]
             if k == "add":
                 e = f"so_fma({ref(x)}, {ref(y)}, {ref(o)})"
@@ -312,7 +391,7 @@ def emit(g, outs):
                 e = f"so_fma(-{ref(x)}, {ref(y)}, {ref(o)})"
             cnt["fma"] += 1
         else:
-            e = f"{ref(a)} {'+' if k == 'add' else '-'} {ref(b)}"; cnt["add"] += 1
+            e = f"so_{k}({ref(a)}, {ref(b)})"; cnt["add"] += 1
         lines.append(f"  const T t{n} = {e};")
     for name, v in outs:
         lines.append(f"  {name} = {'-' if v.s < 0 else ''}{ref(v.n)};")

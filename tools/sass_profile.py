@@ -28,22 +28,27 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def line_table(lib: str, func_substr: str, labels: dict = None):
-    """offset -> (file, line) of the innermost source line, from nvdisasm -g of the cubin inside `lib`.  `labels`, if
-    given, receives branch label -> offset."""
+    """offset -> (file, line) of the innermost source line, from nvdisasm -gi of the cubin inside `lib`; an instruction
+    of a helper inlined into the generated dynamics (so_fma, so_mul, ...) counts as the generated line that calls it.
+    `labels`, if given, receives branch label -> offset."""
     tmp = tempfile.mkdtemp()
     subprocess.check_call(["cuobjdump", "-xelf", "all", os.path.abspath(lib)], cwd=tmp, stdout=subprocess.DEVNULL)
     cubin = [os.path.join(tmp, f) for f in os.listdir(tmp) if f.endswith(".cubin")][0]
-    txt = subprocess.run(["nvdisasm", "-g", "-c", cubin], capture_output=True, text=True).stdout
-    table, cur, on, pending = {}, ("?", 0), False, []
+    txt = subprocess.run(["nvdisasm", "-gi", "-c", cubin], capture_output=True, text=True).stdout
+    table, cur, on, pending, innermost = {}, ("?", 0), False, [], True
     for ln in txt.splitlines():
         if ln.startswith("//---") and ".text." in ln:
             on = func_substr in ln
             continue
         if not on:
             continue
-        m = re.search(r'//## File "([^"]+)", line (\d+)', ln)
-        if m:
-            cur = (os.path.basename(m.group(1)), int(m.group(2)))
+        m = re.search(r'//## File "([^"]+)", line (\d+)(?: inlined at "([^"]+)", line (\d+))?', ln)
+        if m:  # the inline chain, innermost first
+            if innermost:
+                cur = (os.path.basename(m.group(1)), int(m.group(2)))
+            if m.group(3) and os.path.basename(m.group(3)) == "so100_dyn_gen.cuh" and cur[0] != "so100_dyn_gen.cuh":
+                cur = ("so100_dyn_gen.cuh", int(m.group(4)))
+            innermost = False
             continue
         m = re.match(r"(\.L_x_\d+):", ln.strip())
         if m:
@@ -52,6 +57,7 @@ def line_table(lib: str, func_substr: str, labels: dict = None):
         m = re.match(r"\s+/\*([0-9a-f]{4,6})\*/\s+(.*?);", ln)
         if m:
             table[int(m.group(1), 16)] = (cur, m.group(2).strip())
+            innermost = True
             if labels is not None:
                 labels.update((name, int(m.group(1), 16)) for name in pending)
             pending = []
